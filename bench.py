@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""bench.py -- headline benchmark of the B200 descriptor matcher (contract: see the task brief).
+"""bench.py -- headline benchmark of the B200 descriptor matcher; prints one JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one whole matcher call over one synthetic descriptor pair of the named BASELINE.json
 configuration: descriptor upload/packing + forward kNN (+ reverse kNN for mutual) + filter.
@@ -12,6 +12,8 @@ Multi-GPU (torchrun, one rank per GPU): source rows (and, for the mutual pass, t
 across ranks, both descriptor sets replicated; one NCCL all-gather of the reverse table; strong scaling.
 `--impl reference` times the reference's CPU matcher semantics (the oracle port; the reference itself
 cannot be built here: PCL/OpenCV/FLANN absent) on the host cores, bounded sample per step.
+`--dump-outputs DIR` writes what the last timed step returned (see write_outputs); the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import contextlib
@@ -336,6 +338,36 @@ def workload_config(wl, world):
                    "inputs smaller than L2; the step rewrites >126 MB of operands/candidates between kNN passes")}
 
 
+DUMP_BYTES = 60 * 10 ** 6     # --dump-outputs stays under 64 MB, .npy headers included
+
+
+def write_outputs(out_dir, n_rows, records=None, per_row=1, lists=None):
+    """--dump-outputs: what a matcher call hands its caller, as out_dir/<name>.npy -- indices and counts in float64 (exact),
+    distances and thresholds in float32.  `records`: CORR_DTYPE correspondences of n_rows query rows, ascending index_query,
+    at most `per_row` per row; `lists`: the k-lists (idx [n_rows, k], dist [n_rows, k], cnt [n_rows]).  When the largest output
+    the workload can produce does not fit DUMP_BYTES, only the outputs of a seeded sample of query rows are written (their
+    indices in query_rows.npy).  The sample depends on n_rows and the output shape alone, so every build writes the same rows.
+    Returns the names written."""
+    row_bytes = 8 + (per_row * 24 if records is not None else lists[0].shape[1] * 12 + 8)   # + 8: query_rows
+    rows = None
+    if n_rows * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n_rows, DUMP_BYTES // row_bytes, replace=False))
+    if records is not None:
+        if rows is not None:
+            records = records[np.isin(records["index_query"], rows)]
+        arrays = {"index_query": records["index_query"].astype(np.float64), "index_match": records["index_match"].astype(np.float64),
+                  "distance": records["distance"], "threshold": records["threshold"]}
+    else:
+        idx, dist, cnt = lists if rows is None else (a[rows] for a in lists)
+        arrays = {"knn_index": idx.astype(np.float64), "knn_distance": dist, "knn_count": cnt.astype(np.float64)}
+    if rows is not None:
+        arrays["query_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+    return sorted(arrays)
+
+
 # ------------------------------------------------------------------------------------------
 def run_b200(args, wl):
     import torch
@@ -388,8 +420,9 @@ def run_b200(args, wl):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item()), out
 
-    def measure(wl, steps, warmup, with_e2e, with_clocks):
-        """Device-resident value + candidate-kernel roofline (+ e2e through the host-facing C-ABI) of one workload."""
+    def measure(wl, steps, warmup, with_e2e, with_clocks, dump_dir=None):
+        """Device-resident value + candidate-kernel roofline (+ e2e through the host-facing C-ABI) of one workload; with
+        dump_dir, the outputs of the last timed step are written there."""
         desc, n_src, n_tgt, k, mode_name, cfg = WORKLOADS[wl]
         tsharded = mode_name == "knn_target_sharded"
         mode = modes[mode_name]
@@ -406,7 +439,7 @@ def run_b200(args, wl):
             be.upload_device(1, tgt, dim, index_offset=t_off)
             if tsharded:
                 idx, dst, cnt = sm.knn_target_sharded(k)
-                return idx, cnt.sum(), dst
+                return idx, cnt.sum(), dst, cnt
             if world == 1:
                 return be.match_device(k, mode)
             return sm.match_query_sharded(k, mode)      # this rank's slice of the records stays in HBM (see config.note)
@@ -424,6 +457,16 @@ def run_b200(args, wl):
         n_corr = int(out[1].item())
         res = {"value": n_src * steps / (ms_total * 1e-3), "ms_per_step": ms_total / steps, "launches": int(st["launches"]),
                "clocks": clocks, "dim": dim, "stride_b": stride_b, "n_corr": n_corr}
+        if dump_dir:   # copied out before the e2e calls below reuse the context
+            if tsharded:
+                lists = [x.cpu().numpy() for x in (out[0], out[2], out[3])]
+                if rank == 0:
+                    write_outputs(dump_dir, n_src, lists=lists)
+            else:   # several GPUs: the rank slices in rank order are the single-GPU output
+                rec, _ = sm.gather_records(out[0], out[1])
+                if rank == 0:
+                    write_outputs(dump_dir, n_src, records=rec.cpu().numpy().view(M.CORR_DTYPE).reshape(-1),
+                                  per_row=k if mode == M.MODE_MUTUAL else 1)
 
         # ---- roofline of the dominant kernel (tcgen05 candidate pass): CUDA events around every launch of the timed
         #      region above, on the stream the kernel is launched on ----
@@ -481,7 +524,7 @@ def run_b200(args, wl):
         src_np, tgt_np = src.cpu().numpy(), tgt.cpu().numpy()              # pageable, as the reference's pcl::PointCloud is
         src_pin, tgt_pin = torch.from_numpy(src_np).pin_memory(), torch.from_numpy(tgt_np).pin_memory()
         e2e = {}
-        n_steps = max(2, min(steps, 5))
+        n_steps = steps
         if world == 1:
             # exactly the calls the C++ shim makes: b200m_upload x 2 + b200m_match (or b200m_knn for the raw k-lists)
             out_np = np.empty(max(n_src * kk, 1), M.CORR_DTYPE)
@@ -565,7 +608,7 @@ def run_b200(args, wl):
 
     desc, n_src, n_tgt, k, mode_name, cfg = WORKLOADS[wl]
     tsharded = mode_name == "knn_target_sharded"
-    main = measure(wl, args.steps, args.warmup, True, True)
+    main = measure(wl, args.steps, args.warmup, True, True, args.dump_outputs)
 
     # the other single-GPU BASELINE configs, embedded so that a default run shows them too (fewer steps, no e2e)
     others = {}
@@ -641,7 +684,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the embedded c2 / c4 lines of a default (c3, 1 GPU) run")
     ap.add_argument("--other-configs", action="store_true", help="several GPUs: also embed the c4 (query-sharded) and c5 (target-sharded) lines")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU path's outputs (the reference arm times a sample sized by the clock)")
     # stdout carries the ONE JSON line and nothing else: whatever a library prints through C stdio or fd 1 during the run
     # (NCCL's "NCCL version ..." banner does, on boxes where NCCL_DEBUG defaults to VERSION, NCCL_DEBUG_FILE or not) goes to
     # stderr; the line itself is written to the saved descriptor at the end.
