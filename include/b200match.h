@@ -168,6 +168,31 @@ B200M_API int b200m_match(b200m_ctx *ctx, const b200m_params *p, const float *th
                           const float *thr_tgt, b200m_corr *out, size_t cap, size_t *n_out,
                           float *avg_first_dist);
 
+/* ---- batches: many independent (source, target) pairs in one call -----------------------------
+ * Multi-view registration (all pairs of N scans), one scan against many submaps, or a whole table of evaluation
+ * pairs: one call per direction fills the GPU instead of one small call per pair.  All pairs share the descriptor
+ * type (stride_bytes, dim) and the params.  Pair p's output equals, byte for byte, what b200m_upload(0, src_p),
+ * b200m_upload(1, tgt_p) and then b200m_knn (direction 0, all rows) / b200m_match on that pair alone return, with
+ * pair-local indices.  Empty sets are allowed on either side (empty lists, no records).  A batch call REPLACES the
+ * descriptor sets b200m_upload put in the context (upload again before the next single-pair call).  Host pointers. */
+typedef struct {
+    const float *src;   /* first descriptor value of source row 0 (rows stride_bytes apart) */
+    size_t n_src;
+    const float *tgt;
+    size_t n_tgt;
+} b200m_pair;
+/* raw k-lists of every pair, direction 0: rows concatenated in pair order ([sum n_src][k], [sum n_src]), pair-local train
+ * indices, -1 padded as b200m_knn's */
+B200M_API int b200m_knn_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                              size_t stride_bytes, int dim, int32_t *idx, float *dist, int32_t *count);
+/* b200m_match of every pair (modes as b200m_match accepts; CLUSTER is an error): records of pair p are
+ * out[offsets[p] .. offsets[p+1]), ascending index_query, pair-local indices; offsets has n_pairs + 1 entries and is
+ * filled also when cap is too small (error; sum n_src * k always suffices); avg (may be NULL) gets n_pairs averages;
+ * thr_src / thr_tgt are the pairs' thresholds concatenated in pair order (sum n_src / sum n_tgt floats) or both NULL. */
+B200M_API int b200m_match_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                                size_t stride_bytes, int dim, const float *thr_src, const float *thr_tgt,
+                                b200m_corr *out, size_t cap, size_t *offsets, float *avg);
+
 /* ---- device-side building blocks for sharded (multi-GPU) runs ----------------
  * All pointers are device pointers on the context's device; work is queued on the
  * context's stream.  Forward tables cover query rows [row_begin,row_end) of side 0;

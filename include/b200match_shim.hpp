@@ -3,6 +3,8 @@
 //
 //   matchBF<FeatureT> / matchFLANN<FeatureT> / matchLocal<FeatureT>(radius = inf)
 //                                  reference include/matching.h:368-383, :562-678
+//   knnBatch<FeatureT> / matchBatch<FeatureT>
+//                                  many (source, target) cloud pairs in one call: matchBF / the k-list filter per pair
 //   MultivaluedCorrespondence      reference include/common.h:192-195
 //   Correspondence                 reference include/common.h:120-127
 //   FeatureBasedMatcher, FeatureBasedMatcherImpl<FeatureT>::Storage, OneSidedMatcher / LeftToRightMatcher /
@@ -26,6 +28,7 @@
 #include <memory>
 #include <stdexcept>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "b200match.h"
@@ -165,6 +168,78 @@ inline b200m_params make_params(const AlignmentParameters &p, int mode, int k) {
     q.n_gpus = 0;
     q.shard = B200M_SHARD_QUERY;
     return q;
+}
+
+// ---- batches: many (query / source, train / target) cloud pairs in one call (b200m_knn_batch / b200m_match_batch) ----
+// Pair p's result is the one the per-pair call (matchBF, or upload + b200m_match) gives, with pair-local indices.  The batch
+// replaces the descriptor sets of the shared context.
+template <typename FeatureT>
+using CloudPairs = std::vector<std::pair<FeatureCloud<FeatureT>, FeatureCloud<FeatureT>>>;
+
+template <typename FeatureT>
+std::vector<b200m_pair> batch_pairs(const CloudPairs<FeatureT> &pairs, size_t *n_src_total) {
+    std::vector<b200m_pair> v(pairs.size());
+    *n_src_total = 0;
+    for (size_t i = 0; i < pairs.size(); ++i) {
+        v[i].src = reinterpret_cast<const float *>(cloud_data<FeatureT>(pairs[i].first));
+        v[i].n_src = cloud_size<FeatureT>(pairs[i].first);
+        v[i].tgt = reinterpret_cast<const float *>(cloud_data<FeatureT>(pairs[i].second));
+        v[i].n_tgt = cloud_size<FeatureT>(pairs[i].second);
+        *n_src_total += v[i].n_src;
+    }
+    return v;
+}
+
+// matchBF of every pair: result[p] has one entry per query row of pair p
+template <typename FeatureT>
+std::vector<std::vector<MultivaluedCorrespondence>> knnBatch(const CloudPairs<FeatureT> &pairs, const AlignmentParameters &parameters) {
+    size_t nq = 0;
+    std::vector<b200m_pair> bp = batch_pairs<FeatureT>(pairs, &nq);
+    const int k = parameters.randomness;
+    std::vector<int32_t> idx(nq * k);
+    std::vector<float> dist(nq * k);
+    std::vector<int32_t> cnt(nq);
+    b200m_params p = make_params(parameters, B200M_MODE_KNN_ONLY, k);
+    Context &ctx = shared_context(parameters.device);
+    ctx.check(b200m_knn_batch(ctx.get(), &p, bp.data(), (int) bp.size(), sizeof(FeatureT), feature_dim<FeatureT>(), idx.data(),
+                              dist.data(), cnt.data()));
+    std::vector<std::vector<MultivaluedCorrespondence>> out(bp.size());
+    size_t row = 0;
+    for (size_t q = 0; q < bp.size(); ++q) {
+        out[q].resize(bp[q].n_src);
+        for (size_t i = 0; i < bp[q].n_src; ++i, ++row) {
+            out[q][i].match_indices.assign(idx.begin() + row * k, idx.begin() + row * k + cnt[row]);
+            out[q][i].distances.assign(dist.begin() + row * k, dist.begin() + row * k + cnt[row]);
+        }
+    }
+    return out;
+}
+
+struct BatchMatches {
+    std::vector<CorrespondencesPtr> correspondences;   // per pair, ascending index_query, pair-local indices
+    std::vector<float> average_distances;              // per pair: FeatureBasedMatcher::getAverageDistance()
+};
+
+// The k-list filter of every pair: mode B200M_MODE_ONE_SIDED / MUTUAL / RATIO / RATIO_MUTUAL, k = randomness (ratio modes:
+// max(ratio_k, 2)), thresholds = distance_thr -- b200m_match on each pair alone.
+template <typename FeatureT>
+BatchMatches matchBatch(const CloudPairs<FeatureT> &pairs, const AlignmentParameters &parameters, int mode) {
+    size_t nq = 0;
+    std::vector<b200m_pair> bp = batch_pairs<FeatureT>(pairs, &nq);
+    const bool ratio = mode == B200M_MODE_RATIO || mode == B200M_MODE_RATIO_MUTUAL;
+    const int k = ratio ? std::max(parameters.ratio_k, 2) : parameters.randomness;
+    b200m_params p = make_params(parameters, mode, k);
+    Correspondences all(std::max<size_t>(nq * (mode == B200M_MODE_MUTUAL ? k : 1), 1));
+    std::vector<size_t> offsets(bp.size() + 1);
+    BatchMatches r;
+    r.average_distances.resize(bp.size());
+    Context &ctx = shared_context(parameters.device);
+    ctx.check(b200m_match_batch(ctx.get(), &p, bp.data(), (int) bp.size(), sizeof(FeatureT), feature_dim<FeatureT>(), nullptr,
+                                nullptr, reinterpret_cast<b200m_corr *>(all.data()), all.size(), offsets.data(),
+                                r.average_distances.data()));
+    for (size_t q = 0; q < bp.size(); ++q)
+        r.correspondences.push_back(std::make_shared<Correspondences>(all.begin() + offsets[q], all.begin() + offsets[q + 1]));
+    return r;
 }
 
 // matchBF<FeatureT> (reference include/matching.h:594-634): one entry per query, <= k matches, ascending L2.

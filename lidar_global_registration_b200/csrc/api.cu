@@ -155,7 +155,7 @@ void b200m_destroy(b200m_ctx *ctx) {
                     &ctx->ws_out, &ctx->ws_misc, &ctx->ws_fidx, &ctx->ws_fdist, &ctx->ws_fcnt, &ctx->ws_ridx,
                     &ctx->ws_rdist, &ctx->ws_rcnt, &ctx->ws_corr, &ctx->ws_totals, &ctx->ws_part_i, &ctx->ws_part_d,
                     &ctx->ws_done, &ctx->ws_cand_val, &ctx->ws_cand_thr, &ctx->ws_row_list, &ctx->ws_row_flags,
-                    &ctx->ws_sel_ops, &ctx->ws_sel_norm, &ctx->ws_sweep_hint};
+                    &ctx->ws_sel_ops, &ctx->ws_sel_norm, &ctx->ws_sweep_hint, &ctx->ws_batch};
     for (DevBuf *b : ws) b->release();
     tc_release(ctx);
     multiscale_release(ctx);
@@ -243,7 +243,7 @@ static void stage_release(b200m_ctx *ctx) {
     ctx->stage = nullptr;
 }
 
-static bool is_pageable(const void *p) {
+bool is_pageable(const void *p) {
     cudaPointerAttributes a;
     if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
         cudaGetLastError();
@@ -252,7 +252,7 @@ static bool is_pageable(const void *p) {
     return a.type == cudaMemoryTypeUnregistered;
 }
 
-static int staged_h2d(b200m_ctx *ctx, void *dst, const void *src, size_t bytes) {
+int staged_h2d(b200m_ctx *ctx, void *dst, const void *src, size_t bytes) {
     if (!ctx->stage) ctx->stage = new StagePool();
     StagePool *sp = static_cast<StagePool *>(ctx->stage);
     if (!sp->ready) {
@@ -268,7 +268,8 @@ static int staged_h2d(b200m_ctx *ctx, void *dst, const void *src, size_t bytes) 
     for (int c = 0; off < bytes; ++c) {
         const int b = c % StagePool::kBufs;
         const size_t len = bytes - off < StagePool::kChunk ? bytes - off : StagePool::kChunk;
-        if (c >= StagePool::kBufs) CK(cudaEventSynchronize(sp->free_ev[b]));   // the DMA out of this buffer has finished
+        // the DMA out of this buffer has finished (also the one queued by the previous call: a batch stages many sets in a row)
+        CK(cudaEventSynchronize(sp->free_ev[b]));
         const char *s = static_cast<const char *>(src) + off;
         char *d = static_cast<char *>(sp->buf[b]);
         const size_t part = (len / n_thr + 4095) & ~(size_t) 4095;
@@ -289,7 +290,7 @@ static int staged_h2d(b200m_ctx *ctx, void *dst, const void *src, size_t bytes) 
 }
 
 // ---- upload -----------------------------------------------------------------------------
-static int upload_common(b200m_ctx *ctx, int side, const float *device_aos, size_t n, size_t stride_bytes, int dim,
+int upload_common(b200m_ctx *ctx, int side, const float *device_aos, size_t n, size_t stride_bytes, int dim,
                          int64_t index_offset) {
     Side &sd = ctx->side[side];
     sd.n = n;
@@ -312,7 +313,7 @@ static int upload_common(b200m_ctx *ctx, int side, const float *device_aos, size
     return 0;
 }
 
-static int check_upload_args(b200m_ctx *ctx, int side, const float *base, size_t n, size_t stride_bytes, int dim) {
+int check_upload_args(b200m_ctx *ctx, int side, const float *base, size_t n, size_t stride_bytes, int dim) {
     if (side != 0 && side != 1) return b200m_fail_msg(ctx, "b200m_upload: side must be 0 (source) or 1 (target)");
     if (dim < 1 || dim > B200M_MAX_DIM) return b200m_fail_msg(ctx, "b200m_upload: dim out of range [1, 1024]");
     if (stride_bytes % 4 != 0 || stride_bytes < (size_t) dim * 4)
@@ -359,7 +360,7 @@ __global__ void fill_empty_kernel(size_t n_rows, int k, int32_t *idx, float *dis
     if (i < n_rows) count[i] = 0;
 }
 
-static int check_params(b200m_ctx *ctx, const b200m_params *p) {
+int check_params(b200m_ctx *ctx, const b200m_params *p) {
     if (!p) return b200m_fail_msg(ctx, "null params");
     if (p->k < 1 || p->k > B200M_MAX_K) return b200m_fail_msg(ctx, "params.k must be in [1, 32]");
     if (p->mode < B200M_MODE_KNN_ONLY || p->mode > B200M_MODE_CLUSTER) return b200m_fail_msg(ctx, "params.mode unknown");
@@ -418,7 +419,7 @@ __global__ void gather_query_rows_kernel(const int32_t *__restrict__ row_list, s
 // kNN of query rows [row_begin, row_begin + n_rows) of `direction`; with d_flags, only of the flagged (and valid) rows --
 // every other row gets an empty list.  Outputs are indexed by (row - row_begin).
 int b200m_knn_rows(b200m_ctx *ctx, const b200m_params *p, int direction, size_t row_begin, size_t n_rows,
-                   const uint8_t *d_flags, int32_t *d_idx, float *d_dist, int32_t *d_count) {
+                   const uint8_t *d_flags, int32_t *d_idx, float *d_dist, int32_t *d_count, const SegTable *seg) {
     Side &q = ctx->side[direction], &t = ctx->side[1 - direction];
     const int k = p->k;
     cudaStream_t st = ctx->stream;
@@ -465,7 +466,7 @@ int b200m_knn_rows(b200m_ctx *ctx, const b200m_params *p, int direction, size_t 
         StatTimer tf(ctx, &ctx->stats.ms_fallback);
         CK(launch_exact_rows(q.f32.as<float>(), q.valid.as<uint8_t>(), q.dp, q.dim, t.f32.as<float>(),
                              t.valid.as<uint8_t>(), t.n, t.index_offset, row_begin, n_work, nullptr, nullptr, k, d_idx,
-                             d_dist, d_count, 1 << 30, 0, nullptr, nullptr, nullptr, row_map, st));
+                             d_dist, d_count, 1 << 30, 0, nullptr, nullptr, nullptr, row_map, st, seg ? seg->range : nullptr));
         ctx->stats.launches += 1;
         tf.stop();
         return 0;
@@ -494,7 +495,7 @@ int b200m_knn_rows(b200m_ctx *ctx, const b200m_params *p, int direction, size_t 
         }
         StatTimer tc(ctx, &ctx->stats.ms_candidates);
         if (tc_candidates(ctx, direction, row_map ? 0 : row_begin, n_work, k, p->cand_cap, &n_lists, &cap, &has_values, nullptr, 0,
-                          q_ops, q_norm, q_pad))
+                          q_ops, q_norm, q_pad, seg))
             return 1;
         tc.stop();
     }
@@ -531,7 +532,8 @@ int b200m_knn_rows(b200m_ctx *ctx, const b200m_params *p, int direction, size_t 
                              t.valid.as<uint8_t>(), t.n, t.index_offset, row_begin, n_work,
                              ctx->ws_flag_rows.as<int32_t>(), ctx->ws_counters.as<int32_t>(), k, d_idx, d_dist, d_count,
                              (int) (n_work < max_blocks ? n_work : max_blocks), split_blocks, ctx->ws_part_i.as<int32_t>(),
-                             ctx->ws_part_d.as<float>(), ctx->ws_done.as<unsigned int>(), row_map, st));
+                             ctx->ws_part_d.as<float>(), ctx->ws_done.as<unsigned int>(), row_map, st,
+                             seg ? seg->range : nullptr));
         ctx->stats.launches += 2;
         tf.stop();
     }

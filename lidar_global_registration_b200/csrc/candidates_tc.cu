@@ -77,6 +77,8 @@ struct TcParams {
     int sweep_lag;        // tiles between consecutive followers of the rotated sweep; 0: every pair starts at tile 0
     int *sweep_hint;      // [train splits] how many tiles the most advanced CTA pair of a split has swept since the launch began
                           // (chunk-entry kernels: a pair starts a fixed distance behind it and wraps around)
+    const int2 *seg_range;   // batch calls (or null): [query row / 256] = {first, end} train row of that query block's pair; the
+                             // CTA then sweeps split `blockIdx.y` of that pair's train tiles only
     int debug_flags;      // timing experiments only (B200M_TC_DEBUG): 1 = epilogue skips its work, 2 = no MMAs issued,
                           // 4 = no B loads (pair mode), 8 / 16 = ring limited to 4 / 6 stages, 32 = epilogue only
                           // drains TMEM (no filtering), 64 / 128 = force EH = 1 / 2, 256 = fast path only,
@@ -622,7 +624,11 @@ __device__ __forceinline__ void chunk_hits(float m0, float m1, float m2, float m
 //         as soon as both of its 64-column warps have their values in registers, all filtering happens off the chain.
 //       4, 5 ("chunk entries", the default): alternating tiles, but a list entry is a 32-column chunk (first train row,
 //         minimum) instead of a column -- see chunk_hits; drained by 32-column (4) or 16-column (5) TMEM loads.
-template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG>
+// SEG:  (batch calls, production instantiations only) the CTA's train tiles come from TcParams::seg_range.  A compile-time
+//       switch, not a runtime test of the pointer: either half of the lookup (the load, or the early exit) changes the register
+//       allocation of the whole kernel -- the chunk-entry epilogue then spills more and the C2 launch runs 3.25 -> 3.50 ms on
+//       one B200 (profiles/r03_ab_c2_seg_runtime.log).  SEG = false compiles to the single-pair kernel as it was.
+template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG, bool SEG>
 __global__ void __launch_bounds__(EPI ? 640 : 64 + 128 * EH + (SPLITN ? 32 : 0), 1)
 tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_t,
                      const TcParams p) {
@@ -669,9 +675,32 @@ tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int qtile = blockIdx.x, split = blockIdx.y;
-    const int t0 = dump ? p.tiles_per_split : split * p.tiles_per_split;   // dump mode: tiles_per_split holds the tile id
-    const int t1 = dump ? t0 + 1 : min(p.n_ttiles, t0 + p.tiles_per_split);
+    int seg_t0 = 0, seg_tiles = p.n_ttiles, tps = p.tiles_per_split;
+    if constexpr (SEG) {
+        // batch: the train tiles of this query block's pair (segments start at multiples of 256 rows on both sides, so the
+        // two CTAs of a pair -- 256 query rows -- share one range), divided over the splits as a whole array is
+        const int2 r = p.seg_range[(p.q_row0 + qtile * B200M_TILE_M) / B200M_TILE_N];
+        seg_t0 = r.x / B200M_TILE_N;
+        seg_tiles = (r.y + B200M_TILE_N - 1) / B200M_TILE_N - seg_t0;
+        tps = (seg_tiles + (int) gridDim.y - 1) / (int) gridDim.y;
+    }
+    const int t0 = dump ? p.tiles_per_split : seg_t0 + split * tps;   // dump mode: tiles_per_split holds the tile id
+    const int t1 = dump ? t0 + 1 : min(seg_t0 + seg_tiles, t0 + tps);
     const int ka = p.ka;
+    if (SEG && t1 <= t0) {
+        // batch: a pair with fewer train tiles than there are splits (or none) leaves this CTA nothing to sweep.  Its rows'
+        // lists are empty, with the final threshold an empty list has; the range is the same for both CTAs of a pair, so
+        // both leave here, before any barrier, TMEM allocation or pipeline exists.
+        const int local = qtile * B200M_TILE_M + (int) threadIdx.x;
+        if (threadIdx.x < B200M_TILE_M && local < p.n_rows) {
+            for (int l = 0; l < kListsPerSplit; ++l) {
+                const size_t list_row = (size_t) (split * kListsPerSplit + l) * p.n_rows + local;
+                p.cand_cnt[list_row] = 0;
+                if (p.cand_thr) p.cand_thr[list_row] = INFINITY;
+            }
+        }
+        return;
+    }
 
     if (threadIdx.x == 0) {
         asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_q)) : "memory");
@@ -1392,9 +1421,9 @@ int get_tmap(b200m_ctx *ctx, int side, bool as_query, int cluster, const CUtenso
     return 0;
 }
 
-template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG>
+template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG, bool SEG>
 int launch_tc(b200m_ctx *ctx, const CUtensorMap *mq, const CUtensorMap *mt, const TcParams &p, dim3 grid, size_t smem) {
-    CK(cudaFuncSetAttribute(tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+    CK(cudaFuncSetAttribute(tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG, SEG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = grid;
     cfg.blockDim = dim3(EPI ? 640 : 64 + 128 * EH + (SPLITN ? 32 : 0), 1, 1);
@@ -1407,7 +1436,7 @@ int launch_tc(b200m_ctx *ctx, const CUtensorMap *mq, const CUtensorMap *mt, cons
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG>, *mq, *mt, p);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG, SEG>, *mq, *mt, p);
     if (e != cudaSuccess) {
         cudaGetLastError();   // do not leave the launch error behind for the next call
         return b200m_fail_msg(ctx, std::string("tc_candidates launch failed: ") + cudaGetErrorString(e) + " (grid " +
@@ -1433,7 +1462,7 @@ void tc_release(b200m_ctx *ctx) {
 
 int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows, int k, int cap_request,
                   int *n_lists_out, int *cap_out, int *has_values_out, float *dump, size_t dump_t_tile,
-                  const void *q_ops, const float *q_norm, size_t q_pad) {
+                  const void *q_ops, const float *q_norm, size_t q_pad, const SegTable *seg) {
     Side &q = ctx->side[direction], &t = ctx->side[1 - direction];
     const int n_qtiles = (int) ((n_rows + B200M_TILE_M - 1) / B200M_TILE_M);
     // Default = CTA-pair mode (cta_group::2): the two CTAs of a cluster form one M=256 MMA, each keeps its own 128
@@ -1461,6 +1490,9 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
     if (stages < 2) return b200m_fail_msg(ctx, "tc_candidates: descriptor too long for the shared-memory pipeline");
     p.stages = stages;
     p.n_ttiles = (int) (t.n_pad / B200M_TILE_N);
+    // tiles one query block sweeps: all of them, or (batch) those of the largest pair -- splits, list capacity and the
+    // rotated sweep's default are chosen from this
+    const int sweep_tiles = seg ? seg->max_tiles : p.n_ttiles;
     // Short descriptors (FPFH: 3 MMAs per tile) are bound by the epilogue's latency chain: two epilogue warps per
     // scheduler.  Long ones (SHOT: 23 MMAs per tile) hide a four-warp epilogue, and there a thread that owns its whole row
     // also records the accumulator values so that the re-rank can prune by the row's final threshold.
@@ -1491,19 +1523,20 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
         // Each split costs a CTA prologue (about 4 tiles' worth) and a candidate list of its own (about 2 % more work
         // downstream), and keeps at least 8 train tiles.
         const long long units = (n_qtiles + cluster - 1) / cluster, slots = ctx->sm_count / cluster > 0 ? ctx->sm_count / cluster : 1;
-        int max_splits = p.n_ttiles / 8 > 0 ? p.n_ttiles / 8 : 1;
+        int max_splits = sweep_tiles / 8 > 0 ? sweep_tiles / 8 : 1;
         if (max_splits > kMaxLists) max_splits = kMaxLists;
         if (max_splits * lists_per_split > 32) max_splits = 32 / lists_per_split;   // the re-rank reads at most 32 lists per row
         double best = 0;
         for (int sp = 1; sp <= max_splits; ++sp) {
             const long long waves = (units * sp + slots - 1) / slots;
-            const double cost = (double) waves * ((p.n_ttiles + sp - 1) / sp + 4) * (1.0 + 0.02 * (sp - 1));
+            const double cost = (double) waves * ((sweep_tiles + sp - 1) / sp + 4) * (1.0 + 0.02 * (sp - 1));
             if (sp == 1 || cost < best) { best = cost; n_splits = sp; }
         }
         if (ctx->tc_splits > 0) n_splits = ctx->tc_splits < max_splits ? ctx->tc_splits : max_splits;   // B200M_TC_SPLITS: tuning override
     }
-    p.tiles_per_split = (p.n_ttiles + n_splits - 1) / n_splits;
-    n_splits = (p.n_ttiles + p.tiles_per_split - 1) / p.tiles_per_split;
+    p.tiles_per_split = (sweep_tiles + n_splits - 1) / n_splits;
+    n_splits = (sweep_tiles + p.tiles_per_split - 1) / p.tiles_per_split;
+    p.seg_range = seg && !dump ? seg->range : nullptr;
     p.q_row0 = (int) row_begin;
     p.n_rows = (int) n_rows;
     p.k = k;
@@ -1545,7 +1578,8 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
     // default: rotate when the train operands do NOT fit L2 (C4: 256 MB; measured 417 -> 372 ms per launch with 16-24 tiles
     // between followers, 8 and >= 48 are slower than no rotation; operands that fit L2 show no difference) --
     // profiles/r02_notes.md section 14.  B200M_TC_SWEEP_LAG overrides (0 = off).
-    p.sweep_lag = ctx->tc_sweep_lag >= 0 ? ctx->tc_sweep_lag : ((size_t) t.n_pad * (size_t) t.kp * 2 > (size_t) 96 << 20 ? 20 : 0);
+    p.sweep_lag = ctx->tc_sweep_lag >= 0 ? ctx->tc_sweep_lag
+                                         : ((size_t) sweep_tiles * B200M_TILE_N * (size_t) t.kp * 2 > (size_t) 96 << 20 ? 20 : 0);
     p.sweep_hint = ctx->ws_sweep_hint.as<int>();
     p.debug_flags = ctx->tc_debug;
     if (dump) p.tiles_per_split = (int) dump_t_tile;
@@ -1553,20 +1587,23 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
     dim3 grid((unsigned) (dump ? cluster : (n_qtiles + cluster - 1) / cluster * cluster), (unsigned) n_splits, 1);
     int kt = k <= 1 ? 1 : k <= 2 ? 2 : k <= 4 ? 4 : k <= 8 ? 8 : 16;
     int rc;
+    // batch launches (p.seg_range) run the production kernels with the segment lookup: the timing experiments of
+    // B200M_TC_DEBUG do not apply to them, and dump mode is single-pair only
     const bool dbg = dump != nullptr || ctx->tc_debug != 0;
-#define B200M_TC_CASE2(KT_, DBG_)                                                             \
-    rc = pair ? (eh == 2 ? (epi == 5 ? launch_tc<KT_, true, 2, true, 5, DBG_>(ctx, mq, mt, p, grid, smem)        \
-                            : epi == 4 ? launch_tc<KT_, true, 2, true, 4, DBG_>(ctx, mq, mt, p, grid, smem)      \
-                            : epi == 2 ? launch_tc<KT_, true, 2, true, 2, DBG_>(ctx, mq, mt, p, grid, smem)      \
-                            : epi == 1 ? launch_tc<KT_, true, 2, true, 1, DBG_>(ctx, mq, mt, p, grid, smem)      \
-                            : splitn ? launch_tc<KT_, true, 2, true, 0, DBG_>(ctx, mq, mt, p, grid, smem)        \
-                                     : launch_tc<KT_, true, 2, false, 0, DBG_>(ctx, mq, mt, p, grid, smem))      \
-                         : launch_tc<KT_, true, 1, false, 0, DBG_>(ctx, mq, mt, p, grid, smem))                  \
-              : (eh == 2 ? launch_tc<KT_, false, 2, false, 0, DBG_>(ctx, mq, mt, p, grid, smem)                  \
-                         : launch_tc<KT_, false, 1, false, 0, DBG_>(ctx, mq, mt, p, grid, smem))
-#define B200M_TC_CASE(KT_)               \
-    if (dbg) { B200M_TC_CASE2(KT_, true); } \
-    else { B200M_TC_CASE2(KT_, false); }
+#define B200M_TC_CASE2(KT_, DBG_, SEG_)                                                            \
+    rc = pair ? (eh == 2 ? (epi == 5 ? launch_tc<KT_, true, 2, true, 5, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)        \
+                            : epi == 4 ? launch_tc<KT_, true, 2, true, 4, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)      \
+                            : epi == 2 ? launch_tc<KT_, true, 2, true, 2, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)      \
+                            : epi == 1 ? launch_tc<KT_, true, 2, true, 1, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)      \
+                            : splitn ? launch_tc<KT_, true, 2, true, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)        \
+                                     : launch_tc<KT_, true, 2, false, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem))      \
+                         : launch_tc<KT_, true, 1, false, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem))                  \
+              : (eh == 2 ? launch_tc<KT_, false, 2, false, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)                  \
+                         : launch_tc<KT_, false, 1, false, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem))
+#define B200M_TC_CASE(KT_)                              \
+    if (p.seg_range) { B200M_TC_CASE2(KT_, false, true); } \
+    else if (dbg) { B200M_TC_CASE2(KT_, true, false); }    \
+    else { B200M_TC_CASE2(KT_, false, false); }
     switch (kt) {
         case 1: B200M_TC_CASE(1); break;
         case 2: B200M_TC_CASE(2); break;

@@ -55,7 +55,7 @@ exact_rows_kernel(const float *__restrict__ q_f32, const uint8_t *__restrict__ q
                   long long t_off, size_t row_begin, size_t n_rows, const int32_t *__restrict__ row_list,
                   const int32_t *__restrict__ row_list_count, int k, int32_t *__restrict__ idx,
                   float *__restrict__ dist, int32_t *__restrict__ count, int split_max,
-                  const int32_t *__restrict__ row_map) {
+                  const int32_t *__restrict__ row_map, const int2 *__restrict__ seg_range) {
     extern __shared__ float smem[];
     float *sq = smem;                                   // [dp] query row
     float *red_d = smem + dp;                           // [warps]
@@ -87,7 +87,13 @@ exact_rows_kernel(const float *__restrict__ q_f32, const uint8_t *__restrict__ q
         int li[KMAX];
 #pragma unroll
         for (int m = 0; m < KMAX; ++m) { ld[m] = INFINITY; li[m] = INT_MAX; }
-        for (size_t j = tid; j < nt; j += kExactThreads) {
+        size_t j_lo = 0, j_hi = nt;   // batch calls: the train rows of the query's own pair
+        if (seg_range) {
+            const int2 r = seg_range[qi / B200M_TILE_N];
+            j_lo = (size_t) r.x;
+            j_hi = (size_t) r.y;
+        }
+        for (size_t j = j_lo + tid; j < j_hi; j += kExactThreads) {
             if (!t_valid[j]) continue;   // invalid train rows are never candidates (:661)
             float d = __fsqrt_rn(seq_sqdist(sq, t_f32 + j * (size_t) dp, dp));
             if (lex_less(d, (int) j, ld[KMAX - 1], li[KMAX - 1])) {
@@ -289,7 +295,7 @@ exact_rows_split_kernel(const float *__restrict__ q_f32, int dp, const float *__
                         const int32_t *__restrict__ row_list, const int32_t *__restrict__ row_list_count, int k,
                         int32_t *__restrict__ part_i, float *__restrict__ part_d, unsigned int *__restrict__ done,
                         int32_t *__restrict__ idx, float *__restrict__ dist, int32_t *__restrict__ count,
-                        const int32_t *__restrict__ row_map) {
+                        const int32_t *__restrict__ row_map, const int2 *__restrict__ seg_range) {
     extern __shared__ float smem[];
     float *sq = smem;
     float *red_d = smem + dp;
@@ -301,12 +307,18 @@ exact_rows_split_kernel(const float *__restrict__ q_f32, int dp, const float *__
     if (total <= 0 || total > kSplitMaxRows) return;   // many flagged rows: the one-CTA-per-row kernel takes them
     const int tid = threadIdx.x;
     const int S = (int) gridDim.x;
-    const size_t chunk = (nt + S - 1) / S;
-    const size_t j0 = (size_t) blockIdx.x * chunk, j1 = j0 + chunk < nt ? j0 + chunk : nt;
     for (int r = 0; r < total; ++r) {
         const size_t local = (size_t) row_list[r];
         const size_t qi = row_map ? (size_t) row_map[local] : row_begin + local;
         const size_t orow = qi - row_begin;
+        size_t a = 0, b = nt;   // batch calls: the train rows of the query's own pair, sliced over the grid
+        if (seg_range) {
+            const int2 sr = seg_range[qi / B200M_TILE_N];
+            a = (size_t) sr.x;
+            b = (size_t) sr.y;
+        }
+        const size_t chunk = (b - a + S - 1) / S;
+        const size_t j0 = a + (size_t) blockIdx.x * chunk, j1 = j0 + chunk < b ? j0 + chunk : b;
         __syncthreads();
         for (int d = tid; d < dp; d += kExactThreads) sq[d] = q_f32[qi * (size_t) dp + d];
         __syncthreads();
@@ -902,20 +914,20 @@ cudaError_t launch_exact_t(const float *q_f32, const uint8_t *q_valid, int dp, i
                            const uint8_t *t_valid, size_t nt, int64_t t_off, size_t row_begin, size_t n_rows,
                            const int32_t *row_list, const int32_t *row_list_count, int k, int32_t *idx, float *dist,
                            int32_t *count, int blocks, int split_blocks, int32_t *part_i, float *part_d,
-                           unsigned int *done, const int32_t *row_map, cudaStream_t st) {
+                           unsigned int *done, const int32_t *row_map, cudaStream_t st, const int2 *seg_range) {
     size_t smem = sizeof(float) * dp + (sizeof(float) + 2 * sizeof(int)) * (kExactThreads / 32);
     const bool split = row_list && split_blocks > 0 && part_i && part_d && done;
     if (split) {
         exact_rows_split_kernel<KMAX><<<split_blocks, kExactThreads, smem, st>>>(
             q_f32, dp, t_f32, t_valid, nt, (long long) t_off, row_begin, row_list, row_list_count, k, part_i, part_d, done,
-            idx, dist, count, row_map);
+            idx, dist, count, row_map, seg_range);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return e;
     }
     exact_rows_kernel<KMAX><<<blocks, kExactThreads, smem, st>>>(q_f32, q_valid, dp, dim, t_f32, t_valid, nt,
                                                                  (long long) t_off, row_begin, n_rows, row_list,
                                                                  row_list_count, k, idx, dist, count,
-                                                                 split ? kSplitMaxRows : 0, row_map);
+                                                                 split ? kSplitMaxRows : 0, row_map, seg_range);
     return cudaGetLastError();
 }
 
@@ -925,13 +937,14 @@ cudaError_t launch_exact_rows(const float *q_f32, const uint8_t *q_valid, int dp
                               const float *t_f32, const uint8_t *t_valid, size_t nt, int64_t t_index_offset,
                               size_t row_begin, size_t n_rows, const int32_t *row_list, const int32_t *row_list_count,
                               int k, int32_t *idx, float *dist, int32_t *count, int max_blocks, int split_blocks,
-                              int32_t *part_i, float *part_d, unsigned int *done, const int32_t *row_map, cudaStream_t st) {
+                              int32_t *part_i, float *part_d, unsigned int *done, const int32_t *row_map, cudaStream_t st,
+                              const int2 *seg_range) {
     if (n_rows == 0) return cudaSuccess;
     int blocks = (int) (n_rows < (size_t) max_blocks ? n_rows : (size_t) max_blocks);
 #define B200M_EXACT_CASE(K)                                                                                   \
     return launch_exact_t<K>(q_f32, q_valid, dp, dim, t_f32, t_valid, nt, t_index_offset, row_begin, n_rows,  \
                              row_list, row_list_count, k, idx, dist, count, blocks, split_blocks, part_i, part_d, \
-                             done, row_map, st)
+                             done, row_map, st, seg_range)
     if (k <= 1) B200M_EXACT_CASE(1);
     if (k <= 2) B200M_EXACT_CASE(2);
     if (k <= 4) B200M_EXACT_CASE(4);

@@ -179,10 +179,19 @@ filter_scatter_kernel(FilterArgs a, size_t n_elems, const unsigned long long *__
 // neighbour contributes +0.0f, which leaves a non-negative (or non-finite) running sum unchanged bit for bit, so the
 // chain needs no predicate; the rows that do count are tallied on the side.  (The first version -- one warp, 32 shuffles
 // and predicated adds per 32 rows, loads not overlapped -- took ~6 ms for 500k rows; this one ~1.2 ms.)
+// segs != null (batch calls): CTA s runs the same chain over rows [segs[s].x, segs[s].x + segs[s].y) into avg[s].
 constexpr int kAvgChunk = 4096;
 constexpr int kAvgThreads = 256;
 __global__ void __launch_bounds__(kAvgThreads) average_kernel(const float *__restrict__ fdist, const int32_t *__restrict__ fcount,
-                                                              size_t n_rows, int k, float *__restrict__ avg) {
+                                                              size_t n_rows, int k, float *__restrict__ avg,
+                                                              const int2 *__restrict__ segs) {
+    if (segs) {
+        const int2 sg = segs[blockIdx.x];
+        fdist += (size_t) sg.x * k;
+        fcount += sg.x;
+        n_rows = (size_t) sg.y;
+        avg += blockIdx.x;
+    }
     __shared__ __align__(16) float buf[2][kAvgChunk];
     __shared__ unsigned long long n_with;
     const int tid = threadIdx.x;
@@ -294,7 +303,7 @@ cudaError_t launch_filter(int mode, int k, float ratio_thr, float distance_thr, 
         if (e != cudaSuccess) return e;
     }
     if (avg) {
-        average_kernel<<<1, kAvgThreads, 0, st>>>(fdist, fcount, n_rows, k, avg);
+        average_kernel<<<1, kAvgThreads, 0, st>>>(fdist, fcount, n_rows, k, avg, nullptr);
         *n_launches += 1;
     }
     return cudaGetLastError();
@@ -302,7 +311,14 @@ cudaError_t launch_filter(int mode, int k, float ratio_thr, float distance_thr, 
 
 cudaError_t launch_average(const float *fdist, const int32_t *fcount, size_t n_rows, int k, float *avg,
                            cudaStream_t st) {
-    average_kernel<<<1, kAvgThreads, 0, st>>>(fdist, fcount, n_rows, k, avg);
+    average_kernel<<<1, kAvgThreads, 0, st>>>(fdist, fcount, n_rows, k, avg, nullptr);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_average_segments(const float *fdist, const int32_t *fcount, const int2 *segs, int n_segs, int k, float *avg,
+                                    cudaStream_t st) {
+    if (n_segs <= 0) return cudaSuccess;
+    average_kernel<<<(unsigned) n_segs, kAvgThreads, 0, st>>>(fdist, fcount, 0, k, avg, segs);
     return cudaGetLastError();
 }
 

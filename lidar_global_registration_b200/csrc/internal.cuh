@@ -64,6 +64,7 @@ struct b200m_ctx {
     DevBuf ws_row_list, ws_row_flags, ws_sel_ops, ws_sel_norm;   // row selection (masked kNN)
     bool done_init = false;
     DevBuf ws_fidx, ws_fdist, ws_fcnt, ws_ridx, ws_rdist, ws_rcnt, ws_thr[2], ws_corr, ws_totals;
+    DevBuf ws_batch;       // batch calls (batch.cu): segment tables, per-pair bookkeeping and per-pair results
     bool totals_init = false;
     void *tmap_cache = nullptr;
     void *multiscale = nullptr;   // MultiscaleState (multiscale.cu)
@@ -120,6 +121,14 @@ struct StatTimer {
     void stop();
 };
 
+// A batch call's layout (batch.cu), per query direction: every pair's rows start at a multiple of B200M_TILE_N on both
+// sides, and range[query row / B200M_TILE_N] = {first, end} train row of that block's pair.  max_tiles: train tiles of the
+// largest segment.
+struct SegTable {
+    const int2 *range = nullptr;
+    int max_tiles = 0;
+};
+
 // ---- kernel launchers (one translation unit each) ---------------------------
 // pack.cu
 // dense FP32 copy + validity + per-CTA column statistics (sum, min, max over valid rows) into `stats`
@@ -139,7 +148,9 @@ cudaError_t launch_exact_rows(const float *q_f32, const uint8_t *q_valid, int dp
                               int split_blocks, int32_t *part_i, float *part_d, unsigned int *done,
                               // row_map (or null): the call's rows are row_map[0..n_rows) instead of row_begin + 0..n_rows;
                               // results are always stored at (row - row_begin)
-                              const int32_t *row_map, cudaStream_t st);
+                              const int32_t *row_map, cudaStream_t st,
+                              // seg_range (or null): query row qi only looks at train rows [seg_range[qi / 256].x, .y)
+                              const int2 *seg_range = nullptr);
 cudaError_t launch_local_rows(const float *q_f32, const uint8_t *q_valid, int dp, const float *t_f32,
                               const uint8_t *t_valid, size_t nt, int64_t t_index_offset, size_t n_rows,
                               const float *q_xyz, const float *t_xyz, size_t xyz_stride_bytes, float radius, int k,
@@ -168,6 +179,9 @@ cudaError_t launch_filter(int mode, int k, float ratio_thr, float distance_thr, 
 size_t filter_scan_ws_bytes(size_t n_rows, int k);
 cudaError_t launch_average(const float *fdist, const int32_t *fcount, size_t n_rows, int k, float *avg,
                            cudaStream_t st);
+// one average per segment: avg[s] over rows [segs[s].x, segs[s].x + segs[s].y) (one CTA per segment)
+cudaError_t launch_average_segments(const float *fdist, const int32_t *fcount, const int2 *segs, int n_segs, int k, float *avg,
+                                    cudaStream_t st);
 cudaError_t launch_merge(int k, int n_lists, size_t nq, const int32_t *idx_in, const float *dist_in,
                          const int32_t *count_in, int32_t *idx, float *dist, int32_t *count, cudaStream_t st);
 
@@ -180,7 +194,8 @@ cudaError_t launch_merge(int k, int n_lists, size_t nq, const int32_t *idx_in, c
 // rows row_begin.. of the query side's own array.
 int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows, int k, int cap_request,
                   int *n_lists_out, int *cap_out, int *has_values_out, float *dump, size_t dump_t_tile,
-                  const void *q_ops = nullptr, const float *q_norm = nullptr, size_t q_pad = 0);
+                  const void *q_ops = nullptr, const float *q_norm = nullptr, size_t q_pad = 0,
+                  const SegTable *seg = nullptr /* batch: every query block sweeps its own pair's train tiles only */);
 bool tc_supported(const b200m_ctx *ctx, int dim, int k);
 void tc_release(b200m_ctx *ctx);
 
@@ -213,8 +228,17 @@ int launch_local_cells(b200m_ctx *ctx, int direction, const float *d_query_xyz, 
 
 // api.cu: kNN of query rows [row_begin, row_begin + n_rows) of `direction` on device buffers; with d_flags only the flagged
 // (and valid) rows are answered, the others get empty lists.  Outputs are indexed by (row - row_begin).
+// With seg (batch calls, no flags) every query row is answered from its own pair's train rows only.
 extern "C" int b200m_knn_rows(b200m_ctx *ctx, const b200m_params *p, int direction, size_t row_begin, size_t n_rows, const uint8_t *d_flags,
-                   int32_t *d_idx, float *d_dist, int32_t *d_count);
+                   int32_t *d_idx, float *d_dist, int32_t *d_count, const SegTable *seg = nullptr);
+extern "C" {
+int check_params(b200m_ctx *ctx, const b200m_params *p);
+int check_upload_args(b200m_ctx *ctx, int side, const float *base, size_t n, size_t stride_bytes, int dim);
+bool is_pageable(const void *p);
+int staged_h2d(b200m_ctx *ctx, void *dst, const void *src, size_t bytes);   // pageable host -> device through pinned buffers
+// pack `n` rows of device AoS data into side `side` (b200m_upload's device half)
+int upload_common(b200m_ctx *ctx, int side, const float *device_aos, size_t n, size_t stride_bytes, int dim, int64_t index_offset);
+}
 
 // cluster.cu
 void cluster_release(b200m_ctx *ctx);

@@ -51,6 +51,11 @@ class _Scale(C.Structure):
                 ("tgt_desc", C.c_void_p), ("n_tgt", C.c_size_t), ("tgt_map", C.c_void_p)]
 
 
+class _Pair(C.Structure):
+    """b200m_pair: one (source, target) pair of a batch call (host pointers)."""
+    _fields_ = [("src", C.c_void_p), ("n_src", C.c_size_t), ("tgt", C.c_void_p), ("n_tgt", C.c_size_t)]
+
+
 class Stats(C.Structure):
     _fields_ = [("ms_pack", C.c_double), ("ms_prepare", C.c_double), ("ms_candidates", C.c_double),
                 ("ms_rerank", C.c_double), ("ms_fallback", C.c_double), ("ms_filter", C.c_double),
@@ -71,7 +76,8 @@ EXPORTS = ["b200m_create", "b200m_destroy", "b200m_last_error", "b200m_set_strea
            "b200m_match_multiscale", "b200m_comm_unique_id", "b200m_comm_attach", "b200m_comm_rank", "b200m_shard_rows",
            "b200m_upload_replicated", "b200m_match_sharded", "b200m_match_sharded_device", "b200m_knn_target_sharded_device",
            "b200m_create_multi", "b200m_destroy_multi", "b200m_group_last_error", "b200m_group_size", "b200m_group_ctx",
-           "b200m_group_upload", "b200m_group_upload_sharded", "b200m_group_match", "b200m_group_knn"]
+           "b200m_group_upload", "b200m_group_upload_sharded", "b200m_group_match", "b200m_group_knn", "b200m_knn_batch",
+           "b200m_match_batch"]
 
 _lib = None
 
@@ -139,6 +145,9 @@ def load_library():
     L.b200m_group_upload_sharded.argtypes = [vp, C.c_int, fp, sz, sz, C.c_int]
     L.b200m_group_match.argtypes = [vp, C.POINTER(_Params), fp, fp, vp, sz, C.POINTER(sz), C.POINTER(C.c_float)]
     L.b200m_group_knn.argtypes = [vp, C.POINTER(_Params), vp, vp, vp]
+    L.b200m_knn_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Pair), C.c_int, sz, C.c_int, vp, vp, vp]
+    L.b200m_match_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Pair), C.c_int, sz, C.c_int, fp, fp, vp, sz,
+                                    C.POINTER(sz), vp]
     L.b200m_version.restype = C.c_int
     L.b200m_debug_operands.argtypes = [vp, C.c_int, C.c_int, vp, sz, vp, C.POINTER(C.c_float), C.POINTER(i32),
                                        C.POINTER(i64)]
@@ -330,6 +339,72 @@ class Context:
         v = C.c_void_p
         self._ck(self._L.b200m_mark_referenced_device(self._h, k, v(fidx_ptr), v(fcnt_ptr), n_rows, index_offset, v(flags_ptr),
                                                       n_flags))
+
+    # -- batches: many (source, target) pairs in one call -------------------------------------
+    @staticmethod
+    def _pairs(pairs, dim):
+        """-> (the contiguous float32 arrays to keep alive, b200m_pair array, stride_bytes, source row counts)."""
+        keep, width = [], None
+        arr = (_Pair * max(len(pairs), 1))()
+        for i, (s, t) in enumerate(pairs):
+            s, t = np.ascontiguousarray(s, np.float32), np.ascontiguousarray(t, np.float32)
+            if s.ndim != 2 or t.ndim != 2 or s.shape[1] != t.shape[1] or (width is not None and s.shape[1] != width):
+                raise B200MatchError("batch: every set must be a 2-D float32 array [n, stride_floats] of one row length")
+            width = s.shape[1]
+            keep += [s, t]
+            arr[i] = _Pair(s.ctypes.data if s.shape[0] else None, s.shape[0], t.ctypes.data if t.shape[0] else None, t.shape[0])
+        if width is not None and dim > width:
+            raise B200MatchError("dim exceeds the row length")
+        return keep, arr, 4 * (width or dim), [int(s.shape[0]) for s, _ in pairs]
+
+    def _batch_sides(self, pairs):
+        # what the library's two sides hold after a batch call: every set padded to a multiple of 256 rows
+        self.n = [sum(-(-len(pr[s]) // 256) * 256 for pr in pairs) for s in (0, 1)]
+
+    def knn_batch(self, k, pairs, dim, precision=PREC_TC_F16, cand_cap=0):
+        """b200m_knn_batch: `pairs` = [(source rows, target rows), ...] (float32 [n, stride_floats], one row length).
+        Returns one (idx, dist, count) per pair, each equal to upload + knn(k, 0) on that pair alone.  Replaces the sets
+        uploaded before."""
+        keep, arr, stride, ns = self._pairs(pairs, dim)
+        total = sum(ns)
+        idx = np.empty((total, k), np.int32)
+        dist = np.empty((total, k), np.float32)
+        cnt = np.empty((total,), np.int32)
+        p = self._params(k, MODE_KNN_ONLY, precision=precision, cand_cap=cand_cap)
+        self._ck(self._L.b200m_knn_batch(self._h, C.byref(p), arr, len(pairs), stride, dim, idx.ctypes.data, dist.ctypes.data,
+                                         cnt.ctypes.data))
+        self._batch_sides(pairs)
+        off = np.concatenate([[0], np.cumsum(ns)]).astype(np.int64)
+        return [(idx[a:b], dist[a:b], cnt[a:b]) for a, b in zip(off[:-1], off[1:])]
+
+    def match_batch(self, k, mode, pairs, dim, ratio_thr=MATCHING_RATIO_THRESHOLD, distance_thr=FLT_MAX, thr_src=None,
+                    thr_tgt=None, precision=PREC_TC_F16, cand_cap=0):
+        """b200m_match_batch: returns one (correspondences as CORR_DTYPE array, average first-NN distance) per pair, each
+        equal to upload + match on that pair alone (pair-local indices).  thr_src / thr_tgt: None or one threshold array per
+        pair.  Replaces the sets uploaded before."""
+        keep, arr, stride, ns = self._pairs(pairs, dim)
+        if (thr_src is None) != (thr_tgt is None):
+            raise B200MatchError("give both threshold lists or neither")
+        ts = tt = None
+        if thr_src is not None:
+            if len(thr_src) != len(pairs) or len(thr_tgt) != len(pairs):
+                raise B200MatchError("one threshold array per pair and side")
+            for i, (s, t) in enumerate(pairs):
+                if len(thr_src[i]) != len(s) or len(thr_tgt[i]) != len(t):
+                    raise B200MatchError("pair %d: threshold array length != number of rows" % i)
+            ts = np.concatenate([np.asarray(a, np.float32).ravel() for a in thr_src] + [np.zeros(1, np.float32)])
+            tt = np.concatenate([np.asarray(a, np.float32).ravel() for a in thr_tgt] + [np.zeros(1, np.float32)])
+        kk = k if mode == MODE_MUTUAL else 1
+        out = np.empty(max(sum(ns) * kk, 1), CORR_DTYPE)
+        offsets = np.zeros(len(pairs) + 1, np.uint64)
+        avg = np.empty(max(len(pairs), 1), np.float32)
+        p = self._params(k, mode, ratio_thr, distance_thr, precision, cand_cap)
+        self._ck(self._L.b200m_match_batch(self._h, C.byref(p), arr, len(pairs), stride, dim,
+                                           None if ts is None else ts.ctypes.data, None if tt is None else tt.ctypes.data,
+                                           out.ctypes.data, out.shape[0], offsets.ctypes.data_as(C.POINTER(C.c_size_t)),
+                                           avg.ctypes.data))
+        self._batch_sides(pairs)
+        return [(out[int(offsets[i]):int(offsets[i + 1])], float(avg[i])) for i in range(len(pairs))]
 
     # -- whole matcher call ----------------------------------------------------
     def match(self, k, mode, ratio_thr=MATCHING_RATIO_THRESHOLD, distance_thr=FLT_MAX, thr_src=None, thr_tgt=None,
