@@ -345,6 +345,36 @@ B200M_API int b200m_match_multiscale(b200m_ctx *ctx, const b200m_params *p, cons
                                      const float *thr_tgt, b200m_corr *out, size_t cap, size_t *n_out,
                                      float *avg_first_dist);
 
+/* ---- the matcher classes at the WIDE seam, many (source, target) cloud pairs in one call ------------------------------
+ * b200m_match_multiscale of every pair: multi-view registration, one scan against many submaps or an evaluation table
+ * run their OneSided / LeftToRight / ClusterMatcher calls as one batch.  Pair p's records and average equal, byte for
+ * byte, what b200m_match_multiscale returns for pair p alone (with pair-local keypoint ids), the masked reverse pass
+ * included (its output is the same).  All pairs share the descriptor type (stride_bytes, dim), the keypoint row stride,
+ * the params and cluster_k; each pair has its own scales (its common scales, ascending; 0..32 of them, n_scales * k <=
+ * 128), keypoint coordinates and radii.  The validation rules per pair are b200m_match_multiscale's; an error names the
+ * pair (and the scale).  A pair without source keypoints or without scales gives no records and the average FLT_MAX.
+ * Per scale the pairs' descriptor sets are packed as b200m_match_batch packs them and answered by one kNN pass per
+ * direction; the votes, the filter and the 3-D neighbourhoods of the cluster filter run once over all pairs, each pair's
+ * neighbourhoods inside its own keypoints.
+ * Outputs as b200m_match_batch's: records of pair p are out[offsets[p] .. offsets[p+1]) (at most n_src_kps each;
+ * offsets has n_pairs + 1 entries and is filled also when cap is too small), avg (may be NULL) gets n_pairs averages,
+ * thr_src / thr_tgt are the pairs' per-keypoint thresholds concatenated in pair order (sum n_src_kps / sum n_tgt_kps
+ * floats) or both NULL.  Like the other batch calls, this call REPLACES the descriptor sets b200m_upload put in the
+ * context.  Host pointers. */
+typedef struct {
+    const b200m_scale *scales;   /* this pair's common scales, ascending; n_scales in [0, 32] */
+    int n_scales;
+    const float *src_kps_xyz;    /* n_src_kps rows, xyz_stride_bytes apart (may be NULL in ONE_SIDED mode) */
+    size_t n_src_kps;
+    const float *tgt_kps_xyz;
+    size_t n_tgt_kps;
+    float iss_radius_src, iss_radius_tgt;
+} b200m_wide_pair;
+B200M_API int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs, int n_pairs,
+                                           size_t stride_bytes, int dim, size_t xyz_stride_bytes, int cluster_k,
+                                           const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
+                                           size_t *offsets, float *avg);
+
 B200M_API int b200m_version(void);
 
 /* ---- test hooks (used by tests/ only; not part of the reference-facing surface) ----

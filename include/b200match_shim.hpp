@@ -10,6 +10,7 @@
 //   FeatureBasedMatcher, FeatureBasedMatcherImpl<FeatureT>::Storage, OneSidedMatcher / LeftToRightMatcher /
 //   RatioMatcher / ClusterMatcher  (match(), getAverageDistance(), getClassName())
 //                                  reference include/matching.h:25-42, :96-161, :385-551
+//   matchMany<FeatureT>            match() of many OneSided / LeftToRight / ClusterMatchers (cloud pairs) in one call
 // The matcher classes run match_impl as the reference composes it -- match_multiscale (per-scale kNN, spatial vote ->
 // at most one match per keypoint) in one or both directions, then the filter over the voted lists -- in ONE library
 // call (b200m_match_multiscale); the narrow-seam functions share one context per host thread and device, so calling
@@ -421,22 +422,25 @@ public:
         : st_src_(std::move(src)), st_tgt_(std::move(tgt)), parameters_(std::move(parameters)) {}
 
     // match() (reference include/matching.h:148-161): match_impl + finalize
-    CorrespondencesPtr match() override {
-        auto correspondences = match_impl();
-        for (auto &c : *correspondences) {   // finalize (:356-362)
+    CorrespondencesPtr match() override { return finalize(match_impl()); }
+
+    template <typename F>
+    friend std::vector<CorrespondencesPtr> matchMany(const std::vector<std::shared_ptr<FeatureBasedMatcherImpl<F>>> &matchers);
+
+protected:
+    virtual int mode() const = 0;
+
+    // finalize (reference :356-362): keypoint ids -> indices in the clouds
+    CorrespondencesPtr finalize(CorrespondencesPtr correspondences) const {
+        for (auto &c : *correspondences) {
             if (!st_src_.kps_indices.empty()) c.index_query = st_src_.kps_indices[c.index_query];
             if (!st_tgt_.kps_indices.empty()) c.index_match = st_tgt_.kps_indices[c.index_match];
         }
         return correspondences;
     }
 
-protected:
-    virtual int mode() const = 0;
-
-    // match_impl of the three implemented matchers: both match_multiscale calls, the vote, printDebugInfo's average
-    // and the filter loop in one device-resident call
-    virtual CorrespondencesPtr match_impl() {
-        // the scales common to both clouds (reference :268-270)
+    // the scales common to both clouds (reference :268-270) as the library's per-scale rows; *lo = the first one's log2 radius
+    std::vector<b200m_scale> commonScales(int *lo_out = nullptr) const {
         const int lo = std::max(st_src_.min_log2_radius, st_tgt_.min_log2_radius);
         const int hi = std::min(st_src_.max_log2_radius, st_tgt_.max_log2_radius);
         if (hi < lo) throw std::runtime_error("the two clouds have no scale in common");
@@ -461,20 +465,37 @@ protected:
             }
             scales.push_back(sc);
         }
-        // one candidate per keypoint (randomness 1, one scale): the vote is the identity and needs no coordinates
-        std::vector<float> zeros;
-        const float *sx = st_src_.kps_xyz, *tx = st_tgt_.kps_xyz;
-        size_t stride = st_src_.kps_stride_bytes;
-        if (!sx || !tx) {
-            if (parameters_.randomness != 1 || scales.size() != 1 || mode() == B200M_MODE_CLUSTER)
+        if (lo_out) *lo_out = lo;
+        return scales;
+    }
+
+    // the keypoint coordinates of both clouds; one candidate per keypoint (randomness 1, one scale): the vote is the identity
+    // and needs none, `zeros` stands in for them
+    void keypointRows(size_t n_scales, std::vector<float> &zeros, const float **sx, const float **tx, size_t *stride) const {
+        *sx = st_src_.kps_xyz;
+        *tx = st_tgt_.kps_xyz;
+        *stride = st_src_.kps_stride_bytes;
+        if (!*sx || !*tx) {
+            if (parameters_.randomness != 1 || n_scales != 1 || mode() == B200M_MODE_CLUSTER)
                 throw std::runtime_error("randomness * scales > 1 (or the cluster filter) needs the keypoint coordinates of both clouds: "
                                          "match_multiscale's spatial vote keeps one match per keypoint (include/matching.h:327-352)");
             zeros.assign(4 * std::max(st_src_.n_kps, st_tgt_.n_kps) + 4, 0.f);
-            sx = tx = zeros.data();
-            stride = 16;
+            *sx = *tx = zeros.data();
+            *stride = 16;
         } else if (st_src_.kps_stride_bytes != st_tgt_.kps_stride_bytes) {
             throw std::runtime_error("both keypoint clouds must have the same point stride");
         }
+    }
+
+    // match_impl of the three implemented matchers: both match_multiscale calls, the vote, printDebugInfo's average
+    // and the filter loop in one device-resident call
+    virtual CorrespondencesPtr match_impl() {
+        int lo = 0;
+        std::vector<b200m_scale> scales = commonScales(&lo);
+        std::vector<float> zeros;
+        const float *sx, *tx;
+        size_t stride;
+        keypointRows(scales.size(), zeros, &sx, &tx, &stride);
         const bool thr = !st_src_.thresholds.empty() && !st_tgt_.thresholds.empty();
         b200m_params p = make_params(parameters_, mode(), parameters_.randomness);
         auto out = std::make_shared<Correspondences>(st_src_.n_kps);
@@ -562,6 +583,80 @@ protected:
         return out;
     }
 };
+
+// match() of many OneSided / LeftToRight / ClusterMatchers in one library call (b200m_match_multiscale_batch): multi-view
+// registration, one scan against many submaps, an evaluation table.  All matchers must be of one class with the same
+// parameters and keypoint point stride; each pair's common scales are built as match_impl builds them.  result[i] equals
+// matchers[i]->match(), finalize included, and matchers[i]->getAverageDistance() is set.  One GPU only.
+inline bool sameParameters(const AlignmentParameters &a, const AlignmentParameters &b) {
+    return a.use_bfmatcher == b.use_bfmatcher && a.bf_block_size == b.bf_block_size && a.ratio_k == b.ratio_k &&
+           a.cluster_k == b.cluster_k && a.randomness == b.randomness && a.distance_thr == b.distance_thr &&
+           a.matching_id == b.matching_id && a.ratio_thr == b.ratio_thr && a.match_search_radius == b.match_search_radius &&
+           a.device == b.device && a.devices == b.devices && a.precision == b.precision;
+}
+
+template <typename FeatureT>
+std::vector<CorrespondencesPtr> matchMany(const std::vector<std::shared_ptr<FeatureBasedMatcherImpl<FeatureT>>> &matchers) {
+    std::vector<CorrespondencesPtr> result;
+    if (matchers.empty()) return result;
+    const FeatureBasedMatcherImpl<FeatureT> &m0 = *matchers[0];
+    const AlignmentParameters &pa = m0.parameters_;
+    const int mode = m0.mode();
+    if (mode != B200M_MODE_ONE_SIDED && mode != B200M_MODE_MUTUAL && mode != B200M_MODE_CLUSTER)
+        throw std::runtime_error("matchMany: OneSided, LeftToRight and ClusterMatchers only (RatioMatcher: matchBatch)");
+    const size_t n = matchers.size();
+    std::vector<std::vector<b200m_scale>> scales(n);
+    std::vector<std::vector<float>> zeros(n);
+    std::vector<b200m_wide_pair> pairs(n);
+    std::vector<float> thr_src, thr_tgt;
+    bool thr = false;
+    size_t stride = 0, n_src = 0;
+    for (size_t i = 0; i < n; ++i) {
+        const FeatureBasedMatcherImpl<FeatureT> &m = *matchers[i];
+        if (m.mode() != mode || matchers[i]->getClassName() != matchers[0]->getClassName() || !sameParameters(m.parameters_, pa))
+            throw std::runtime_error("matchMany: every matcher must be of one class with the same AlignmentParameters");
+        if (m.parameters_.devices.size() > 1) throw std::runtime_error("matchMany: one GPU only (parameters.devices has several)");
+        scales[i] = m.commonScales();
+        const float *sx, *tx;
+        size_t st;
+        m.keypointRows(scales[i].size(), zeros[i], &sx, &tx, &st);
+        if (i && st != stride) throw std::runtime_error("matchMany: every keypoint cloud must have the same point stride");
+        stride = st;
+        pairs[i] = b200m_wide_pair{scales[i].data(), (int) scales[i].size(), sx, m.st_src_.n_kps, tx, m.st_tgt_.n_kps,
+                                   m.st_src_.iss_radius, m.st_tgt_.iss_radius};
+        thr = thr || (!m.st_src_.thresholds.empty() && !m.st_tgt_.thresholds.empty());
+        n_src += m.st_src_.n_kps;
+    }
+    if (thr) {   // a matcher without thresholds gets +inf ones: min(max(inf, .), distance_thr) = distance_thr, as with none
+        for (size_t i = 0; i < n; ++i) {
+            const FeatureBasedMatcherImpl<FeatureT> &m = *matchers[i];
+            const bool own = !m.st_src_.thresholds.empty() && !m.st_tgt_.thresholds.empty();
+            const float inf = std::numeric_limits<float>::infinity();
+            if (own) {
+                thr_src.insert(thr_src.end(), m.st_src_.thresholds.begin(), m.st_src_.thresholds.begin() + m.st_src_.n_kps);
+                thr_tgt.insert(thr_tgt.end(), m.st_tgt_.thresholds.begin(), m.st_tgt_.thresholds.begin() + m.st_tgt_.n_kps);
+            } else {
+                thr_src.insert(thr_src.end(), m.st_src_.n_kps, inf);
+                thr_tgt.insert(thr_tgt.end(), m.st_tgt_.n_kps, inf);
+            }
+        }
+        thr_src.push_back(0.f);
+        thr_tgt.push_back(0.f);
+    }
+    b200m_params p = make_params(pa, mode, pa.randomness);
+    Correspondences all(std::max<size_t>(n_src, 1));
+    std::vector<size_t> offsets(n + 1);
+    std::vector<float> avg(n);
+    Context &ctx = shared_context(pa.device);
+    ctx.check(b200m_match_multiscale_batch(ctx.get(), &p, pairs.data(), (int) n, sizeof(FeatureT), feature_dim<FeatureT>(), stride,
+                                           pa.cluster_k, thr ? thr_src.data() : nullptr, thr ? thr_tgt.data() : nullptr,
+                                           reinterpret_cast<b200m_corr *>(all.data()), all.size(), offsets.data(), avg.data()));
+    for (size_t i = 0; i < n; ++i) {
+        matchers[i]->average_distance_ = avg[i];
+        result.push_back(matchers[i]->finalize(std::make_shared<Correspondences>(all.begin() + offsets[i], all.begin() + offsets[i + 1])));
+    }
+    return result;
+}
 
 // getFeatureBasedMatcherFromParameters (reference src/matching.cpp:21-76) for one feature type.
 template <typename FeatureT>

@@ -161,6 +161,7 @@ void b200m_destroy(b200m_ctx *ctx) {
     multiscale_release(ctx);
     cluster_release(ctx);
     wide_release(ctx);
+    wide_batch_release(ctx);
     comm_release(ctx);
     local_release(ctx);
     stage_release(ctx);

@@ -34,23 +34,6 @@
 
 namespace {
 
-// per pair: {first source row, first target row, source rows, first row of the pair in the dense k-list output}
-struct BatchLayout {
-    size_t n_rows[2] = {0, 0};   // padded rows per side
-    size_t real_src = 0;         // sum of the pairs' source rows
-    SegTable seg[2];             // per query direction
-    const int32_t *block_pair = nullptr;   // [source rows / 256] pair of that source block
-    const int4 *pair_info = nullptr;       // [n_pairs]
-    const int2 *avg_segs = nullptr;        // [n_pairs] {first source row, source rows}
-    unsigned long long *n_out = nullptr;   // result area: record count, then per-pair counts and averages
-    unsigned *counts = nullptr;
-    float *avgs = nullptr;
-    size_t result_bytes = 0;
-};
-
-inline size_t pad_rows(size_t n) { return (n + B200M_TILE_N - 1) / B200M_TILE_N * B200M_TILE_N; }
-inline size_t align16(size_t b) { return (b + 15) & ~(size_t) 15; }
-
 __global__ void localize_lists_kernel(const int32_t *__restrict__ idx, const float *__restrict__ dist,
                                       const int32_t *__restrict__ cnt, size_t n_rows, int k,
                                       const int32_t *__restrict__ block_pair, const int4 *__restrict__ pair_info,
@@ -85,6 +68,8 @@ __global__ void localize_records_kernel(b200m_corr *__restrict__ rec, const unsi
         if ((int) (threadIdx.x & 31) == __ffs((int) peers) - 1) atomicAdd(counts + p, (unsigned) __popc(peers));
     }
 }
+
+}  // namespace
 
 // Validates the batch, packs both sides in the padded layout (replacing what b200m_upload put in the context) and
 // uploads the segment tables.
@@ -177,8 +162,6 @@ int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b20
     }
     return 0;
 }
-
-}  // namespace
 
 extern "C" {
 

@@ -22,8 +22,13 @@ constexpr int kMaxClusterK = 64;
 
 __device__ __forceinline__ bool lex_less(float d1, int i1, float d2, int i2) { return d1 < d2 || (d1 == d2 && i1 < i2); }
 
+// SEG (batch calls): the points of many pairs back to back, seg_off[p] = first point of pair p; point i only scans its own
+// pair's points [seg_off[p], seg_off[p + 1]) and reports global ids.  A compile-time flag, so the single-pair instantiation
+// is the kernel it was.
+template <bool SEG>
 __global__ void __launch_bounds__(kKnn3dWarps * 32)
-knn3d_kernel(const float *__restrict__ xyz, size_t stride_floats, size_t n, int k, int32_t *__restrict__ nbr) {
+knn3d_kernel(const float *__restrict__ xyz, size_t stride_floats, size_t n, int k, int32_t *__restrict__ nbr,
+             const int32_t *__restrict__ seg_off = nullptr, int n_seg = 0) {
     __shared__ float s_d[kKnn3dWarps][kMaxClusterK];
     __shared__ int s_i[kKnn3dWarps][kMaxClusterK];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -36,15 +41,21 @@ knn3d_kernel(const float *__restrict__ xyz, size_t stride_floats, size_t n, int 
         const float ax = xyz[i * stride_floats], ay = xyz[i * stride_floats + 1], az = xyz[i * stride_floats + 2];
         float tau_d = INFINITY;
         int tau_i = INT_MAX;
-        for (size_t base = 0; base < n; base += 32) {
+        size_t first = 0, end = n;
+        if constexpr (SEG) {
+            const int p = pair_of(seg_off, n_seg, (long long) i);
+            first = (size_t) seg_off[p];
+            end = (size_t) seg_off[p + 1];
+        }
+        for (size_t base = first; base < end; base += 32) {
             const size_t j = base + lane;
             float d = INFINITY;
-            if (j < n) {
+            if (j < end) {
                 const float *b = xyz + j * stride_floats;
                 const float dx = __fsub_rn(ax, b[0]), dy = __fsub_rn(ay, b[1]), dz = __fsub_rn(az, b[2]);
                 d = __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
             }
-            unsigned mask = __ballot_sync(0xffffffffu, j < n && lex_less(d, (int) j, tau_d, tau_i));
+            unsigned mask = __ballot_sync(0xffffffffu, j < end && lex_less(d, (int) j, tau_d, tau_i));
             while (mask) {
                 const int b = __ffs((int) mask) - 1;
                 mask &= mask - 1;
@@ -136,6 +147,48 @@ void cluster_release(b200m_ctx *ctx) {
     ctx->cluster = nullptr;
 }
 
+int cluster_filter_batch_device(b200m_ctx *ctx, const b200m_params *p, int cluster_k, float cluster_thr, size_t n_src, size_t n_tgt,
+                                const int32_t *d_fidx, const float *d_fdist, const int32_t *d_fcount, const int32_t *d_ridx,
+                                const int32_t *d_rcount, const float *d_src_xyz, const float *d_tgt_xyz, size_t xyz_stride_bytes,
+                                const int32_t *d_src_off, const int32_t *d_tgt_off, int n_pairs, const float *d_thr_src,
+                                const float *d_thr_tgt, b200m_corr *d_out, size_t cap, unsigned long long *d_n_out) {
+    if (cluster_k < 1 || cluster_k > kMaxClusterK) return b200m_fail_msg(ctx, "b200m_cluster_filter: cluster_k must be in [1, 64]");
+    const int k = p->k;
+    ClusterState *cs = cl_state(ctx);
+    cudaStream_t st = ctx->stream;
+    if (n_src == 0 || n_tgt == 0) {
+        CK(cudaMemsetAsync(d_n_out, 0, sizeof(unsigned long long), st));
+        return 0;
+    }
+    CK(cs->nbr_src.reserve(sizeof(int32_t) * n_src * cluster_k));
+    CK(cs->nbr_tgt.reserve(sizeof(int32_t) * n_tgt * cluster_k));
+    CK(cs->cdist.reserve(sizeof(float) * n_src * k));
+    StatTimer t(ctx, &ctx->stats.ms_filter);
+    const size_t cap_blocks = (size_t) ctx->sm_count * 8;
+    const size_t ns[2] = {n_src, n_tgt};
+    const float *xyz[2] = {d_src_xyz, d_tgt_xyz};
+    const int32_t *off[2] = {d_src_off, d_tgt_off};
+    int32_t *nbr[2] = {cs->nbr_src.as<int32_t>(), cs->nbr_tgt.as<int32_t>()};
+    for (int s = 0; s < 2; ++s) {
+        const size_t want = (ns[s] + kKnn3dWarps - 1) / kKnn3dWarps;
+        knn3d_kernel<true><<<(unsigned) (want < cap_blocks ? want : cap_blocks), kKnn3dWarps * 32, 0, st>>>(
+            xyz[s], xyz_stride_bytes / 4, ns[s], cluster_k, nbr[s], off[s], n_pairs);
+        CK(cudaGetLastError());
+    }
+    const size_t n_elems = n_src * (size_t) k;
+    cluster_dist_kernel<<<(unsigned) ((n_elems + 127) / 128), 128, 0, st>>>(
+        n_src, n_tgt, k, cluster_k, cluster_thr, d_fidx, d_fcount, d_ridx, d_rcount, nbr[0], nbr[1], cs->cdist.as<float>());
+    CK(cudaGetLastError());
+    CK(ctx->ws_scan.reserve(filter_scan_ws_bytes(n_src, k)));
+    int launches = 3;
+    CK(launch_filter(B200M_MODE_CLUSTER, k, p->ratio_thr, p->distance_thr, 0, n_src, d_fidx, d_fdist, d_fcount, nullptr, nullptr,
+                     nullptr, 0, d_thr_src, d_thr_tgt, 0, 0, d_out, cap, d_n_out, nullptr, ctx->ws_scan.p, ctx->ws_scan.cap, st,
+                     &launches, cs->cdist.as<float>()));
+    ctx->stats.launches += launches;
+    t.stop();
+    return 0;
+}
+
 extern "C" {
 
 int b200m_knn3d_device(b200m_ctx *ctx, const float *d_xyz, size_t n, size_t xyz_stride_bytes, int k, int32_t *d_nbr) {
@@ -146,7 +199,7 @@ int b200m_knn3d_device(b200m_ctx *ctx, const float *d_xyz, size_t n, size_t xyz_
     if (n == 0) return 0;
     if (!d_xyz || !d_nbr) return b200m_fail_msg(ctx, "b200m_knn3d: null pointer");
     size_t want = (n + kKnn3dWarps - 1) / kKnn3dWarps, cap = (size_t) ctx->sm_count * 8;
-    knn3d_kernel<<<(unsigned) (want < cap ? want : cap), kKnn3dWarps * 32, 0, ctx->stream>>>(d_xyz, xyz_stride_bytes / 4, n, k, d_nbr);
+    knn3d_kernel<false><<<(unsigned) (want < cap ? want : cap), kKnn3dWarps * 32, 0, ctx->stream>>>(d_xyz, xyz_stride_bytes / 4, n, k, d_nbr);
     CK(cudaGetLastError());
     ctx->stats.launches += 1;
     return 0;

@@ -70,6 +70,7 @@ struct b200m_ctx {
     void *multiscale = nullptr;   // MultiscaleState (multiscale.cu)
     void *cluster = nullptr;      // ClusterState (cluster.cu)
     void *wide = nullptr;         // WideState (wide.cu)
+    void *wide_batch = nullptr;   // WideBatchState (wide_batch.cu)
     void *comm = nullptr;         // Comm (multi.cu): this context's rank in an NCCL communicator
     void *local = nullptr;        // LocalState (local.cu): the cell list of the gated kNN
     void *stage = nullptr;        // StagePool (api.cu): pinned bounce buffers for uploads from pageable host memory
@@ -128,6 +129,28 @@ struct SegTable {
     const int2 *range = nullptr;
     int max_tiles = 0;
 };
+
+inline size_t pad_rows(size_t n) { return (n + B200M_TILE_N - 1) / B200M_TILE_N * B200M_TILE_N; }
+inline size_t align16(size_t b) { return (b + 15) & ~(size_t) 15; }
+
+// batch.cu: what stage_batch leaves on the device.  Pair p's rows start at the sum of pad_rows() of the pairs before it.
+// pair_info[p] = {first source row, first target row, source rows, first row of the pair in the dense k-list output}
+struct BatchLayout {
+    size_t n_rows[2] = {0, 0};   // padded rows per side
+    size_t real_src = 0;         // sum of the pairs' source rows
+    SegTable seg[2];             // per query direction
+    const int32_t *block_pair = nullptr;   // [source rows / 256] pair of that source block
+    const int4 *pair_info = nullptr;       // [n_pairs]
+    const int2 *avg_segs = nullptr;        // [n_pairs] {first source row, source rows}
+    unsigned long long *n_out = nullptr;   // result area: record count, then per-pair counts and averages
+    unsigned *counts = nullptr;
+    float *avgs = nullptr;
+    size_t result_bytes = 0;
+};
+// Validates the pairs, packs both sides in the padded layout (replacing what b200m_upload put in the context) and uploads
+// the segment tables into ctx->ws_batch.
+int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                size_t stride_bytes, int dim, BatchLayout *L);
 
 // ---- kernel launchers (one translation unit each) ---------------------------
 // pack.cu
@@ -214,8 +237,16 @@ int ms_add_device(b200m_ctx *ctx, MultiscaleState *ms, int scale, size_t n_rows,
 int ms_vote_device(b200m_ctx *ctx, MultiscaleState *ms, const float *d_train_xyz, size_t xyz_stride_bytes, float iss_radius,
                    int32_t *d_idx, float *d_dist, int32_t *d_count);
 
+// Batch form of ms_vote_device (used by wide_batch.cu): the query keypoints of all pairs back to back, train ids global over the
+// concatenated train keypoints; query keypoint i belongs to pair p with kp_off[p] <= i < kp_off[p + 1] and votes with
+// radii[p].
+int ms_vote_batch_device(b200m_ctx *ctx, MultiscaleState *ms, const float *d_train_xyz, size_t xyz_stride_bytes,
+                         const int32_t *d_kp_off, int n_pairs, const float *d_radii, int32_t *d_idx, float *d_dist,
+                         int32_t *d_count);
+
 // wide.cu
 void wide_release(b200m_ctx *ctx);
+void wide_batch_release(b200m_ctx *ctx);
 
 // multi.cu
 void comm_release(b200m_ctx *ctx);
@@ -242,3 +273,19 @@ int upload_common(b200m_ctx *ctx, int side, const float *device_aos, size_t n, s
 
 // cluster.cu
 void cluster_release(b200m_ctx *ctx);
+// b200m_cluster_filter_device over many pairs' keypoints back to back (used by wide_batch.cu): the 3-D neighbourhoods stay inside a
+// keypoint's own pair (src_off / tgt_off: [n_pairs + 1] first keypoint of every pair and the total), every id is global.
+int cluster_filter_batch_device(b200m_ctx *ctx, const b200m_params *p, int cluster_k, float cluster_thr, size_t n_src, size_t n_tgt,
+                                const int32_t *d_fidx, const float *d_fdist, const int32_t *d_fcount, const int32_t *d_ridx,
+                                const int32_t *d_rcount, const float *d_src_xyz, const float *d_tgt_xyz, size_t xyz_stride_bytes,
+                                const int32_t *d_src_off, const int32_t *d_tgt_off, int n_pairs, const float *d_thr_src,
+                                const float *d_thr_tgt, b200m_corr *d_out, size_t cap, unsigned long long *d_n_out);
+__device__ __forceinline__ int pair_of(const int32_t *__restrict__ off, int n_pairs, long long i) {
+    // the last pair p with off[p] <= i (empty pairs share their offset with the next one)
+    int lo = 0, hi = n_pairs;   // off[lo] <= i < off[hi]
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (off[mid] <= i) lo = mid; else hi = mid;
+    }
+    return lo;
+}

@@ -42,12 +42,18 @@ __global__ void ms_scatter_kernel(size_t n_rows, int k, int scale, int n_scales,
 
 constexpr int kMaxVoteCands = 128;
 
+// SEG (batch calls, wide_batch.cu): the query keypoints of many pairs back to back, iss_radius = radii[pair of kp].  A
+// compile-time flag, so the single-pair instantiation is the kernel it was.
+template <bool SEG>
 __global__ void ms_vote_kernel(size_t n_query_kps, int n_scales, int k, const int32_t *__restrict__ s_idx,
                                const float *__restrict__ s_dist, const int32_t *__restrict__ s_cnt,
                                const float *__restrict__ xyz, size_t xyz_stride_floats, float iss_radius,
-                               int32_t *__restrict__ out_idx, float *__restrict__ out_dist, int32_t *__restrict__ out_cnt) {
+                               int32_t *__restrict__ out_idx, float *__restrict__ out_dist, int32_t *__restrict__ out_cnt,
+                               const int32_t *__restrict__ kp_off = nullptr, int n_pairs = 0,
+                               const float *__restrict__ radii = nullptr) {
     const size_t kp = (size_t) blockIdx.x * blockDim.x + threadIdx.x;
     if (kp >= n_query_kps) return;
+    if constexpr (SEG) iss_radius = radii[pair_of(kp_off, n_pairs, (long long) kp)];
     // candidate m of the concatenated list = m-th entry when the scales' lists are walked in order
     const int32_t *ci = s_idx + kp * (size_t) n_scales * k;
     const float *cd = s_dist + kp * (size_t) n_scales * k;
@@ -159,9 +165,21 @@ int ms_vote_device(b200m_ctx *ctx, MultiscaleState *ms, const float *d_train_xyz
         return b200m_fail_msg(ctx, "b200m_multiscale_vote: xyz stride must be a multiple of 4 and >= 12 bytes");
     if (ms->n_query_kps == 0) return 0;
     if (!d_train_xyz || !d_idx || !d_dist || !d_count) return b200m_fail_msg(ctx, "b200m_multiscale_vote: null pointer");
-    ms_vote_kernel<<<(unsigned) ((ms->n_query_kps + 127) / 128), 128, 0, ctx->stream>>>(
+    ms_vote_kernel<false><<<(unsigned) ((ms->n_query_kps + 127) / 128), 128, 0, ctx->stream>>>(
         ms->n_query_kps, ms->n_scales, ms->k, ms->idx.as<int32_t>(), ms->dist.as<float>(), ms->cnt.as<int32_t>(), d_train_xyz,
         xyz_stride_bytes / 4, iss_radius, d_idx, d_dist, d_count);
+    CK(cudaGetLastError());
+    ctx->stats.launches += 1;
+    return 0;
+}
+
+int ms_vote_batch_device(b200m_ctx *ctx, MultiscaleState *ms, const float *d_train_xyz, size_t xyz_stride_bytes,
+                         const int32_t *d_kp_off, int n_pairs, const float *d_radii, int32_t *d_idx, float *d_dist,
+                         int32_t *d_count) {
+    if (ms->n_query_kps == 0) return 0;
+    ms_vote_kernel<true><<<(unsigned) ((ms->n_query_kps + 127) / 128), 128, 0, ctx->stream>>>(
+        ms->n_query_kps, ms->n_scales, ms->k, ms->idx.as<int32_t>(), ms->dist.as<float>(), ms->cnt.as<int32_t>(), d_train_xyz,
+        xyz_stride_bytes / 4, 0.f, d_idx, d_dist, d_count, d_kp_off, n_pairs, d_radii);
     CK(cudaGetLastError());
     ctx->stats.launches += 1;
     return 0;
