@@ -375,6 +375,30 @@ B200M_API int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *p
                                            const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
                                            size_t *offsets, float *avg);
 
+/* ---- the matcher classes at the WIDE seam with AlignmentParameters::guess set, many cloud pairs in one call ----------
+ * With a guess, match_multiscale answers every scale with matchLocal (include/matching.h:297-311, :637-678): the query
+ * keypoints are moved by the guess (the reverse call, inverse_tn, by its inverse) and only train keypoints within
+ * match_search_radius compete.  This is b200m_match_multiscale_batch with that kNN: for pair p and scale s, source row r
+ * is gated at src_kps_moved[src_map[r]] against the target keypoints tgt_kps_xyz (unmoved); in the reverse pass target
+ * row c is gated at tgt_kps_moved[tgt_map[c]] against the source keypoints (unmoved).  The gate and the order are
+ * b200m_knn_local's: FP32 L2_Simple squared distance < radius*radius (radius 0 or NaN: nothing passes; FLT_MAX or inf:
+ * every finite row), entries ordered by (descriptor distance, spatial distance, index), a non-finite query keypoint or
+ * descriptor gets an empty list, a non-finite train row is never returned.  The moved coordinates come from the caller
+ * (pcl::transformPointCloudWithNormals in a PCL build), so the transform's arithmetic stays the caller's; the library never
+ * inverts a matrix.  Everything after the kNN -- remap, votes over the unmoved keypoints, average, filter, outputs and
+ * errors -- is b200m_match_multiscale_batch's.  p->precision does not apply (exact CUDA-core path).  A single pair is a
+ * batch of one.  Host pointers; this call REPLACES the descriptor sets b200m_upload put in the context. */
+typedef struct {
+    const float *src_kps_moved;   /* n_src_kps rows, xyz_stride_bytes apart: the source keypoints moved by this pair's guess */
+    const float *tgt_kps_moved;   /* n_tgt_kps rows: the target keypoints moved by the guess's inverse (may be NULL in
+                                     ONE_SIDED mode) */
+} b200m_local_pair;
+B200M_API int b200m_match_multiscale_local_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs,
+                                                 const b200m_local_pair *locals, int n_pairs, size_t stride_bytes, int dim,
+                                                 size_t xyz_stride_bytes, int cluster_k, float match_search_radius,
+                                                 const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
+                                                 size_t *offsets, float *avg);
+
 B200M_API int b200m_version(void);
 
 /* ---- test hooks (used by tests/ only; not part of the reference-facing surface) ----

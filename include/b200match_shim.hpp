@@ -11,6 +11,8 @@
 //   RatioMatcher / ClusterMatcher  (match(), getAverageDistance(), getClassName())
 //                                  reference include/matching.h:25-42, :96-161, :385-551
 //   matchMany<FeatureT>            match() of many OneSided / LeftToRight / ClusterMatchers (cloud pairs) in one call
+// With AlignmentParameters::guess set, the matcher classes and matchMany run match_multiscale's matchLocal form
+// (b200m_match_multiscale_local_batch): each scale's kNN gated at match_search_radius around the moved keypoints.
 // The matcher classes run match_impl as the reference composes it -- match_multiscale (per-scale kNN, spatial vote ->
 // at most one match per keypoint) in one or both directions, then the filter over the voted lists -- in ONE library
 // call (b200m_match_multiscale); the narrow-seam functions share one context per host thread and device, so calling
@@ -24,9 +26,11 @@
 #pragma once
 #include <algorithm>
 #include <array>
+#include <cmath>
 #include <limits>
 #include <map>
 #include <memory>
+#include <optional>
 #include <stdexcept>
 #include <string>
 #include <utility>
@@ -90,6 +94,8 @@ struct AlignmentParameters {
     std::string matching_id = "lr"; // :149  one_sided | lr | ratio | cluster
     float ratio_thr = 1.1f;         // MATCHING_RATIO_THRESHOLD, include/common.h:50
     float match_search_radius = std::numeric_limits<float>::max();   // :160  matchLocal's 3-D gate
+    std::optional<std::array<float, 16>> guess;   // :161  prior pose, row-major (Eigen::Matrix4f): match_multiscale then uses
+                                                  // matchLocal (include/matching.h:297-311)
     int device = 0;
     std::vector<int> devices;       // more than one entry: the call is partitioned over these GPUs inside the library
                                     // (b200m_create_multi: source rows sharded, target replicated, NCCL over NVLink)
@@ -290,6 +296,44 @@ std::vector<MultivaluedCorrespondence> matchLocal(const FeatureCloud<FeatureT> &
     return matchBF<FeatureT>(query_features, train_features, parameters);
 }
 
+// The keypoints moved by `guess` (row-major 4x4): x' = ((g00 x + g01 y) + g02 z) + g03 in float, every product and sum
+// rounded on its own (Eigen's affine product order).  `n` rows `in_stride` floats apart in, `out_stride` floats apart out;
+// only the first three floats of an output row are written.
+inline void moveKeypoints(const float *kps, size_t n, size_t in_stride, const std::array<float, 16> &guess, float *out,
+                          size_t out_stride) {
+    for (size_t i = 0; i < n; ++i) {
+        const float *q = kps + i * in_stride;
+        for (int r = 0; r < 3; ++r)
+            out[i * out_stride + r] = guess[4 * r] * q[0] + guess[4 * r + 1] * q[1] + guess[4 * r + 2] * q[2] + guess[4 * r + 3];
+    }
+}
+
+// The inverse of a guess (the pose of the reverse matchLocal call, inverse_tn): Gauss-Jordan with partial pivoting in
+// double, rounded to float.
+inline std::array<float, 16> invertGuess(const std::array<float, 16> &g) {
+    double a[4][8];
+    for (int r = 0; r < 4; ++r)
+        for (int c = 0; c < 8; ++c) a[r][c] = c < 4 ? (double) g[4 * r + c] : (c - 4 == r ? 1.0 : 0.0);
+    for (int c = 0; c < 4; ++c) {
+        int piv = c;
+        for (int r = c + 1; r < 4; ++r)
+            if (std::abs(a[r][c]) > std::abs(a[piv][c])) piv = r;
+        if (a[piv][c] == 0.0) throw std::runtime_error("the guess is not invertible");
+        for (int j = 0; j < 8; ++j) std::swap(a[c][j], a[piv][j]);
+        const double d = a[c][c];
+        for (int j = 0; j < 8; ++j) a[c][j] /= d;
+        for (int r = 0; r < 4; ++r)
+            if (r != c) {
+                const double f = a[r][c];
+                for (int j = 0; j < 8; ++j) a[r][j] -= f * a[c][j];
+            }
+    }
+    std::array<float, 16> inv;
+    for (int r = 0; r < 4; ++r)
+        for (int c = 0; c < 4; ++c) inv[4 * r + c] = (float) a[r][4 + c];
+    return inv;
+}
+
 // matchLocal<FeatureT> as match_multiscale calls it when AlignmentParameters::guess is set (reference
 // include/matching.h:378-383, :637-678): the query keypoints are moved by `guess` (row-major 4x4, the reference's
 // Eigen::Matrix4f; pcl::transformPointCloudWithNormals, :644), and only train rows whose keypoint lies within
@@ -307,11 +351,7 @@ std::vector<MultivaluedCorrespondence> matchLocal(const float *query_kps, const 
     const size_t nq = cloud_size<FeatureT>(query_features), fl = kps_stride_bytes / 4;
     const int k = parameters.randomness;
     std::vector<float> moved(nq * 3);
-    for (size_t i = 0; i < nq; ++i) {   // Eigen's affine product: x' = m00 x + m01 y + m02 z + m03 (float)
-        const float *q = query_kps + i * fl;
-        for (int r = 0; r < 3; ++r)
-            moved[3 * i + r] = guess[4 * r] * q[0] + guess[4 * r + 1] * q[1] + guess[4 * r + 2] * q[2] + guess[4 * r + 3];
-    }
+    moveKeypoints(query_kps, nq, fl, guess, moved.data(), 3);
     std::vector<float> train_xyz(cloud_size<FeatureT>(train_features) * 3);
     for (size_t j = 0; j < train_xyz.size() / 3; ++j)
         for (int r = 0; r < 3; ++r) train_xyz[3 * j + r] = train_kps[j * fl + r];
@@ -487,6 +527,19 @@ protected:
         }
     }
 
+    // with a guess: the keypoints of both clouds moved for the two matchLocal directions -- the source by the guess, the
+    // target by its inverse -- in the keypoint rows' own stride
+    void movedRows(std::vector<float> &ms, std::vector<float> &mt) const {
+        if (!st_src_.kps_xyz || !st_tgt_.kps_xyz)
+            throw std::runtime_error("a guess needs the keypoint coordinates of both clouds: matchLocal gates on them "
+                                     "(include/matching.h:637-678)");
+        const size_t fl = st_src_.kps_stride_bytes / 4;
+        ms.assign(st_src_.n_kps * fl + 4, 0.f);
+        mt.assign(st_tgt_.n_kps * fl + 4, 0.f);
+        moveKeypoints(st_src_.kps_xyz, st_src_.n_kps, fl, *parameters_.guess, ms.data(), fl);
+        moveKeypoints(st_tgt_.kps_xyz, st_tgt_.n_kps, fl, invertGuess(*parameters_.guess), mt.data(), fl);
+    }
+
     // match_impl of the three implemented matchers: both match_multiscale calls, the vote, printDebugInfo's average
     // and the filter loop in one device-resident call
     virtual CorrespondencesPtr match_impl() {
@@ -495,11 +548,28 @@ protected:
         std::vector<float> zeros;
         const float *sx, *tx;
         size_t stride;
+        if (parameters_.guess && parameters_.devices.size() > 1)
+            throw std::runtime_error("a guess runs on one GPU only (parameters.devices has several)");
         keypointRows(scales.size(), zeros, &sx, &tx, &stride);
+        std::vector<float> ms, mt;
+        if (parameters_.guess) movedRows(ms, mt);
         const bool thr = !st_src_.thresholds.empty() && !st_tgt_.thresholds.empty();
         b200m_params p = make_params(parameters_, mode(), parameters_.randomness);
         auto out = std::make_shared<Correspondences>(st_src_.n_kps);
         size_t n = 0;
+        if (parameters_.guess) {   // matchLocal per scale and direction: a batch of one pair
+            const b200m_wide_pair wp{scales.data(), (int) scales.size(), sx, st_src_.n_kps, tx, st_tgt_.n_kps, st_src_.iss_radius,
+                                     st_tgt_.iss_radius};
+            const b200m_local_pair lp{ms.data(), mt.data()};
+            size_t offsets[2] = {0, 0};
+            Context &ctx = shared_context(parameters_.device);
+            ctx.check(b200m_match_multiscale_local_batch(
+                ctx.get(), &p, &wp, &lp, 1, sizeof(FeatureT), feature_dim<FeatureT>(), stride, parameters_.cluster_k,
+                parameters_.match_search_radius, thr ? st_src_.thresholds.data() : nullptr, thr ? st_tgt_.thresholds.data() : nullptr,
+                reinterpret_cast<b200m_corr *>(out->data()), std::max<size_t>(out->size(), 1), offsets, &average_distance_));
+            out->resize(offsets[1]);
+            return out;
+        }
         if (parameters_.devices.size() > 1) {
             // several GPUs: the library partitions the k-list matcher call (b200m_group_match).  That IS match_impl when every
             // keypoint has one candidate (randomness 1, one scale, identity maps: the vote keeps it); the voted multi-scale
@@ -566,6 +636,7 @@ public:
 protected:
     int mode() const override { return B200M_MODE_RATIO; }
     CorrespondencesPtr match_impl() override {
+        if (this->parameters_.guess) throw std::runtime_error("RatioMatcher: a guess is not supported (the reference's is a stub)");
         if (this->st_src_.kps_features_multiscale.size() != 1 || this->st_tgt_.kps_features_multiscale.size() != 1)
             throw std::runtime_error("RatioMatcher is defined on a single scale");
         Context &ctx = shared_context(this->parameters_.device);
@@ -586,8 +657,9 @@ protected:
 
 // match() of many OneSided / LeftToRight / ClusterMatchers in one library call (b200m_match_multiscale_batch): multi-view
 // registration, one scan against many submaps, an evaluation table.  All matchers must be of one class with the same
-// parameters and keypoint point stride; each pair's common scales are built as match_impl builds them.  result[i] equals
-// matchers[i]->match(), finalize included, and matchers[i]->getAverageDistance() is set.  One GPU only.
+// parameters (the guess aside: each matcher may have its own) and keypoint point stride; each pair's common scales are
+// built as match_impl builds them.  Either every matcher has a guess (b200m_match_multiscale_local_batch) or none has.
+// result[i] equals matchers[i]->match(), finalize included, and matchers[i]->getAverageDistance() is set.  One GPU only.
 inline bool sameParameters(const AlignmentParameters &a, const AlignmentParameters &b) {
     return a.use_bfmatcher == b.use_bfmatcher && a.bf_block_size == b.bf_block_size && a.ratio_k == b.ratio_k &&
            a.cluster_k == b.cluster_k && a.randomness == b.randomness && a.distance_thr == b.distance_thr &&
@@ -608,6 +680,9 @@ std::vector<CorrespondencesPtr> matchMany(const std::vector<std::shared_ptr<Feat
     std::vector<std::vector<b200m_scale>> scales(n);
     std::vector<std::vector<float>> zeros(n);
     std::vector<b200m_wide_pair> pairs(n);
+    std::vector<b200m_local_pair> locals(n);
+    std::vector<std::vector<float>> moved(2 * n);
+    const bool guessed = pa.guess.has_value();
     std::vector<float> thr_src, thr_tgt;
     bool thr = false;
     size_t stride = 0, n_src = 0;
@@ -616,10 +691,16 @@ std::vector<CorrespondencesPtr> matchMany(const std::vector<std::shared_ptr<Feat
         if (m.mode() != mode || matchers[i]->getClassName() != matchers[0]->getClassName() || !sameParameters(m.parameters_, pa))
             throw std::runtime_error("matchMany: every matcher must be of one class with the same AlignmentParameters");
         if (m.parameters_.devices.size() > 1) throw std::runtime_error("matchMany: one GPU only (parameters.devices has several)");
+        if (m.parameters_.guess.has_value() != guessed)
+            throw std::runtime_error("matchMany: give every matcher a guess or none (the guessed and unguessed kNN are different calls)");
         scales[i] = m.commonScales();
         const float *sx, *tx;
         size_t st;
         m.keypointRows(scales[i].size(), zeros[i], &sx, &tx, &st);
+        if (guessed) {
+            m.movedRows(moved[2 * i], moved[2 * i + 1]);
+            locals[i] = b200m_local_pair{moved[2 * i].data(), moved[2 * i + 1].data()};
+        }
         if (i && st != stride) throw std::runtime_error("matchMany: every keypoint cloud must have the same point stride");
         stride = st;
         pairs[i] = b200m_wide_pair{scales[i].data(), (int) scales[i].size(), sx, m.st_src_.n_kps, tx, m.st_tgt_.n_kps,
@@ -648,9 +729,15 @@ std::vector<CorrespondencesPtr> matchMany(const std::vector<std::shared_ptr<Feat
     std::vector<size_t> offsets(n + 1);
     std::vector<float> avg(n);
     Context &ctx = shared_context(pa.device);
-    ctx.check(b200m_match_multiscale_batch(ctx.get(), &p, pairs.data(), (int) n, sizeof(FeatureT), feature_dim<FeatureT>(), stride,
-                                           pa.cluster_k, thr ? thr_src.data() : nullptr, thr ? thr_tgt.data() : nullptr,
-                                           reinterpret_cast<b200m_corr *>(all.data()), all.size(), offsets.data(), avg.data()));
+    if (guessed)
+        ctx.check(b200m_match_multiscale_local_batch(ctx.get(), &p, pairs.data(), locals.data(), (int) n, sizeof(FeatureT),
+                                                     feature_dim<FeatureT>(), stride, pa.cluster_k, pa.match_search_radius,
+                                                     thr ? thr_src.data() : nullptr, thr ? thr_tgt.data() : nullptr,
+                                                     reinterpret_cast<b200m_corr *>(all.data()), all.size(), offsets.data(), avg.data()));
+    else
+        ctx.check(b200m_match_multiscale_batch(ctx.get(), &p, pairs.data(), (int) n, sizeof(FeatureT), feature_dim<FeatureT>(), stride,
+                                               pa.cluster_k, thr ? thr_src.data() : nullptr, thr ? thr_tgt.data() : nullptr,
+                                               reinterpret_cast<b200m_corr *>(all.data()), all.size(), offsets.data(), avg.data()));
     for (size_t i = 0; i < n; ++i) {
         matchers[i]->average_distance_ = avg[i];
         result.push_back(matchers[i]->finalize(std::make_shared<Correspondences>(all.begin() + offsets[i], all.begin() + offsets[i + 1])));

@@ -256,6 +256,25 @@ void comm_release(b200m_ctx *ctx);
 void local_release(b200m_ctx *ctx);
 int launch_local_cells(b200m_ctx *ctx, int direction, const float *d_query_xyz, const float *d_train_xyz, size_t xyz_stride_bytes,
                        float radius, int k, int32_t *d_idx, float *d_dist, int32_t *d_count);
+// The batch form for b200m_match_multiscale_local_batch (wide_batch.cu): one scale and direction of every pair at once over
+// the padded layout stage_batch left in the context; train indices come out as global padded rows.  Per side (0 = source,
+// 1 = target) the scale's block -> pair table, row -> keypoint map over the padded rows and keypoint offsets ([n_pairs + 1]).
+struct LocalBatch {
+    int direction = 0, scale = 0, n_pairs = 0, k = 1;
+    const int4 *rows = nullptr;   // [n_pairs] {first source row, source rows, first target row, target rows} of this scale
+    const int32_t *blk[2] = {nullptr, nullptr}, *map[2] = {nullptr, nullptr}, *kp_off[2] = {nullptr, nullptr};
+    const float *q_xyz = nullptr;   // the query side's keypoints MOVED by the guess (forward) / its inverse (reverse)
+    const float *t_xyz = nullptr;   // the train side's keypoints, unmoved
+    size_t xyz_stride_bytes = 16;
+    float radius = 0.f;
+    unsigned long long *bad = nullptr;   // flag_bad() key of the first out-of-range map entry
+};
+int launch_local_cells_batch(b200m_ctx *ctx, const LocalBatch &a, int32_t *d_idx, float *d_dist, int32_t *d_count);
+
+// first out-of-range map entry of a batch call, smallest (scale, pair, side) wins; side 0 = a source map, 1 = a target map
+__device__ __forceinline__ void flag_bad(unsigned long long *bad, int scale, int pair, int side) {
+    atomicMin(bad, ((unsigned long long) scale << 48) | ((unsigned long long) pair << 16) | (unsigned long long) side);
+}
 
 // api.cu: kNN of query rows [row_begin, row_begin + n_rows) of `direction` on device buffers; with d_flags only the flagged
 // (and valid) rows are answered, the others get empty lists.  Outputs are indexed by (row - row_begin).

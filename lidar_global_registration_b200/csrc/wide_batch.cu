@@ -18,6 +18,10 @@
 //                   single-pair cluster distance and compaction.
 //   output          records ascend in global source keypoint, i.e. in pair order; one kernel makes them pair-local and
 //                   counts them per pair; the average is average_kernel's chain over each pair's voted forward lists.
+//
+// b200m_match_multiscale_local_batch is the same driver with a guess: per scale and direction the kNN pass is the gated
+// kNN of local.cu's batch form (launch_local_cells_batch) over the caller's moved query keypoints; everything after it is
+// unchanged (DESIGN.md section 3.13).
 #include <string.h>
 
 #include <algorithm>
@@ -31,16 +35,12 @@ namespace {
 struct WideBatchState {
     MultiscaleState fwd, rev;
     DevBuf tables, xyz_s, xyz_t, kidx, kdist, kcnt, vfi, vfd, vfc, vri, vrd, vrc;
+    DevBuf mov_s, mov_t;   // guessed calls: the moved source / target keypoints
 };
 
 WideBatchState *wb_state(b200m_ctx *ctx) {
     if (!ctx->wide_batch) ctx->wide_batch = new WideBatchState();
     return static_cast<WideBatchState *>(ctx->wide_batch);
-}
-
-// first out-of-range map entry, smallest (scale, pair, side) wins; side 0 = a source map, 1 = a target map
-__device__ __forceinline__ void flag_bad(unsigned long long *bad, int scale, int pair, int side) {
-    atomicMin(bad, ((unsigned long long) scale << 48) | ((unsigned long long) pair << 16) | (unsigned long long) side);
 }
 
 // ms_scatter_kernel over the padded global rows of one scale and direction (q_side 0: queries = source rows).
@@ -113,22 +113,26 @@ void wide_batch_release(b200m_ctx *ctx) {
         for (DevBuf *x : b) x->release();
     }
     DevBuf *b[] = {&ws->tables, &ws->xyz_s, &ws->xyz_t, &ws->kidx, &ws->kdist, &ws->kcnt, &ws->vfi, &ws->vfd, &ws->vfc,
-                   &ws->vri, &ws->vrd, &ws->vrc};
+                   &ws->vri, &ws->vrd, &ws->vrc, &ws->mov_s, &ws->mov_t};
     for (DevBuf *x : b) x->release();
     delete ws;
     ctx->wide_batch = nullptr;
 }
 
-extern "C" int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs, int n_pairs,
-                                            size_t stride_bytes, int dim, size_t xyz_stride_bytes, int cluster_k,
-                                            const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
-                                            size_t *offsets, float *avg) {
-    const std::string fn = "b200m_match_multiscale_batch: ";
+namespace {
+
+// gated = false: b200m_match_multiscale_batch; true: the guessed form, whose kNN passes are gated by `radius`
+int match_multiscale_batch(b200m_ctx *ctx, const char *name, const b200m_params *p, const b200m_wide_pair *pairs, bool gated,
+                           const b200m_local_pair *locals, int n_pairs, size_t stride_bytes, int dim, size_t xyz_stride_bytes,
+                           int cluster_k, float radius, const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
+                           size_t *offsets, float *avg) {
+    const std::string fn = std::string(name) + ": ";
     if (!ctx) return b200m_fail_msg(nullptr, "null context");
     CK(cudaSetDevice(ctx->device));
     if (!p || !offsets) return b200m_fail_msg(ctx, fn + "null params / offsets");
     if (n_pairs < 0) return b200m_fail_msg(ctx, fn + "n_pairs < 0");
     if (n_pairs > 0 && !pairs) return b200m_fail_msg(ctx, fn + "null pairs");
+    if (gated && n_pairs > 0 && !locals) return b200m_fail_msg(ctx, fn + "null local pairs");
     for (int i = 0; i <= n_pairs; ++i) offsets[i] = 0;
     const int mode = p->mode;
     if (mode != B200M_MODE_ONE_SIDED && mode != B200M_MODE_MUTUAL && mode != B200M_MODE_CLUSTER)
@@ -162,6 +166,8 @@ extern "C" int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *
         if (!w.n_src_kps) continue;
         if ((w.n_tgt_kps && !w.tgt_kps_xyz) || (two_way && !w.src_kps_xyz))
             return b200m_fail_msg(ctx, pi + "null keypoint coordinates");
+        if (gated && (!locals[i].src_kps_moved || (two_way && w.n_tgt_kps && !locals[i].tgt_kps_moved)))
+            return b200m_fail_msg(ctx, pi + "null moved keypoint coordinates");
         for (int s = 0; s < w.n_scales; ++s) {
             const b200m_scale &sc = w.scales[s];
             if ((sc.n_src && !sc.src_desc) || (sc.n_tgt && !sc.tgt_desc))
@@ -254,6 +260,8 @@ extern "C" int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *
     // keypoint coordinates of all pairs back to back, `xyz_stride_bytes` apart
     CK(ws->xyz_t.reserve(NT * xyz_stride_bytes + 16));
     if (two_way) CK(ws->xyz_s.reserve(NS * xyz_stride_bytes + 16));
+    if (gated) CK(ws->mov_s.reserve(NS * xyz_stride_bytes + 16));
+    if (gated && two_way) CK(ws->mov_t.reserve(NT * xyz_stride_bytes + 16));
     for (int i = 0; i < n_pairs; ++i) {
         if (!pairs[i].n_src_kps) continue;
         if (copy_xyz(ctx, ws->xyz_t.as<char>() + (size_t) kp_off[1][i] * xyz_stride_bytes, pairs[i].tgt_kps_xyz, pairs[i].n_tgt_kps,
@@ -262,6 +270,14 @@ extern "C" int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *
         if (two_way && copy_xyz(ctx, ws->xyz_s.as<char>() + (size_t) kp_off[0][i] * xyz_stride_bytes, pairs[i].src_kps_xyz,
                                 pairs[i].n_src_kps, xyz_stride_bytes))
             return 1;
+        if (gated) {
+            if (copy_xyz(ctx, ws->mov_s.as<char>() + (size_t) kp_off[0][i] * xyz_stride_bytes, locals[i].src_kps_moved,
+                         pairs[i].n_src_kps, xyz_stride_bytes))
+                return 1;
+            if (two_way && copy_xyz(ctx, ws->mov_t.as<char>() + (size_t) kp_off[1][i] * xyz_stride_bytes, locals[i].tgt_kps_moved,
+                                    pairs[i].n_tgt_kps, xyz_stride_bytes))
+                return 1;
+        }
     }
     if (ms_begin(ctx, &ws->fwd, NS, n_scales, k)) return 1;
     if (two_way && ms_begin(ctx, &ws->rev, NT, n_scales, k)) return 1;
@@ -275,6 +291,7 @@ extern "C" int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *
     }
     b200m_params pk = *p;
     pk.mode = B200M_MODE_KNN_ONLY;
+    if (gated) pk.precision = B200M_PREC_F32_EXACT;   // the gated kNN is exact CUDA-core arithmetic: no tensor-core set-up
     std::vector<b200m_pair> sp(n_pairs);
     for (int s = 0; s < n_scales; ++s) {
         for (int i = 0; i < n_pairs; ++i) {
@@ -283,7 +300,7 @@ extern "C" int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *
                                n_rows(i, s, 1)};
         }
         BatchLayout L;
-        if (stage_batch(ctx, "b200m_match_multiscale_batch", &pk, sp.data(), n_pairs, stride_bytes, dim, &L)) return 1;
+        if (stage_batch(ctx, name, &pk, sp.data(), n_pairs, stride_bytes, dim, &L)) return 1;
         const size_t S = L.n_rows[0], T = L.n_rows[1], n_max = std::max(S, T);
         CK(ws->kidx.reserve(sizeof(int32_t) * (n_max * k + 1)));
         CK(ws->kdist.reserve(sizeof(float) * (n_max * k + 1)));
@@ -294,9 +311,30 @@ extern "C" int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *
             const size_t nq = dir ? T : S;
             if (!nq) continue;
             MultiscaleState &ms = dir ? ws->rev : ws->fwd;
-            if (b200m_knn_rows(ctx, &pk, dir, 0, nq, nullptr, ws->kidx.as<int32_t>(), ws->kdist.as<float>(), ws->kcnt.as<int32_t>(),
-                               &L.seg[dir]))
+            if (gated) {
+                LocalBatch lb;
+                lb.direction = dir;
+                lb.scale = s;
+                lb.n_pairs = n_pairs;
+                lb.k = k;
+                lb.rows = d_rows;
+                for (int side = 0; side < 2; ++side) {
+                    lb.blk[side] = reinterpret_cast<const int32_t *>(d + o_blk[side][s]);
+                    lb.map[side] = side ? d_map1 : d_map0;
+                    lb.kp_off[side] = side ? d_off1 : d_off0;
+                }
+                lb.q_xyz = dir ? ws->mov_t.as<float>() : ws->mov_s.as<float>();
+                lb.t_xyz = dir ? ws->xyz_s.as<float>() : ws->xyz_t.as<float>();
+                lb.xyz_stride_bytes = xyz_stride_bytes;
+                lb.radius = radius;
+                lb.bad = d_bad;
+                StatTimer tf(ctx, &ctx->stats.ms_fallback);
+                if (launch_local_cells_batch(ctx, lb, ws->kidx.as<int32_t>(), ws->kdist.as<float>(), ws->kcnt.as<int32_t>())) return 1;
+                tf.stop();
+            } else if (b200m_knn_rows(ctx, &pk, dir, 0, nq, nullptr, ws->kidx.as<int32_t>(), ws->kdist.as<float>(),
+                                      ws->kcnt.as<int32_t>(), &L.seg[dir])) {
                 return 1;
+            }
             ms_scatter_batch_kernel<<<(unsigned) ((nq + 255) / 256), 256, 0, st>>>(
                 nq, k, s, n_scales, dir, ws->kidx.as<int32_t>(), ws->kdist.as<float>(), ws->kcnt.as<int32_t>(),
                 reinterpret_cast<const int32_t *>(d + o_blk[dir][s]), d_rows, dir ? d_map1 : d_map0, dir ? d_map0 : d_map1,
@@ -364,4 +402,23 @@ extern "C" int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *
         CK(cudaStreamSynchronize(st));
     }
     return 0;
+}
+
+}  // namespace
+
+extern "C" int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs, int n_pairs,
+                                            size_t stride_bytes, int dim, size_t xyz_stride_bytes, int cluster_k,
+                                            const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
+                                            size_t *offsets, float *avg) {
+    return match_multiscale_batch(ctx, "b200m_match_multiscale_batch", p, pairs, false, nullptr, n_pairs, stride_bytes, dim,
+                                  xyz_stride_bytes, cluster_k, 0.f, thr_src, thr_tgt, out, cap, offsets, avg);
+}
+
+extern "C" int b200m_match_multiscale_local_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs,
+                                                  const b200m_local_pair *locals, int n_pairs, size_t stride_bytes, int dim,
+                                                  size_t xyz_stride_bytes, int cluster_k, float match_search_radius,
+                                                  const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
+                                                  size_t *offsets, float *avg) {
+    return match_multiscale_batch(ctx, "b200m_match_multiscale_local_batch", p, pairs, true, locals, n_pairs, stride_bytes, dim,
+                                  xyz_stride_bytes, cluster_k, match_search_radius, thr_src, thr_tgt, out, cap, offsets, avg);
 }
