@@ -399,6 +399,39 @@ B200M_API int b200m_match_multiscale_local_batch(b200m_ctx *ctx, const b200m_par
                                                  const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
                                                  size_t *offsets, float *avg);
 
+/* ---- device-resident batch calls: the four batch calls on descriptors, maps, keypoints and records in HBM -------------
+ * For a caller whose sets already live on the GPU (a GPU feature stage, a torch pipeline, sets reused across calls).
+ * Each takes its host form's arguments: the arrays of b200m_pair / b200m_wide_pair / b200m_scale / b200m_local_pair and
+ * every size and radius in them stay HOST memory, but every data pointer inside them (descriptors, index maps, keypoint
+ * coordinates, moved keypoints) and the threshold arrays are DEVICE pointers on the context's device.  Different pairs may
+ * point at the same memory (one scan against many submaps).  Pair p's records, offsets, average and k-lists are byte for
+ * byte what the host form returns on the same data; validation, errors (under the new name), "replaces the uploaded sets"
+ * and the capacity rule are the host form's.
+ * Outputs: b200m_knn_batch_device writes d_idx [sum n_src][k], d_dist and d_count (device); the match calls write the
+ * records to d_out (device, `cap` records) and offsets [n_pairs + 1] / avg [n_pairs] to HOST arrays (the call reads its
+ * result area back once anyway, and the caller needs host integers to split the records).  Work is queued on the
+ * context's stream; on return the records and k-lists are ordered on that stream, not yet complete.
+ * Every non-null data pointer is checked with cudaPointerGetAttributes before anything is queued: it must be device or
+ * managed memory of the context's device, otherwise the call fails with an error naming the pair, scale and field.
+ * Only the call's own tables go host -> device (segment, row and block tables, offsets, radii); the descriptors are
+ * packed where they are and maps, coordinates and thresholds are filed by one gather kernel per table, so the number of
+ * launches and copies does not depend on n_pairs (DESIGN.md section 3.14). */
+B200M_API int b200m_knn_batch_device(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                                     size_t stride_bytes, int dim, int32_t *d_idx, float *d_dist, int32_t *d_count);
+B200M_API int b200m_match_batch_device(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                                       size_t stride_bytes, int dim, const float *d_thr_src, const float *d_thr_tgt,
+                                       b200m_corr *d_out, size_t cap, size_t *offsets, float *avg);
+B200M_API int b200m_match_multiscale_batch_device(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs,
+                                                  int n_pairs, size_t stride_bytes, int dim, size_t xyz_stride_bytes,
+                                                  int cluster_k, const float *d_thr_src, const float *d_thr_tgt,
+                                                  b200m_corr *d_out, size_t cap, size_t *offsets, float *avg);
+B200M_API int b200m_match_multiscale_local_batch_device(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs,
+                                                        const b200m_local_pair *locals, int n_pairs, size_t stride_bytes,
+                                                        int dim, size_t xyz_stride_bytes, int cluster_k,
+                                                        float match_search_radius, const float *d_thr_src,
+                                                        const float *d_thr_tgt, b200m_corr *d_out, size_t cap,
+                                                        size_t *offsets, float *avg);
+
 B200M_API int b200m_version(void);
 
 /* ---- test hooks (used by tests/ only; not part of the reference-facing surface) ----

@@ -292,7 +292,7 @@ int staged_h2d(b200m_ctx *ctx, void *dst, const void *src, size_t bytes) {
 
 // ---- upload -----------------------------------------------------------------------------
 int upload_common(b200m_ctx *ctx, int side, const float *device_aos, size_t n, size_t stride_bytes, int dim,
-                         int64_t index_offset) {
+                         int64_t index_offset, const int32_t *seg_blk, const SetRef *sets) {
     Side &sd = ctx->side[side];
     sd.n = n;
     sd.n_pad = (n + B200M_TILE_N - 1) / B200M_TILE_N * B200M_TILE_N;
@@ -308,7 +308,7 @@ int upload_common(b200m_ctx *ctx, int side, const float *device_aos, size_t n, s
     CK(sd.stats.reserve(pack_stats_bytes(ctx->sm_count, sd.dp)));
     StatTimer t(ctx, &ctx->stats.ms_pack);
     CK(launch_pack_f32(device_aos, n, stride_bytes, dim, sd.dp, sd.f32.as<float>(), sd.valid.as<uint8_t>(),
-                       sd.stats.as<float>(), ctx->sm_count, ctx->stream));
+                       sd.stats.as<float>(), ctx->sm_count, ctx->stream, seg_blk, sets));
     ctx->stats.launches += 1;
     t.stop();
     return 0;

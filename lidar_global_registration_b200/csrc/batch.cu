@@ -21,6 +21,7 @@
 // FP16, any upper bound on |b16|); only the candidate counts can differ, never the exact re-rank's answer.
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -69,12 +70,52 @@ __global__ void localize_records_kernel(b200m_corr *__restrict__ rec, const unsi
     }
 }
 
+// One CTA column per set (blockIdx.x), its rows spread over blockIdx.y and the threads: w words of every row.
+__global__ void gather_sets_kernel(const GatherSet *__restrict__ sets, int w, size_t dst_stride, uint32_t *__restrict__ dst) {
+    const GatherSet g = sets[blockIdx.x];
+    const uint32_t *src = static_cast<const uint32_t *>(g.src);
+    for (long long r = (long long) blockIdx.y * blockDim.x + threadIdx.x; r < g.rows; r += (long long) gridDim.y * blockDim.x) {
+        uint32_t *d = dst + (size_t) (g.dst_row + r) * dst_stride;
+        if (!src) {
+            d[0] = (uint32_t) r;
+            continue;
+        }
+        for (int c = 0; c < w; ++c) d[c] = __ldg(src + r * g.src_stride + c);
+    }
+}
+
 }  // namespace
 
+cudaError_t launch_gather_sets(const GatherSet *d_sets, int n_sets, size_t max_rows, int w, size_t dst_stride_words, void *dst,
+                               cudaStream_t st) {
+    if (n_sets == 0 || max_rows == 0) return cudaSuccess;
+    const unsigned chunks = (unsigned) std::min<size_t>((max_rows + 255) / 256, 32);
+    gather_sets_kernel<<<dim3((unsigned) n_sets, chunks), 256, 0, st>>>(d_sets, w, dst_stride_words, static_cast<uint32_t *>(dst));
+    return cudaGetLastError();
+}
+
+int check_device_ptr(b200m_ctx *ctx, const std::string &where, const void *ptr) {
+    if (!ptr) return 0;
+    cudaPointerAttributes a;
+    const cudaError_t e = cudaPointerGetAttributes(&a, ptr);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return b200m_fail_msg(ctx, where + " is not device memory (" + cudaGetErrorString(e) + ")");
+    }
+    if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)
+        return b200m_fail_msg(ctx, where + " is not device memory (" +
+                                       (a.type == cudaMemoryTypeHost ? "page-locked host memory" : "host memory") + ")");
+    if (a.device != ctx->device)
+        return b200m_fail_msg(ctx, where + " is memory of device " + std::to_string(a.device) + ", the context's device is " +
+                                       std::to_string(ctx->device));
+    return 0;
+}
+
 // Validates the batch, packs both sides in the padded layout (replacing what b200m_upload put in the context) and
-// uploads the segment tables.
+// uploads the segment tables.  dev: the descriptor pointers are device pointers, checked here and read in place by the
+// segmented pack (the per-pair SetRef tables and side 1's block table go up with the other tables).
 int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
-                size_t stride_bytes, int dim, BatchLayout *L) {
+                size_t stride_bytes, int dim, BatchLayout *L, bool dev, const float *d_thr_src, const float *d_thr_tgt) {
     const std::string f(fn);
     if (n_pairs < 0) return b200m_fail_msg(ctx, f + ": n_pairs < 0");
     if (n_pairs > 0 && !pairs) return b200m_fail_msg(ctx, f + ": null pairs");
@@ -93,6 +134,8 @@ int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b20
         const float *base[2] = {pairs[i].src, pairs[i].tgt};
         for (int s = 0; s < 2; ++s) {
             if (n[s] && !base[s]) return b200m_fail_msg(ctx, f + ": null descriptor pointer in pair " + std::to_string(i));
+            if (dev && n[s] && check_device_ptr(ctx, f + ": pair " + std::to_string(i) + ": " + (s ? "tgt" : "src"), base[s]))
+                return 1;
             start[s][i] = L->n_rows[s];
             L->n_rows[s] += pad_rows(n[s]);
             if (n[s] > max_rows[s]) max_rows[s] = n[s];
@@ -107,21 +150,44 @@ int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b20
     const size_t o_bpair = align16(o_range1 + sizeof(int2) * nb[1]);
     const size_t o_info = align16(o_bpair + sizeof(int32_t) * nb[0]);
     const size_t o_avgs = align16(o_info + sizeof(int4) * n_pairs);
-    const size_t o_res = align16(o_avgs + sizeof(int2) * n_pairs);
+    // device calls only: side 1's block -> pair table and both sides' SetRef tables
+    const size_t o_bpair1 = align16(o_avgs + sizeof(int2) * n_pairs);
+    const size_t o_sets0 = align16(o_bpair1 + (dev ? sizeof(int32_t) * nb[1] : 0));
+    const size_t o_sets1 = o_sets0 + (dev ? sizeof(SetRef) * n_pairs : 0);
+    // ... and the gather tables of b200m_match_batch_device's thresholds
+    const bool thr = dev && d_thr_src;
+    const size_t o_thr0 = align16(o_sets1 + (dev ? sizeof(SetRef) * n_pairs : 0));
+    const size_t o_thr1 = o_thr0 + (thr ? sizeof(GatherSet) * n_pairs : 0);
+    const size_t o_res = align16(o_thr1 + (thr ? sizeof(GatherSet) * n_pairs : 0));
     L->result_bytes = 16 + align16(sizeof(unsigned) * n_pairs) + sizeof(float) * n_pairs;
     std::vector<char> h(o_res);
     int2 *range0 = reinterpret_cast<int2 *>(h.data() + o_range0), *range1 = reinterpret_cast<int2 *>(h.data() + o_range1);
     int32_t *bpair = reinterpret_cast<int32_t *>(h.data() + o_bpair);
     int4 *info = reinterpret_cast<int4 *>(h.data() + o_info);
     int2 *avg_segs = reinterpret_cast<int2 *>(h.data() + o_avgs);
-    size_t dense = 0;
+    int32_t *bpair1 = reinterpret_cast<int32_t *>(h.data() + o_bpair1);
+    SetRef *sets[2] = {reinterpret_cast<SetRef *>(h.data() + o_sets0), reinterpret_cast<SetRef *>(h.data() + o_sets1)};
+    GatherSet *thr_sets[2] = {reinterpret_cast<GatherSet *>(h.data() + o_thr0), reinterpret_cast<GatherSet *>(h.data() + o_thr1)};
+    size_t dense = 0, dense_t = 0;
     for (int i = 0; i < n_pairs; ++i) {
         const int s0 = (int) start[0][i], t0 = (int) start[1][i], ns = (int) pairs[i].n_src, nt = (int) pairs[i].n_tgt;
+        if (thr) {   // the thresholds are concatenated in pair order, dense
+            thr_sets[0][i] = GatherSet{d_thr_src + dense, 1, s0, ns, 0};
+            thr_sets[1][i] = GatherSet{d_thr_tgt + dense_t, 1, t0, nt, 0};
+            dense_t += (size_t) nt;
+        }
         for (size_t b = s0 / B200M_TILE_N; b < (s0 + pad_rows(ns)) / B200M_TILE_N; ++b) {
             range0[b] = make_int2(t0, t0 + nt);
             bpair[b] = i;
         }
-        for (size_t b = t0 / B200M_TILE_N; b < (t0 + pad_rows(nt)) / B200M_TILE_N; ++b) range1[b] = make_int2(s0, s0 + ns);
+        for (size_t b = t0 / B200M_TILE_N; b < (t0 + pad_rows(nt)) / B200M_TILE_N; ++b) {
+            range1[b] = make_int2(s0, s0 + ns);
+            if (dev) bpair1[b] = i;
+        }
+        if (dev) {
+            sets[0][i] = SetRef{pairs[i].src, s0, ns};
+            sets[1][i] = SetRef{pairs[i].tgt, t0, nt};
+        }
         info[i] = make_int4(s0, t0, ns, (int) dense);
         avg_segs[i] = make_int2(s0, ns);
         dense += (size_t) ns;
@@ -138,6 +204,19 @@ int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b20
     L->n_out = reinterpret_cast<unsigned long long *>(d + o_res);
     L->counts = reinterpret_cast<unsigned *>(d + o_res + 16);
     L->avgs = reinterpret_cast<float *>(d + o_res + 16 + align16(sizeof(unsigned) * n_pairs));
+    if (thr) {
+        L->thr_sets[0] = reinterpret_cast<const GatherSet *>(d + o_thr0);
+        L->thr_sets[1] = reinterpret_cast<const GatherSet *>(d + o_thr1);
+    }
+    L->max_rows[0] = max_rows[0];
+    L->max_rows[1] = max_rows[1];
+    if (dev) {   // the segmented pack reads every pair's rows where they are and writes the gap rows itself
+        const int32_t *blk[2] = {L->block_pair, reinterpret_cast<const int32_t *>(d + o_bpair1)};
+        const SetRef *d_sets[2] = {reinterpret_cast<const SetRef *>(d + o_sets0), reinterpret_cast<const SetRef *>(d + o_sets1)};
+        for (int s = 0; s < 2; ++s)
+            if (upload_common(ctx, s, nullptr, L->n_rows[s], stride_bytes, dim, 0, blk[s], d_sets[s])) return 1;
+        return 0;
+    }
     // descriptors: gap bytes 0xFF (NaN rows), then every pair's rows at its offset -- (n - 1) * stride + dim floats, as
     // b200m_upload copies: the caller owns only `dim` floats of a set's last row
     for (int s = 0; s < 2; ++s) {
@@ -163,16 +242,21 @@ int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b20
     return 0;
 }
 
-extern "C" {
+namespace {
 
-int b200m_knn_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
-                    int32_t *idx, float *dist, int32_t *count) {
+// dev: b200m_knn_batch_device (device descriptors, the k-lists are written to the caller's device arrays in place)
+int knn_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+              size_t stride_bytes, int dim, int32_t *idx, float *dist, int32_t *count) {
     REQUIRE_CTX();
     if (check_params(ctx, p)) return 1;
+    const std::string f(fn);
+    if (dev && (check_device_ptr(ctx, f + ": idx", idx) || check_device_ptr(ctx, f + ": dist", dist) ||
+                check_device_ptr(ctx, f + ": count", count)))
+        return 1;
     BatchLayout L;
-    if (stage_batch(ctx, "b200m_knn_batch", p, pairs, n_pairs, stride_bytes, dim, &L)) return 1;
+    if (stage_batch(ctx, fn, p, pairs, n_pairs, stride_bytes, dim, &L, dev)) return 1;
     if (L.real_src == 0) return 0;
-    if (!idx || !dist || !count) return b200m_fail_msg(ctx, "b200m_knn_batch: null output pointer");
+    if (!idx || !dist || !count) return b200m_fail_msg(ctx, f + ": null output pointer");
     const int k = p->k;
     const size_t S = L.n_rows[0];
     cudaStream_t st = ctx->stream;
@@ -182,8 +266,17 @@ int b200m_knn_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pai
     if (b200m_knn_rows(ctx, p, 0, 0, S, nullptr, ctx->ws_fidx.as<int32_t>(), ctx->ws_fdist.as<float>(), ctx->ws_fcnt.as<int32_t>(),
                        &L.seg[0]))
         return 1;
-    // the pairs' real rows back to back, with pair-local train indices (the reverse-table buffers are free here)
+    // the pairs' real rows back to back, with pair-local train indices (the reverse-table buffers are free here; a device
+    // call writes the caller's arrays directly)
     const size_t R = L.real_src;
+    if (dev) {
+        localize_lists_kernel<<<(unsigned) ((S + 255) / 256), 256, 0, st>>>(
+            ctx->ws_fidx.as<int32_t>(), ctx->ws_fdist.as<float>(), ctx->ws_fcnt.as<int32_t>(), S, k, L.block_pair, L.pair_info,
+            idx, dist, count);
+        CK(cudaGetLastError());
+        ctx->stats.launches += 1;
+        return 0;
+    }
     CK(ctx->ws_ridx.reserve(sizeof(int32_t) * R * k));
     CK(ctx->ws_rdist.reserve(sizeof(float) * R * k));
     CK(ctx->ws_rcnt.reserve(sizeof(int32_t) * R));
@@ -199,19 +292,25 @@ int b200m_knn_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pai
     return 0;
 }
 
-int b200m_match_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
-                      const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap, size_t *offsets, float *avg) {
+// dev: b200m_match_batch_device (device descriptors and thresholds, records to the caller's device buffer)
+int match_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                size_t stride_bytes, int dim, const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
+                size_t *offsets, float *avg) {
     REQUIRE_CTX();
     if (check_params(ctx, p)) return 1;
-    if (p->mode == B200M_MODE_KNN_ONLY) return b200m_fail_msg(ctx, "b200m_match_batch: use b200m_knn_batch for raw k-lists");
+    const std::string f(fn);
+    if (p->mode == B200M_MODE_KNN_ONLY) return b200m_fail_msg(ctx, f + ": use b200m_knn_batch for raw k-lists");
     if (p->mode == B200M_MODE_CLUSTER)
-        return b200m_fail_msg(ctx, "b200m_match_batch: the cluster filter needs keypoint coordinates, use b200m_match_cluster");
-    if (!offsets) return b200m_fail_msg(ctx, "b200m_match_batch: null offsets");
+        return b200m_fail_msg(ctx, f + ": the cluster filter needs keypoint coordinates, use b200m_match_cluster");
+    if (!offsets) return b200m_fail_msg(ctx, f + ": null offsets");
     if ((thr_src == nullptr) != (thr_tgt == nullptr))
-        return b200m_fail_msg(ctx, "b200m_match_batch: give both threshold arrays or neither");
+        return b200m_fail_msg(ctx, f + ": give both threshold arrays or neither");
+    if (dev && (check_device_ptr(ctx, f + ": thr_src", thr_src) || check_device_ptr(ctx, f + ": thr_tgt", thr_tgt) ||
+                check_device_ptr(ctx, f + ": out", out)))
+        return 1;
     for (int i = 0; i <= n_pairs; ++i) offsets[i] = 0;
     BatchLayout L;
-    if (stage_batch(ctx, "b200m_match_batch", p, pairs, n_pairs, stride_bytes, dim, &L)) return 1;
+    if (stage_batch(ctx, fn, p, pairs, n_pairs, stride_bytes, dim, &L, dev, thr_src, thr_tgt)) return 1;
     if (L.real_src == 0) {
         if (avg)
             for (int i = 0; i < n_pairs; ++i) avg[i] = 3.402823466e+38F;   // FLT_MAX, reference include/matching.h:41
@@ -236,7 +335,16 @@ int b200m_match_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *p
             return 1;
     }
     const float *d_thr_s = nullptr, *d_thr_t = nullptr;
-    if (thr_src && T) {   // the pairs' thresholds in the padded layout (gap rows never produce a record)
+    if (thr_src && T && dev) {   // the gather kernel files the device thresholds in the padded layout
+        CK(ctx->ws_thr[0].reserve(sizeof(float) * S));
+        CK(ctx->ws_thr[1].reserve(sizeof(float) * T));
+        for (int s = 0; s < 2; ++s) {
+            CK(launch_gather_sets(L.thr_sets[s], n_pairs, L.max_rows[s], 1, 1, ctx->ws_thr[s].p, st));
+            ctx->stats.launches += 1;
+        }
+        d_thr_s = ctx->ws_thr[0].as<float>();
+        d_thr_t = ctx->ws_thr[1].as<float>();
+    } else if (thr_src && T) {   // the pairs' thresholds in the padded layout (gap rows never produce a record)
         std::vector<float> hs(S, 0.f), ht(T, 0.f);
         size_t cs = 0, ct = 0, os = 0, ot = 0;
         for (int i = 0; i < n_pairs; ++i) {
@@ -279,13 +387,44 @@ int b200m_match_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *p
     const unsigned *cnt = reinterpret_cast<const unsigned *>(res.data() + 16);
     for (int i = 0; i < n_pairs; ++i) offsets[i + 1] = offsets[i] + cnt[i];
     if (avg) memcpy(avg, res.data() + 16 + align16(sizeof(unsigned) * n_pairs), sizeof(float) * n_pairs);
-    if (n > cap) return b200m_fail_msg(ctx, "b200m_match_batch: output capacity too small (" + std::to_string(n) + " correspondences)");
+    if (n > cap) return b200m_fail_msg(ctx, f + ": output capacity too small (" + std::to_string(n) + " correspondences)");
     if (n) {
-        if (!out) return b200m_fail_msg(ctx, "b200m_match_batch: null output buffer");
+        if (!out) return b200m_fail_msg(ctx, f + ": null output buffer");
+        if (dev) {   // stream-ordered: the caller's next work on the stream sees the records
+            CK(cudaMemcpyAsync(out, ctx->ws_corr.p, sizeof(b200m_corr) * n, cudaMemcpyDeviceToDevice, st));
+            return 0;
+        }
         CK(cudaMemcpyAsync(out, ctx->ws_corr.p, sizeof(b200m_corr) * n, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
     }
     return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int b200m_knn_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
+                    int32_t *idx, float *dist, int32_t *count) {
+    return knn_batch(ctx, "b200m_knn_batch", false, p, pairs, n_pairs, stride_bytes, dim, idx, dist, count);
+}
+
+int b200m_knn_batch_device(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes,
+                           int dim, int32_t *d_idx, float *d_dist, int32_t *d_count) {
+    return knn_batch(ctx, "b200m_knn_batch_device", true, p, pairs, n_pairs, stride_bytes, dim, d_idx, d_dist, d_count);
+}
+
+int b200m_match_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
+                      const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap, size_t *offsets, float *avg) {
+    return match_batch(ctx, "b200m_match_batch", false, p, pairs, n_pairs, stride_bytes, dim, thr_src, thr_tgt, out, cap, offsets,
+                       avg);
+}
+
+int b200m_match_batch_device(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes,
+                             int dim, const float *d_thr_src, const float *d_thr_tgt, b200m_corr *d_out, size_t cap, size_t *offsets,
+                             float *avg) {
+    return match_batch(ctx, "b200m_match_batch_device", true, p, pairs, n_pairs, stride_bytes, dim, d_thr_src, d_thr_tgt, d_out, cap,
+                       offsets, avg);
 }
 
 }  // extern "C"

@@ -130,6 +130,13 @@ struct SegTable {
     int max_tiles = 0;
 };
 
+// A device batch call's descriptor set in the padded layout: `rows` rows at `base` (the caller's device memory, the
+// call's stride apart) fill padded rows [first, first + rows) of their side.
+struct alignas(16) SetRef {
+    const float *base;
+    int first, rows;
+};
+
 inline size_t pad_rows(size_t n) { return (n + B200M_TILE_N - 1) / B200M_TILE_N * B200M_TILE_N; }
 inline size_t align16(size_t b) { return (b + 15) & ~(size_t) 15; }
 
@@ -146,18 +153,40 @@ struct BatchLayout {
     unsigned *counts = nullptr;
     float *avgs = nullptr;
     size_t result_bytes = 0;
+    size_t max_rows[2] = {0, 0};                   // largest set per side
+    const struct GatherSet *thr_sets[2] = {nullptr, nullptr};   // device calls with thresholds: [n_pairs] per side
 };
 // Validates the pairs, packs both sides in the padded layout (replacing what b200m_upload put in the context) and uploads
-// the segment tables into ctx->ws_batch.
+// the segment tables into ctx->ws_batch.  dev: every descriptor pointer is a device pointer of the context's device
+// (checked; the segmented pack reads the sets in place); d_thr_src / d_thr_tgt (dev only): the concatenated device
+// thresholds, for which gather tables into the padded layout go up with the segment tables.
 int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
-                size_t stride_bytes, int dim, BatchLayout *L);
+                size_t stride_bytes, int dim, BatchLayout *L, bool dev = false, const float *d_thr_src = nullptr,
+                const float *d_thr_tgt = nullptr);
+
+// Device batch calls: `rows` rows of `w` 4-byte words, src_stride words apart at `src`, go to rows dst_row.. of a
+// destination (dst_stride words apart).  src = null writes the identity (row r -> r, w = 1): a NULL index map.
+struct alignas(16) GatherSet {
+    const void *src;
+    long long src_stride;
+    int dst_row, rows;
+    int pad;
+};
+// batch.cu: one launch for n_sets sets (max_rows: the largest)
+cudaError_t launch_gather_sets(const GatherSet *d_sets, int n_sets, size_t max_rows, int w, size_t dst_stride_words, void *dst,
+                               cudaStream_t st);
+// 0 when ptr is null or device / managed memory of the context's device; else fails with "<where> is not device memory ..."
+int check_device_ptr(b200m_ctx *ctx, const std::string &where, const void *ptr);
 
 // ---- kernel launchers (one translation unit each) ---------------------------
 // pack.cu
 // dense FP32 copy + validity + per-CTA column statistics (sum, min, max over valid rows) into `stats`
 // (pack_stats_bytes() bytes), which launch_tc_prepare turns into the common centre and FP16 scale
+// With `sets` (device batch calls) the rows come from the caller's sets instead of `aos`: padded row r is row
+// r - sets[b].first of set b = seg_blk[r / 256] (a gap row past the set's end packs as NaN, see pack.cu)
 cudaError_t launch_pack_f32(const float *aos, size_t n, size_t stride_bytes, int dim, int dp,
-                            float *f32, uint8_t *valid, float *stats, int sm_count, cudaStream_t st);
+                            float *f32, uint8_t *valid, float *stats, int sm_count, cudaStream_t st,
+                            const int32_t *seg_blk = nullptr, const SetRef *sets = nullptr);
 size_t pack_stats_bytes(int sm_count, int dp);
 cudaError_t launch_tc_prepare(b200m_ctx *ctx);   // centre/scale + FP16 operand tiles for both sides
 
@@ -287,7 +316,9 @@ int check_upload_args(b200m_ctx *ctx, int side, const float *base, size_t n, siz
 bool is_pageable(const void *p);
 int staged_h2d(b200m_ctx *ctx, void *dst, const void *src, size_t bytes);   // pageable host -> device through pinned buffers
 // pack `n` rows of device AoS data into side `side` (b200m_upload's device half)
-int upload_common(b200m_ctx *ctx, int side, const float *device_aos, size_t n, size_t stride_bytes, int dim, int64_t index_offset);
+// with `sets` the segmented pack of a device batch call (see launch_pack_f32)
+int upload_common(b200m_ctx *ctx, int side, const float *device_aos, size_t n, size_t stride_bytes, int dim, int64_t index_offset,
+                  const int32_t *seg_blk = nullptr, const SetRef *sets = nullptr);
 }
 
 // cluster.cu

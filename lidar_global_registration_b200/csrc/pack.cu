@@ -31,10 +31,15 @@ __host__ __device__ inline size_t stats_floats(int dp) { return (size_t) 3 * dp 
 // copied, its validity decided (every value finite), and -- for valid rows only -- folded into the lane's running
 // column sum / min / max, from which tc_prepare derives the common centre and the FP16 scale without reading the data
 // again.
-template <int NI>
+// SEG (device batch calls): `aos` is unused; row `row` of the padded layout belongs to set seg_blk[row / 256], which
+// starts at padded row sets[.].first and has sets[.].rows rows at sets[.].base + local * stride_floats.  The rows after
+// a set's last row (up to its next multiple of 256) are written as the staging path's 0xFF bytes pack: NaN (all ones)
+// in the descriptor columns, 0 in the padding columns, invalid.
+template <int NI, bool SEG>
 __global__ void __launch_bounds__(kPackWarps * 32)
 pack_f32_kernel(const float *__restrict__ aos, size_t n, size_t stride_floats, int dim, int dp,
-                float *__restrict__ f32, uint8_t *__restrict__ valid, float *__restrict__ stats) {
+                float *__restrict__ f32, uint8_t *__restrict__ valid, float *__restrict__ stats,
+                const int32_t *__restrict__ seg_blk, const SetRef *__restrict__ sets) {
     extern __shared__ float sh[];   // [3][dp]
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     float sum[NI], mn[NI], mx[NI];
@@ -42,15 +47,28 @@ pack_f32_kernel(const float *__restrict__ aos, size_t n, size_t stride_floats, i
     for (int i = 0; i < NI; ++i) { sum[i] = 0.f; mn[i] = INFINITY; mx[i] = -INFINITY; }
     float cnt = 0.f;
     for (size_t row = (size_t) blockIdx.x * kPackWarps + warp; row < n; row += (size_t) gridDim.x * kPackWarps) {
-        const float *src = aos + row * stride_floats;
         float *dst = f32 + row * (size_t) dp;
         float v[NI];
         bool ok = true;
+        if constexpr (SEG) {
+            const SetRef set = sets[seg_blk[row / B200M_TILE_N]];
+            const size_t local = row - (size_t) set.first;
+            const bool gap = local >= (size_t) set.rows;
+            const float *src = set.base + (gap ? 0 : local) * stride_floats;
 #pragma unroll
-        for (int i = 0; i < NI; ++i) {
-            const int d = lane + 32 * i;
-            v[i] = d < dim ? __ldg(src + d) : 0.f;
-            ok = ok && isfinite(v[i]);
+            for (int i = 0; i < NI; ++i) {
+                const int d = lane + 32 * i;
+                v[i] = d < dim ? (gap ? __int_as_float(-1) : __ldg(src + d)) : 0.f;
+                ok = ok && isfinite(v[i]);
+            }
+        } else {
+            const float *src = aos + row * stride_floats;
+#pragma unroll
+            for (int i = 0; i < NI; ++i) {
+                const int d = lane + 32 * i;
+                v[i] = d < dim ? __ldg(src + d) : 0.f;
+                ok = ok && isfinite(v[i]);
+            }
         }
 #pragma unroll
         for (int i = 0; i < NI; ++i) {
@@ -241,13 +259,21 @@ int pack_stats_blocks(int sm_count) { return sm_count * 2; }
 size_t pack_stats_bytes(int sm_count, int dp) { return sizeof(float) * (size_t) pack_stats_blocks(sm_count) * stats_floats(dp); }
 
 cudaError_t launch_pack_f32(const float *aos, size_t n, size_t stride_bytes, int dim, int dp,
-                            float *f32, uint8_t *valid, float *stats, int sm_count, cudaStream_t st) {
+                            float *f32, uint8_t *valid, float *stats, int sm_count, cudaStream_t st,
+                            const int32_t *seg_blk, const SetRef *sets) {
     if (n == 0) return cudaSuccess;
     const unsigned blocks = (unsigned) pack_stats_blocks(sm_count);
     const size_t smem = sizeof(float) * 3 * (size_t) dp;
     const int ni = (dp + 31) / 32;
 #define B200M_PACK_CASE(NI)                                                                                          \
-    pack_f32_kernel<NI><<<blocks, kPackWarps * 32, smem, st>>>(aos, n, stride_bytes / 4, dim, dp, f32, valid, stats)
+    do {                                                                                                             \
+        if (sets)                                                                                                    \
+            pack_f32_kernel<NI, true><<<blocks, kPackWarps * 32, smem, st>>>(aos, n, stride_bytes / 4, dim, dp, f32, \
+                                                                             valid, stats, seg_blk, sets);           \
+        else                                                                                                         \
+            pack_f32_kernel<NI, false><<<blocks, kPackWarps * 32, smem, st>>>(aos, n, stride_bytes / 4, dim, dp, f32,\
+                                                                              valid, stats, nullptr, nullptr);       \
+    } while (0)
     if (ni <= 2) B200M_PACK_CASE(2);
     else if (ni <= 5) B200M_PACK_CASE(5);
     else if (ni <= 11) B200M_PACK_CASE(11);

@@ -121,11 +121,14 @@ void wide_batch_release(b200m_ctx *ctx) {
 
 namespace {
 
-// gated = false: b200m_match_multiscale_batch; true: the guessed form, whose kNN passes are gated by `radius`
-int match_multiscale_batch(b200m_ctx *ctx, const char *name, const b200m_params *p, const b200m_wide_pair *pairs, bool gated,
-                           const b200m_local_pair *locals, int n_pairs, size_t stride_bytes, int dim, size_t xyz_stride_bytes,
-                           int cluster_k, float radius, const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
-                           size_t *offsets, float *avg) {
+// gated = false: b200m_match_multiscale_batch; true: the guessed form, whose kNN passes are gated by `radius`.
+// dev: the *_device forms -- every data pointer of the pairs, the thresholds and `out` are device pointers (checked before
+// anything is queued); descriptors are packed in place, maps and coordinates are filed by gather_sets_kernel, thresholds
+// are read in place and the records stay on the device.
+int match_multiscale_batch(b200m_ctx *ctx, const char *name, bool dev, const b200m_params *p, const b200m_wide_pair *pairs,
+                           bool gated, const b200m_local_pair *locals, int n_pairs, size_t stride_bytes, int dim,
+                           size_t xyz_stride_bytes, int cluster_k, float radius, const float *thr_src, const float *thr_tgt,
+                           b200m_corr *out, size_t cap, size_t *offsets, float *avg) {
     const std::string fn = std::string(name) + ": ";
     if (!ctx) return b200m_fail_msg(nullptr, "null context");
     CK(cudaSetDevice(ctx->device));
@@ -163,6 +166,20 @@ int match_multiscale_batch(b200m_ctx *ctx, const char *name, const b200m_params 
             tot[1] >= ((size_t) 1 << 31))
             return b200m_fail_msg(ctx, pi + "more than 2^31-1 keypoints per side in the batch");
         eff[i] = w.n_src_kps ? w.n_scales : 0;
+        if (dev) {
+            if (check_device_ptr(ctx, pi + "src_kps_xyz", w.src_kps_xyz) || check_device_ptr(ctx, pi + "tgt_kps_xyz", w.tgt_kps_xyz))
+                return 1;
+            if (gated && (check_device_ptr(ctx, pi + "src_kps_moved", locals[i].src_kps_moved) ||
+                          check_device_ptr(ctx, pi + "tgt_kps_moved", locals[i].tgt_kps_moved)))
+                return 1;
+            for (int s = 0; s < w.n_scales; ++s) {
+                const b200m_scale &sc = w.scales[s];
+                const std::string ps = pi + "scale " + std::to_string(s) + ": ";
+                if (check_device_ptr(ctx, ps + "src_desc", sc.src_desc) || check_device_ptr(ctx, ps + "tgt_desc", sc.tgt_desc) ||
+                    check_device_ptr(ctx, ps + "src_map", sc.src_map) || check_device_ptr(ctx, ps + "tgt_map", sc.tgt_map))
+                    return 1;
+            }
+        }
         if (!w.n_src_kps) continue;
         if ((w.n_tgt_kps && !w.tgt_kps_xyz) || (two_way && !w.src_kps_xyz))
             return b200m_fail_msg(ctx, pi + "null keypoint coordinates");
@@ -175,6 +192,9 @@ int match_multiscale_batch(b200m_ctx *ctx, const char *name, const b200m_params 
         }
         n_scales = std::max(n_scales, w.n_scales);
     }
+    if (dev && (check_device_ptr(ctx, fn + "thr_src", thr_src) || check_device_ptr(ctx, fn + "thr_tgt", thr_tgt) ||
+                check_device_ptr(ctx, fn + "out", out)))
+        return 1;
     kp_off[0][n_pairs] = (int32_t) tot[0];
     kp_off[1][n_pairs] = (int32_t) tot[1];
     const size_t NS = tot[0], NT = tot[1];
@@ -214,12 +234,26 @@ int match_multiscale_batch(b200m_ctx *ctx, const char *name, const b200m_params 
             o = align16(o + sizeof(int32_t) * (rows_pad[side][s] / B200M_TILE_N));
         }
     }
+    // device calls: the gather tables of the maps (every side, scale and pair) and of the four coordinate tables; the maps
+    // come last and are not uploaded (gather_sets_kernel fills their real rows, gap rows are never read)
+    size_t o_gmap = 0, o_gxyz = 0, n_gmap = 0;
+    if (dev) {
+        for (int side = 0; side < 2; ++side)
+            for (int s = 0; s < n_scales; ++s)
+                for (int i = 0; i < n_pairs; ++i) n_gmap += n_rows(i, s, side) ? 1 : 0;
+        o_gmap = o;
+        o = align16(o + sizeof(GatherSet) * n_gmap);
+        o_gxyz = o;   // [4][n_pairs]: xyz_t, xyz_s, mov_s, mov_t
+        o = align16(o + sizeof(GatherSet) * 4 * n_pairs);
+    }
+    const size_t maps_begin = o;
     for (int side = 0; side < 2; ++side)
         for (int s = 0; s < n_scales; ++s) {
             o_map[side].push_back(o);
             o = align16(o + sizeof(int32_t) * rows_pad[side][s]);
         }
-    std::vector<char> h(o, 0);
+    const size_t table_bytes = o;
+    std::vector<char> h(dev ? maps_begin : table_bytes, 0);
     *reinterpret_cast<unsigned long long *>(h.data() + o_bad) = ~0ull;
     memcpy(h.data() + o_off0, kp_off[0].data(), sizeof(int32_t) * (n_pairs + 1));
     memcpy(h.data() + o_off1, kp_off[1].data(), sizeof(int32_t) * (n_pairs + 1));
@@ -228,6 +262,9 @@ int match_multiscale_batch(b200m_ctx *ctx, const char *name, const b200m_params 
         reinterpret_cast<float *>(h.data() + o_rad1)[i] = pairs[i].iss_radius_tgt;
         reinterpret_cast<int2 *>(h.data() + o_segs)[i] = make_int2(kp_off[0][i], (int) pairs[i].n_src_kps);
     }
+    GatherSet *gmap = dev ? reinterpret_cast<GatherSet *>(h.data() + o_gmap) : nullptr;
+    size_t max_map_rows = 0;
+    n_gmap = 0;
     for (int s = 0; s < n_scales; ++s) {
         size_t start[2] = {0, 0};
         int4 *rows = reinterpret_cast<int4 *>(h.data() + o_rows[s]);
@@ -237,21 +274,49 @@ int match_multiscale_batch(b200m_ctx *ctx, const char *name, const b200m_params 
             for (int side = 0; side < 2; ++side) {
                 int32_t *blk = reinterpret_cast<int32_t *>(h.data() + o_blk[side][s]);
                 for (size_t b = start[side] / B200M_TILE_N; b < (start[side] + pad_rows(n[side])) / B200M_TILE_N; ++b) blk[b] = i;
-                int32_t *map = reinterpret_cast<int32_t *>(h.data() + o_map[side][s]) + start[side];
                 const int32_t *given = n[side] ? (side ? pairs[i].scales[s].tgt_map : pairs[i].scales[s].src_map) : nullptr;
-                if (given)
-                    memcpy(map, given, sizeof(int32_t) * n[side]);
-                else
-                    for (size_t r = 0; r < n[side]; ++r) map[r] = (int32_t) r;
+                if (dev) {   // filed on the device, after the table upload (a NULL map: identity)
+                    if (n[side]) {
+                        gmap[n_gmap++] = GatherSet{given, 1, (int) (o_map[side][s] / 4 + start[side]), (int) n[side], 0};
+                        max_map_rows = std::max(max_map_rows, n[side]);
+                    }
+                } else {
+                    int32_t *map = reinterpret_cast<int32_t *>(h.data() + o_map[side][s]) + start[side];
+                    if (given)
+                        memcpy(map, given, sizeof(int32_t) * n[side]);
+                    else
+                        for (size_t r = 0; r < n[side]; ++r) map[r] = (int32_t) r;
+                }
                 start[side] += pad_rows(n[side]);
             }
         }
     }
+    // coordinates of the pairs that take part (the host copy's rule): the first three floats of a row, which is all the
+    // gather of local.cu, the vote and knn3d read
+    GatherSet *gxyz = dev ? reinterpret_cast<GatherSet *>(h.data() + o_gxyz) : nullptr;
+    size_t max_kps[2] = {0, 0};
+    if (dev) {
+        const long long xs = (long long) (xyz_stride_bytes / 4);
+        for (int i = 0; i < n_pairs; ++i) {
+            const b200m_wide_pair &w = pairs[i];
+            if (!w.n_src_kps) continue;
+            gxyz[i] = GatherSet{w.tgt_kps_xyz, xs, kp_off[1][i], (int) w.n_tgt_kps, 0};
+            if (two_way) gxyz[n_pairs + i] = GatherSet{w.src_kps_xyz, xs, kp_off[0][i], (int) w.n_src_kps, 0};
+            if (gated) gxyz[2 * n_pairs + i] = GatherSet{locals[i].src_kps_moved, xs, kp_off[0][i], (int) w.n_src_kps, 0};
+            if (gated && two_way) gxyz[3 * n_pairs + i] = GatherSet{locals[i].tgt_kps_moved, xs, kp_off[1][i], (int) w.n_tgt_kps, 0};
+            max_kps[0] = std::max(max_kps[0], w.n_src_kps);
+            max_kps[1] = std::max(max_kps[1], w.n_tgt_kps);
+        }
+    }
     cudaStream_t st = ctx->stream;
     WideBatchState *ws = wb_state(ctx);
-    CK(ws->tables.reserve(h.size()));
+    CK(ws->tables.reserve(table_bytes));
     char *d = ws->tables.as<char>();
     CK(cudaMemcpyAsync(d, h.data(), h.size(), cudaMemcpyHostToDevice, st));
+    if (dev) {
+        CK(launch_gather_sets(reinterpret_cast<const GatherSet *>(d + o_gmap), (int) n_gmap, max_map_rows, 1, 1, d, st));
+        ctx->stats.launches += n_gmap ? 1 : 0;
+    }
     unsigned long long *d_n = reinterpret_cast<unsigned long long *>(d + o_n), *d_bad = reinterpret_cast<unsigned long long *>(d + o_bad);
     unsigned *d_counts = reinterpret_cast<unsigned *>(d + o_counts);
     float *d_avgs = reinterpret_cast<float *>(d + o_avgs);
@@ -262,7 +327,19 @@ int match_multiscale_batch(b200m_ctx *ctx, const char *name, const b200m_params 
     if (two_way) CK(ws->xyz_s.reserve(NS * xyz_stride_bytes + 16));
     if (gated) CK(ws->mov_s.reserve(NS * xyz_stride_bytes + 16));
     if (gated && two_way) CK(ws->mov_t.reserve(NT * xyz_stride_bytes + 16));
-    for (int i = 0; i < n_pairs; ++i) {
+    if (dev) {
+        const size_t xs = xyz_stride_bytes / 4;
+        const GatherSet *g = reinterpret_cast<const GatherSet *>(d + o_gxyz);
+        DevBuf *dst[4] = {&ws->xyz_t, &ws->xyz_s, &ws->mov_s, &ws->mov_t};
+        const bool used[4] = {true, two_way, gated, gated && two_way};
+        const size_t mx[4] = {max_kps[1], max_kps[0], max_kps[0], max_kps[1]};
+        for (int t = 0; t < 4; ++t) {
+            if (!used[t] || !mx[t]) continue;
+            CK(launch_gather_sets(g + (size_t) t * n_pairs, n_pairs, mx[t], 3, xs, dst[t]->p, st));
+            ctx->stats.launches += 1;
+        }
+    }
+    for (int i = 0; i < n_pairs && !dev; ++i) {
         if (!pairs[i].n_src_kps) continue;
         if (copy_xyz(ctx, ws->xyz_t.as<char>() + (size_t) kp_off[1][i] * xyz_stride_bytes, pairs[i].tgt_kps_xyz, pairs[i].n_tgt_kps,
                      xyz_stride_bytes))
@@ -300,7 +377,7 @@ int match_multiscale_batch(b200m_ctx *ctx, const char *name, const b200m_params 
                                n_rows(i, s, 1)};
         }
         BatchLayout L;
-        if (stage_batch(ctx, name, &pk, sp.data(), n_pairs, stride_bytes, dim, &L)) return 1;
+        if (stage_batch(ctx, name, &pk, sp.data(), n_pairs, stride_bytes, dim, &L, dev)) return 1;
         const size_t S = L.n_rows[0], T = L.n_rows[1], n_max = std::max(S, T);
         CK(ws->kidx.reserve(sizeof(int32_t) * (n_max * k + 1)));
         CK(ws->kdist.reserve(sizeof(float) * (n_max * k + 1)));
@@ -351,7 +428,10 @@ int match_multiscale_batch(b200m_ctx *ctx, const char *name, const b200m_params 
                                         ws->vri.as<int32_t>(), ws->vrd.as<float>(), ws->vrc.as<int32_t>()))
         return 1;
     const float *d_thr_s = nullptr, *d_thr_t = nullptr;
-    if (thr_src && NT) {   // keypoint tables are dense: the concatenated thresholds are indexed by the global ids as they are
+    if (thr_src && NT && dev) {   // the device thresholds are the dense keypoint-table layout already
+        d_thr_s = thr_src;
+        d_thr_t = thr_tgt;
+    } else if (thr_src && NT) {   // keypoint tables are dense: the concatenated thresholds are indexed by the global ids as they are
         CK(ctx->ws_thr[0].reserve(sizeof(float) * NS));
         CK(ctx->ws_thr[1].reserve(sizeof(float) * NT));
         CK(cudaMemcpyAsync(ctx->ws_thr[0].p, thr_src, sizeof(float) * NS, cudaMemcpyHostToDevice, st));
@@ -398,6 +478,10 @@ int match_multiscale_batch(b200m_ctx *ctx, const char *name, const b200m_params 
     if (n > cap) return b200m_fail_msg(ctx, fn + "output capacity too small (" + std::to_string(n) + " correspondences)");
     if (n) {
         if (!out) return b200m_fail_msg(ctx, fn + "null output buffer");
+        if (dev) {   // stream-ordered: the caller's next work on the stream sees the records
+            CK(cudaMemcpyAsync(out, ctx->ws_corr.p, sizeof(b200m_corr) * n, cudaMemcpyDeviceToDevice, st));
+            return 0;
+        }
         CK(cudaMemcpyAsync(out, ctx->ws_corr.p, sizeof(b200m_corr) * n, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
     }
@@ -410,8 +494,16 @@ extern "C" int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *
                                             size_t stride_bytes, int dim, size_t xyz_stride_bytes, int cluster_k,
                                             const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
                                             size_t *offsets, float *avg) {
-    return match_multiscale_batch(ctx, "b200m_match_multiscale_batch", p, pairs, false, nullptr, n_pairs, stride_bytes, dim,
+    return match_multiscale_batch(ctx, "b200m_match_multiscale_batch", false, p, pairs, false, nullptr, n_pairs, stride_bytes, dim,
                                   xyz_stride_bytes, cluster_k, 0.f, thr_src, thr_tgt, out, cap, offsets, avg);
+}
+
+extern "C" int b200m_match_multiscale_batch_device(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs, int n_pairs,
+                                                   size_t stride_bytes, int dim, size_t xyz_stride_bytes, int cluster_k,
+                                                   const float *d_thr_src, const float *d_thr_tgt, b200m_corr *d_out, size_t cap,
+                                                   size_t *offsets, float *avg) {
+    return match_multiscale_batch(ctx, "b200m_match_multiscale_batch_device", true, p, pairs, false, nullptr, n_pairs, stride_bytes,
+                                  dim, xyz_stride_bytes, cluster_k, 0.f, d_thr_src, d_thr_tgt, d_out, cap, offsets, avg);
 }
 
 extern "C" int b200m_match_multiscale_local_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs,
@@ -419,6 +511,16 @@ extern "C" int b200m_match_multiscale_local_batch(b200m_ctx *ctx, const b200m_pa
                                                   size_t xyz_stride_bytes, int cluster_k, float match_search_radius,
                                                   const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
                                                   size_t *offsets, float *avg) {
-    return match_multiscale_batch(ctx, "b200m_match_multiscale_local_batch", p, pairs, true, locals, n_pairs, stride_bytes, dim,
-                                  xyz_stride_bytes, cluster_k, match_search_radius, thr_src, thr_tgt, out, cap, offsets, avg);
+    return match_multiscale_batch(ctx, "b200m_match_multiscale_local_batch", false, p, pairs, true, locals, n_pairs, stride_bytes,
+                                  dim, xyz_stride_bytes, cluster_k, match_search_radius, thr_src, thr_tgt, out, cap, offsets, avg);
+}
+
+extern "C" int b200m_match_multiscale_local_batch_device(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs,
+                                                         const b200m_local_pair *locals, int n_pairs, size_t stride_bytes, int dim,
+                                                         size_t xyz_stride_bytes, int cluster_k, float match_search_radius,
+                                                         const float *d_thr_src, const float *d_thr_tgt, b200m_corr *d_out,
+                                                         size_t cap, size_t *offsets, float *avg) {
+    return match_multiscale_batch(ctx, "b200m_match_multiscale_local_batch_device", true, p, pairs, true, locals, n_pairs,
+                                  stride_bytes, dim, xyz_stride_bytes, cluster_k, match_search_radius, d_thr_src, d_thr_tgt, d_out,
+                                  cap, offsets, avg);
 }

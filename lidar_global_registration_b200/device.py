@@ -1,6 +1,6 @@
 """Device-resident and multi-GPU drivers of the matcher on torch tensors (HBM buffers, the current torch stream).
 
-    GpuBackend      one b200m context working on torch device buffers (no host copies)
+    GpuBackend      one b200m context working on torch device buffers (no host copies), single pairs and batches
     ShardedMatcher  SURVEY 8e, one process per GPU: query-sharded / target-replicated matcher and the target-sharded kNN.
                     With a GpuBackend this is a THIN caller of the library -- partitioning, the NCCL exchange step and
                     the merge live in libb200match.so (csrc/multi.cu: b200m_match_sharded_device,
@@ -147,6 +147,165 @@ class GpuBackend:
                 rev = self.knn(k, 1, 0, nt)
         return self.filter(k, mode, 0, nq, fwd, rev, nt if rev is not None else 0, ratio_thr, distance_thr,
                            want_avg=want_avg)
+
+    # -- batches on device-resident sets (b200m_*_batch_device) ------------------------------------------
+    def _check_rows(self, t, what, dtype=torch.float32, min_cols=1):
+        """A 2-D tensor of `dtype` with unit column stride on this backend's device -> its row stride in elements (None
+        for an empty set)."""
+        if not isinstance(t, torch.Tensor) or t.dtype != dtype or t.dim() != 2 or t.device != self.device:
+            raise M.B200MatchError("%s: must be a 2-D %s tensor on %s" % (what, dtype, self.device))
+        if t.shape[1] < min_cols:
+            raise M.B200MatchError("%s: rows must have at least %d columns" % (what, min_cols))
+        if t.shape[0] == 0:
+            return None
+        if t.stride(1) != 1 and t.shape[1] > 1:
+            raise M.B200MatchError("%s: the columns must be contiguous (unit column stride)" % what)
+        return t.stride(0)
+
+    def _check_vec(self, t, what, n, dtype):
+        if not isinstance(t, torch.Tensor) or t.dtype != dtype or t.dim() != 1 or t.device != self.device:
+            raise M.B200MatchError("%s: must be a 1-D %s tensor on %s" % (what, dtype, self.device))
+        if t.shape[0] != n:
+            raise M.B200MatchError("%s: %d entries, %d expected" % (what, t.shape[0], n))
+        if n > 1 and t.stride(0) != 1:
+            raise M.B200MatchError("%s: must be contiguous" % what)
+
+    @staticmethod
+    def _one_stride(strides, what):
+        got = {st for st in strides if st is not None}
+        if len(got) > 1:
+            raise M.B200MatchError("%s: every set of the batch must have the same row stride (got %s)" % (what, sorted(got)))
+        return got.pop() if got else None
+
+    @staticmethod
+    def _ptr(t):
+        return t.data_ptr() if t is not None and t.numel() else 0
+
+    def _set_pairs(self, pairs, dim):
+        """[(src, tgt), ...] float32 CUDA tensors -> ([(ptr, n, ptr, n)], row stride in bytes)."""
+        strides = []
+        for i, pr in enumerate(pairs):
+            if len(pr) != 2:
+                raise M.B200MatchError("pair %d: a (source rows, target rows) tuple is needed" % i)
+            for side, t in zip(("src", "tgt"), pr):
+                strides.append(self._check_rows(t, "pair %d: %s" % (i, side), min_cols=dim))
+        stride = self._one_stride(strides, "batch") or dim
+        return [(self._ptr(s), s.shape[0], self._ptr(t), t.shape[0]) for s, t in pairs], stride * 4
+
+    def _thresholds(self, thr_src, thr_tgt, counts):
+        """one 1-D float32 tensor per pair and side -> the two concatenations (device tensors) or (None, None)."""
+        if (thr_src is None) != (thr_tgt is None):
+            raise M.B200MatchError("give both threshold lists or neither")
+        if thr_src is None:
+            return None, None
+        if len(thr_src) != len(counts) or len(thr_tgt) != len(counts):
+            raise M.B200MatchError("one threshold array per pair and side")
+        for i, (ns, nt) in enumerate(counts):
+            self._check_vec(thr_src[i], "pair %d: thr_src" % i, ns, torch.float32)
+            self._check_vec(thr_tgt[i], "pair %d: thr_tgt" % i, nt, torch.float32)
+        pad = [torch.zeros(1, dtype=torch.float32, device=self.device)]
+        return torch.cat(list(thr_src) + pad), torch.cat(list(thr_tgt) + pad)
+
+    def knn_batch(self, k, pairs, dim):
+        """b200m_knn_batch_device on [(source rows, target rows), ...] (float32 CUDA tensors [n, >= dim], unit column
+        stride, one row stride in the batch; row slices of a larger tensor and one tensor in many pairs are fine).
+        -> one (idx, dist, cnt) CUDA tensor view per pair, equal to Context.knn_batch on the same data."""
+        ptrs, stride = self._set_pairs(pairs, dim)
+        total = sum(p[1] for p in ptrs)
+        idx = torch.empty((total, k), dtype=torch.int32, device=self.device)
+        dist = torch.empty((total, k), dtype=torch.float32, device=self.device)
+        cnt = torch.empty((total,), dtype=torch.int32, device=self.device)
+        self.use_torch_stream()
+        self.ctx.knn_batch_device(k, ptrs, stride, dim, self._ptr(idx), self._ptr(dist), self._ptr(cnt), self.precision,
+                                  self.cand_cap)
+        out, a = [], 0
+        for p in ptrs:
+            out.append((idx[a:a + p[1]], dist[a:a + p[1]], cnt[a:a + p[1]]))
+            a += p[1]
+        return out
+
+    def match_batch(self, k, mode, pairs, dim, ratio_thr=M.MATCHING_RATIO_THRESHOLD, distance_thr=M.FLT_MAX, thr_src=None,
+                    thr_tgt=None):
+        """b200m_match_batch_device: -> one (records int32 [n, 4] CUDA view (CORR_DTYPE layout), average) per pair, equal
+        to Context.match_batch on the same data.  thr_src / thr_tgt: None or one 1-D float32 CUDA tensor per pair."""
+        ptrs, stride = self._set_pairs(pairs, dim)
+        ts, tt = self._thresholds(thr_src, thr_tgt, [(p[1], p[3]) for p in ptrs])
+        kk = k if mode == M.MODE_MUTUAL else 1
+        cap = max(sum(p[1] for p in ptrs) * kk, 1)
+        out = torch.empty((cap, 4), dtype=torch.int32, device=self.device)
+        self.use_torch_stream()
+        offsets, avg = self.ctx.match_batch_device(k, mode, ptrs, stride, dim, out.data_ptr(), cap, self._ptr(ts), self._ptr(tt),
+                                                   ratio_thr, distance_thr, self.precision, self.cand_cap)
+        return [(out[int(offsets[i]):int(offsets[i + 1])], float(avg[i])) for i in range(len(pairs))]
+
+    def match_wide_batch(self, k, mode, pairs, dim=None, cluster_k=M.MATCHING_CLUSTER_K, distance_thr=M.FLT_MAX, thr_src=None,
+                         thr_tgt=None):
+        """b200m_match_multiscale_batch_device: the dicts of Context.match_wide_batch (src_scales / tgt_scales = lists of
+        (features, index map or None), src_kps_xyz, tgt_kps_xyz, iss_radius_src, iss_radius_tgt) with CUDA tensors:
+        float32 features and coordinates [n, >= 3], int32 maps.  -> one (records view, average) per pair."""
+        return self._wide_batch(k, mode, pairs, None, dim, cluster_k, distance_thr, thr_src, thr_tgt)
+
+    def match_wide_local_batch(self, k, mode, pairs, match_search_radius, dim=None, cluster_k=M.MATCHING_CLUSTER_K,
+                               distance_thr=M.FLT_MAX, thr_src=None, thr_tgt=None):
+        """b200m_match_multiscale_local_batch_device: match_wide_batch's dicts plus src_kps_moved / tgt_kps_moved (the
+        latter may be None in ONE_SIDED mode), as Context.match_wide_local_batch takes them."""
+        return self._wide_batch(k, mode, pairs, float(match_search_radius), dim, cluster_k, distance_thr, thr_src, thr_tgt)
+
+    def _wide_batch(self, k, mode, pairs, radius, dim, cluster_k, distance_thr, thr_src, thr_tgt):
+        fs = [dict(pr) if isinstance(pr, dict) else dict(zip(M.Context._WIDE_FIELDS, pr)) for pr in pairs]
+        desc_strides, xyz_strides, width, out_pairs, counts = [], [], None, [], []
+        for i, f in enumerate(fs):
+            if len(f["src_scales"]) != len(f["tgt_scales"]):
+                raise M.B200MatchError("pair %d: need the same number of scales on both sides" % i)
+            scales = []
+            for s, ((sf, sm), (tf, tm)) in enumerate(zip(f["src_scales"], f["tgt_scales"])):
+                for side, t, m in (("src", sf, sm), ("tgt", tf, tm)):
+                    desc_strides.append(self._check_rows(t, "pair %d: scale %d: %s features" % (i, s, side)))
+                    if width is not None and t.shape[1] != width:
+                        raise M.B200MatchError("pair %d: scale %d: every descriptor row must have the same length" % (i, s))
+                    width = t.shape[1]
+                    if m is not None:
+                        self._check_vec(m, "pair %d: scale %d: %s map" % (i, s, side), t.shape[0], torch.int32)
+                scales.append((self._ptr(sf), sf.shape[0], self._ptr(sm), self._ptr(tf), tf.shape[0], self._ptr(tm)))
+            xs = {}
+            for key in ("src_kps_xyz", "tgt_kps_xyz") + (("src_kps_moved", "tgt_kps_moved") if radius is not None else ()):
+                x = f.get(key)
+                if x is not None:
+                    xyz_strides.append(self._check_rows(x, "pair %d: %s" % (i, key), min_cols=3))
+                xs[key] = x
+            if xs["tgt_kps_xyz"] is None:
+                raise M.B200MatchError("pair %d: tgt_kps_xyz is needed" % i)
+            ns = xs["src_kps_xyz"].shape[0] if xs["src_kps_xyz"] is not None else int(f.get("n_src_kps", 0))
+            nt = xs["tgt_kps_xyz"].shape[0]
+            if radius is not None:
+                for key, n in (("src_kps_moved", ns), ("tgt_kps_moved", nt)):
+                    if xs[key] is not None and xs[key].shape[0] != n:
+                        raise M.B200MatchError("pair %d: moved keypoints must have the rows of the unmoved ones" % i)
+            counts.append((ns, nt))
+            d = dict(scales=scales, n_src_kps=ns, n_tgt_kps=nt, iss_radius_src=float(f["iss_radius_src"]),
+                     iss_radius_tgt=float(f["iss_radius_tgt"]))
+            for key, x in xs.items():
+                d[key] = self._ptr(x)
+            out_pairs.append(d)
+        width = width or int(dim or 1)
+        dim = int(dim or width)
+        if dim > width:
+            raise M.B200MatchError("dim exceeds the row length")
+        stride = self._one_stride(desc_strides, "descriptor sets") or width
+        xyz_stride = self._one_stride(xyz_strides, "keypoint coordinates") or 4
+        ts, tt = self._thresholds(thr_src, thr_tgt, counts)
+        cap = max(sum(ns for ns, _ in counts), 1)
+        out = torch.empty((cap, 4), dtype=torch.int32, device=self.device)
+        self.use_torch_stream()
+        if radius is None:
+            offsets, avg = self.ctx.match_wide_batch_device(k, mode, out_pairs, stride * 4, dim, xyz_stride * 4, out.data_ptr(), cap,
+                                                            cluster_k, distance_thr, self._ptr(ts), self._ptr(tt), self.precision,
+                                                            self.cand_cap)
+        else:
+            offsets, avg = self.ctx.match_wide_local_batch_device(k, mode, out_pairs, radius, stride * 4, dim, xyz_stride * 4,
+                                                                  out.data_ptr(), cap, cluster_k, distance_thr, self._ptr(ts),
+                                                                  self._ptr(tt))
+        return [(out[int(offsets[i]):int(offsets[i + 1])], float(avg[i])) for i in range(len(pairs))]
 
 
 def records_to_numpy(records, n_out):

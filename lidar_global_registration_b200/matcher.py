@@ -90,7 +90,8 @@ EXPORTS = ["b200m_create", "b200m_destroy", "b200m_last_error", "b200m_set_strea
            "b200m_upload_replicated", "b200m_match_sharded", "b200m_match_sharded_device", "b200m_knn_target_sharded_device",
            "b200m_create_multi", "b200m_destroy_multi", "b200m_group_last_error", "b200m_group_size", "b200m_group_ctx",
            "b200m_group_upload", "b200m_group_upload_sharded", "b200m_group_match", "b200m_group_knn", "b200m_knn_batch",
-           "b200m_match_batch", "b200m_match_multiscale_batch", "b200m_match_multiscale_local_batch"]
+           "b200m_match_batch", "b200m_match_multiscale_batch", "b200m_match_multiscale_local_batch", "b200m_knn_batch_device",
+           "b200m_match_batch_device", "b200m_match_multiscale_batch_device", "b200m_match_multiscale_local_batch_device"]
 
 _lib = None
 
@@ -165,6 +166,10 @@ def load_library():
                                                fp, fp, vp, sz, C.POINTER(sz), vp]
     L.b200m_match_multiscale_local_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_WidePair), C.POINTER(_LocalPair), C.c_int, sz,
                                                      C.c_int, sz, C.c_int, C.c_float, fp, fp, vp, sz, C.POINTER(sz), vp]
+    L.b200m_knn_batch_device.argtypes = L.b200m_knn_batch.argtypes
+    L.b200m_match_batch_device.argtypes = L.b200m_match_batch.argtypes
+    L.b200m_match_multiscale_batch_device.argtypes = L.b200m_match_multiscale_batch.argtypes
+    L.b200m_match_multiscale_local_batch_device.argtypes = L.b200m_match_multiscale_local_batch.argtypes
     L.b200m_version.restype = C.c_int
     L.b200m_debug_operands.argtypes = [vp, C.c_int, C.c_int, vp, sz, vp, C.POINTER(C.c_float), C.POINTER(i32),
                                        C.POINTER(i64)]
@@ -406,7 +411,10 @@ class Context:
 
     def _batch_sides(self, pairs):
         # what the library's two sides hold after a batch call: every set padded to a multiple of 256 rows
-        self.n = [sum(-(-len(pr[s]) // 256) * 256 for pr in pairs) for s in (0, 1)]
+        self._batch_rows([(len(s), len(t)) for s, t in pairs])
+
+    def _batch_rows(self, counts):
+        self.n = [sum(-(-int(c[s]) // 256) * 256 for c in counts) for s in (0, 1)]
 
     def knn_batch(self, k, pairs, dim, precision=PREC_TC_F16, cand_cap=0):
         """b200m_knn_batch: `pairs` = [(source rows, target rows), ...] (float32 [n, stride_floats], one row length).
@@ -452,6 +460,87 @@ class Context:
                                            avg.ctypes.data))
         self._batch_sides(pairs)
         return [(out[int(offsets[i]):int(offsets[i + 1])], float(avg[i])) for i in range(len(pairs))]
+
+    # -- device-resident batches: every data pointer below is a device pointer on this context's device --------------
+    @staticmethod
+    def _device_pairs(pairs):
+        """[(src_ptr, n_src, tgt_ptr, n_tgt), ...] -> b200m_pair array."""
+        arr = (_Pair * max(len(pairs), 1))()
+        for i, (s, ns, t, nt) in enumerate(pairs):
+            arr[i] = _Pair(s or None, int(ns), t or None, int(nt))
+        return arr
+
+    def knn_batch_device(self, k, pairs, stride_bytes, dim, idx_ptr, dist_ptr, cnt_ptr, precision=PREC_TC_F16, cand_cap=0):
+        """b200m_knn_batch_device: `pairs` = [(src_ptr, n_src, tgt_ptr, n_tgt), ...]; the k-lists go to the device arrays
+        idx [sum n_src][k], dist, cnt.  Replaces the sets uploaded before."""
+        p = self._params(k, MODE_KNN_ONLY, precision=precision, cand_cap=cand_cap)
+        v = C.c_void_p
+        self._ck(self._L.b200m_knn_batch_device(self._h, C.byref(p), self._device_pairs(pairs), len(pairs), stride_bytes, dim,
+                                                v(idx_ptr), v(dist_ptr), v(cnt_ptr)))
+        self._batch_rows([(ns, nt) for _, ns, _, nt in pairs])
+
+    def match_batch_device(self, k, mode, pairs, stride_bytes, dim, out_ptr, cap, thr_src=0, thr_tgt=0,
+                           ratio_thr=MATCHING_RATIO_THRESHOLD, distance_thr=FLT_MAX, precision=PREC_TC_F16, cand_cap=0):
+        """b200m_match_batch_device: `pairs` as knn_batch_device's; records go to the device buffer out_ptr (`cap` records),
+        thr_src / thr_tgt are device pointers to the concatenated thresholds or 0.  -> (offsets uint64 [n_pairs + 1],
+        averages float32 [n_pairs]) on the host."""
+        offsets = np.zeros(len(pairs) + 1, np.uint64)
+        avg = np.empty(max(len(pairs), 1), np.float32)
+        p = self._params(k, mode, ratio_thr, distance_thr, precision, cand_cap)
+        v = C.c_void_p
+        self._ck(self._L.b200m_match_batch_device(self._h, C.byref(p), self._device_pairs(pairs), len(pairs), stride_bytes, dim,
+                                                  v(thr_src), v(thr_tgt), v(out_ptr), cap,
+                                                  offsets.ctypes.data_as(C.POINTER(C.c_size_t)), avg.ctypes.data))
+        self._batch_rows([(ns, nt) for _, ns, _, nt in pairs])
+        return offsets, avg[:len(pairs)]
+
+    def match_wide_batch_device(self, k, mode, pairs, stride_bytes, dim, xyz_stride_bytes, out_ptr, cap,
+                                cluster_k=MATCHING_CLUSTER_K, distance_thr=FLT_MAX, thr_src=0, thr_tgt=0, precision=PREC_TC_F16,
+                                cand_cap=0):
+        """b200m_match_multiscale_batch_device.  Each entry of `pairs` is a dict: scales = [(src_ptr, n_src, src_map_ptr,
+        tgt_ptr, n_tgt, tgt_map_ptr), ...] (map 0: identity), src_kps_xyz / tgt_kps_xyz (pointers), n_src_kps, n_tgt_kps,
+        iss_radius_src, iss_radius_tgt.  -> (offsets, averages) as match_batch_device's."""
+        return self._wide_batch_device(k, mode, pairs, None, stride_bytes, dim, xyz_stride_bytes, out_ptr, cap, cluster_k,
+                                       distance_thr, thr_src, thr_tgt, precision, cand_cap)
+
+    def match_wide_local_batch_device(self, k, mode, pairs, match_search_radius, stride_bytes, dim, xyz_stride_bytes, out_ptr,
+                                      cap, cluster_k=MATCHING_CLUSTER_K, distance_thr=FLT_MAX, thr_src=0, thr_tgt=0):
+        """b200m_match_multiscale_local_batch_device: match_wide_batch_device's dicts plus the pointers src_kps_moved and
+        tgt_kps_moved (0 allowed in ONE_SIDED mode)."""
+        return self._wide_batch_device(k, mode, pairs, float(match_search_radius), stride_bytes, dim, xyz_stride_bytes, out_ptr,
+                                       cap, cluster_k, distance_thr, thr_src, thr_tgt, PREC_TC_F16, 0)
+
+    def _wide_batch_device(self, k, mode, pairs, radius, stride_bytes, dim, xyz_stride_bytes, out_ptr, cap, cluster_k,
+                           distance_thr, thr_src, thr_tgt, precision, cand_cap):
+        keep, arr = [], (_WidePair * max(len(pairs), 1))()
+        locs = (_LocalPair * max(len(pairs), 1))()
+        for i, f in enumerate(pairs):
+            sc = (_Scale * max(len(f["scales"]), 1))()
+            for s, (a, na, ma, b, nb, mb) in enumerate(f["scales"]):
+                sc[s] = _Scale(a or None, int(na), ma or None, b or None, int(nb), mb or None)
+            keep.append(sc)
+            arr[i] = _WidePair(C.cast(sc, C.c_void_p), len(f["scales"]), f.get("src_kps_xyz") or None, int(f["n_src_kps"]),
+                               f.get("tgt_kps_xyz") or None, int(f["n_tgt_kps"]), float(f["iss_radius_src"]),
+                               float(f["iss_radius_tgt"]))
+            if radius is not None:
+                locs[i] = _LocalPair(f.get("src_kps_moved") or None, f.get("tgt_kps_moved") or None)
+        offsets = np.zeros(len(pairs) + 1, np.uint64)
+        avg = np.empty(max(len(pairs), 1), np.float32)
+        p = self._params(k, mode, distance_thr=distance_thr, precision=precision, cand_cap=cand_cap)
+        v = C.c_void_p
+        tail = (v(thr_src), v(thr_tgt), v(out_ptr), cap, offsets.ctypes.data_as(C.POINTER(C.c_size_t)), avg.ctypes.data)
+        if radius is None:
+            self._ck(self._L.b200m_match_multiscale_batch_device(self._h, C.byref(p), arr, len(pairs), stride_bytes, dim,
+                                                                 xyz_stride_bytes, int(cluster_k), *tail))
+        else:
+            self._ck(self._L.b200m_match_multiscale_local_batch_device(self._h, C.byref(p), arr, locs, len(pairs), stride_bytes, dim,
+                                                                       xyz_stride_bytes, int(cluster_k), radius, *tail))
+        # what the library's two sides hold afterwards: the last scale's sets of every pair, each padded to 256 rows
+        n_last = max((len(f["scales"]) for f in pairs if f["n_src_kps"]), default=0)
+        if n_last:
+            self._batch_rows([(f["scales"][n_last - 1][1], f["scales"][n_last - 1][4])
+                              if f["n_src_kps"] and len(f["scales"]) >= n_last else (0, 0) for f in pairs])
+        return offsets, avg[:len(pairs)]
 
     # -- whole matcher call ----------------------------------------------------
     def match(self, k, mode, ratio_thr=MATCHING_RATIO_THRESHOLD, distance_thr=FLT_MAX, thr_src=None, thr_tgt=None,
