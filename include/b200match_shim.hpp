@@ -19,7 +19,7 @@
 // them per scale and per direction does not pay for streams and device allocations again.
 //
 // With -DB200MATCH_WITH_PCL the feature types are PCL's (pcl::FPFHSignature33, pcl::SHOT352,
-// pcl::Histogram<135>) and clouds are pcl::PointCloud<FeatureT>::ConstPtr exactly as in the reference; without
+// pcl::Histogram<135>, pcl::UniqueShapeContext1960) and clouds are pcl::PointCloud<FeatureT>::ConstPtr exactly as in the reference; without
 // it (this repository's tests: PCL is not installed) layout-identical mirror structs are used and a "cloud"
 // is a std::vector<FeatureT>.  Errors surface as std::runtime_error -- the convention of the reference's
 // rassert (include/utils.h:9).  There is no CPU fallback anywhere below.
@@ -51,9 +51,11 @@ namespace b200match {
 struct FPFHSignature33 { float histogram[33]; static constexpr int descriptorSize() { return 33; } };
 struct SHOT352 { float descriptor[352]; float rf[9]; static constexpr int descriptorSize() { return 352; } };
 struct Histogram135 { float histogram[135]; static constexpr int descriptorSize() { return 135; } };
+struct UniqueShapeContext1960 { float descriptor[1960]; float rf[9]; static constexpr int descriptorSize() { return 1960; } };
 static_assert(sizeof(FPFHSignature33) == 132, "pcl::FPFHSignature33 is 132 bytes");
 static_assert(sizeof(SHOT352) == 1444, "pcl::SHOT352 is 1444 bytes");
 static_assert(sizeof(Histogram135) == 540, "pcl::Histogram<135> is 540 bytes");
+static_assert(sizeof(UniqueShapeContext1960) == 7876, "pcl::UniqueShapeContext1960 is 7876 bytes");
 template <typename FeatureT> using FeatureCloud = std::vector<FeatureT>;
 template <typename FeatureT> inline const FeatureT *cloud_data(const FeatureCloud<FeatureT> &c) { return c.data(); }
 template <typename FeatureT> inline size_t cloud_size(const FeatureCloud<FeatureT> &c) { return c.size(); }

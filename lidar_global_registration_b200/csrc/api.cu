@@ -316,7 +316,7 @@ int upload_common(b200m_ctx *ctx, int side, const float *device_aos, size_t n, s
 
 int check_upload_args(b200m_ctx *ctx, int side, const float *base, size_t n, size_t stride_bytes, int dim) {
     if (side != 0 && side != 1) return b200m_fail_msg(ctx, "b200m_upload: side must be 0 (source) or 1 (target)");
-    if (dim < 1 || dim > B200M_MAX_DIM) return b200m_fail_msg(ctx, "b200m_upload: dim out of range [1, 1024]");
+    if (dim < 1 || dim > B200M_MAX_DIM) return b200m_fail_msg(ctx, "b200m_upload: dim out of range [1, 2048]");
     if (stride_bytes % 4 != 0 || stride_bytes < (size_t) dim * 4)
         return b200m_fail_msg(ctx, "b200m_upload: stride_bytes must be a multiple of 4 and >= 4*dim");
     if (n > 0 && !base) return b200m_fail_msg(ctx, "b200m_upload: null descriptor pointer");

@@ -119,7 +119,7 @@ int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b20
     const std::string f(fn);
     if (n_pairs < 0) return b200m_fail_msg(ctx, f + ": n_pairs < 0");
     if (n_pairs > 0 && !pairs) return b200m_fail_msg(ctx, f + ": null pairs");
-    if (dim < 1 || dim > B200M_MAX_DIM) return b200m_fail_msg(ctx, f + ": dim out of range [1, 1024]");
+    if (dim < 1 || dim > B200M_MAX_DIM) return b200m_fail_msg(ctx, f + ": dim out of range [1, 2048]");
     if (stride_bytes % 4 != 0 || stride_bytes < (size_t) dim * 4)
         return b200m_fail_msg(ctx, f + ": stride_bytes must be a multiple of 4 and >= 4*dim");
     if (p->precision == B200M_PREC_TC_F16 && !ctx->tc_pair && ctx->tc_cluster == 4)

@@ -40,7 +40,8 @@ constexpr int kTmemCols = 512;
 constexpr int kTailBytes = 8576;         // barriers (<= 33 x 8 B) + TMEM slot + published thresholds (up to 4 x 128 x 4 B) + row
                                          // constants (2 KB) + the lists' published smallest values (4 KB)
 constexpr int kMaxStages = 12;
-constexpr int kMaxKAtoms = 10;
+constexpr int kMaxKAtoms = 10;           // A resident in shared memory (kp <= 640)
+constexpr int kMaxKAtomsStreamed = 32;   // K-streamed form: A and B through the ring (kp <= 2048)
 constexpr int kMaxLists = 16;
 // Cycle stamps (B200M_TC_DEBUG & 1024) exist only in a library built with -DB200M_TC_TRACE (B200M_TC_TRACE=1 in the
 // environment of build.py): their local arrays slow every debug instantiation down, also with the flag off.
@@ -628,10 +629,14 @@ __device__ __forceinline__ void chunk_hits(float m0, float m1, float m2, float m
 //       switch, not a runtime test of the pointer: either half of the lookup (the load, or the early exit) changes the register
 //       allocation of the whole kernel -- the chunk-entry epilogue then spills more and the C2 launch runs 3.25 -> 3.50 ms on
 //       one B200 (profiles/r03_ab_c2_seg_runtime.log).  SEG = false compiles to the single-pair kernel as it was.
-template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG, bool SEG>
+// KS:   (pair mode, EH = 1, kp > 640: 11..32 K atoms) K-streamed operands.  The query tile no longer stays resident: a ring
+//       stage holds this CTA's A atom (128 rows x 64 halves, 16 KB) followed by its half of the B atom (16 KB), and the
+//       producer loads ka stages per train tile.  The certificate's accumulation slop grows with the K steps (DESIGN.md §4).
+template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG, bool SEG, bool KS = false>
 __global__ void __launch_bounds__(EPI ? 640 : 64 + 128 * EH + (SPLITN ? 32 : 0), 1)
 tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_t,
                      const TcParams p) {
+    static_assert(!KS || (PAIR && EH == 1 && !SPLITN && EPI == 0), "the K-streamed form is a pair-mode, EH = 1 kernel");
     const int dflags = DBG ? p.debug_flags : 0;
     float *const dump = DBG ? p.dump : nullptr;
     constexpr bool ALT = EPI != 0;   // the sixteen-warp layouts (warp roles, register re-division, four lists per row)
@@ -657,7 +662,7 @@ tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     const uint32_t smem_u = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const uint32_t sA_u = smem_u;
-    const uint32_t sB_u = sA_u + (uint32_t) (p.ka * kATileBytes);
+    const uint32_t sB_u = KS ? sA_u : sA_u + (uint32_t) (p.ka * kATileBytes);   // KS: the ring starts the segment
     const uint32_t bars_u = sB_u + (uint32_t) (p.stages * p.stage_bytes);
     // barrier map: [0..S) full, [S..2S) empty, 2S a_full, then tmem_full[kAcc], tmem_empty[kAcc], the TMEM slot, thresholds
     const int stages = p.stages;
@@ -779,7 +784,7 @@ tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
             const uint32_t lead_a = map_to_cta(bar_a, 0);
             const uint32_t lead_full0 = map_to_cta(bar_full0, 0);
             const int row_off = (int) crank * (B200M_TILE_N / 2);
-            if (elect_one()) {
+            if (!KS && elect_one()) {
                 if (crank == 0) mbar_arrive_expect_tx(bar_a, (uint32_t) (2 * ka * kATileBytes));
                 for (int a = 0; a < ka; ++a) tma_load_2d_2sm(sA_u + (uint32_t) (a * kATileBytes), &tmap_q, lead_a, a * 64, q_row);
             }
@@ -788,7 +793,9 @@ tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
             // opaque register copies of the ring's addresses (see the epilogue: keeps ptxas from re-deriving them per tile)
             uint32_t r_empty = bar_empty0, r_full = bar_full0, r_lead_full = lead_full0, r_sb = sB_u;
             asm volatile("" : "+r"(r_empty), "+r"(r_full), "+r"(r_lead_full), "+r"(r_sb));
-            const uint32_t stage_bytes = (uint32_t) (kStageBytes / 2);   // pair mode: half a train tile per CTA
+            // pair mode: half a train tile per CTA (KS: behind this CTA's query atom)
+            const uint32_t stage_bytes = (uint32_t) (KS ? kATileBytes + kStageBytes / 2 : kStageBytes / 2);
+            const uint32_t b_off = KS ? (uint32_t) kATileBytes : 0u;
             int t = t0 + sweep_start;   // rotated sweep (chunk-entry kernels; 0 otherwise): t0 + start, ..., t1 - 1, t0, ...
             for (int lt = (dflags & 65536) ? t1 - t0 : 0; lt < t1 - t0; ++lt) {
                 for (int a = 0; a < ka; ++a) {
@@ -798,7 +805,8 @@ tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
                             if (crank == 0) mbar_arrive(r_full + 8u * s);
                         } else {
                             if (crank == 0) mbar_arrive_expect_tx(r_full + 8u * s, 2u * stage_bytes);
-                            tma_load_2d_2sm(r_sb + s * stage_bytes, &tmap_t, r_lead_full + 8u * s, a * 64,
+                            if (KS) tma_load_2d_2sm(r_sb + s * stage_bytes, &tmap_q, r_lead_full + 8u * s, a * 64, q_row);
+                            tma_load_2d_2sm(r_sb + s * stage_bytes + b_off, &tmap_t, r_lead_full + 8u * s, a * 64,
                                             t * B200M_TILE_N + row_off);
                         }
                         // every 32 tiles the leader says where it is: pairs that start from now on start there
@@ -841,7 +849,7 @@ tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
         // per instruction: warp-uniform control flow, ring position kept as counters (no divisions), descriptors
         // advanced by adding to their low word, the four K steps of an atom unrolled. =====
         if (!PAIR || crank == 0) {   // pair mode: the leader CTA issues for both SMs
-            mbar_wait(bar_a, 0);
+            if (!KS) mbar_wait(bar_a, 0);
             tc_fence_after();
             const uint64_t desc_a0 = make_kmajor_sw128_desc(sA_u);
             const uint64_t desc_b0 = make_kmajor_sw128_desc(sB_u);
@@ -955,8 +963,9 @@ tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
                 const bool tr_on = trace && ti >= 0 && ti < kTraceTiles;
                 for (int a = 0; a < ka; ++a) {
                     if (!no_ring) mbar_wait(bar_full0 + 8u * s, ph);
-                    const uint64_t da = desc_a0 + (uint64_t) ((uint32_t) a * a_step);
-                    const uint64_t db = desc_b0 + (uint64_t) (s * b_step);
+                    // KS: A atom at the start of the stage, the B half behind it
+                    const uint64_t da = KS ? desc_b0 + (uint64_t) (s * b_step) : desc_a0 + (uint64_t) ((uint32_t) a * a_step);
+                    const uint64_t db = KS ? da + (uint64_t) (kATileBytes >> 4) : desc_b0 + (uint64_t) (s * b_step);
                     // K steps of this atom: 4, or what is left of the row in the last one; +32 B (2 descriptor
                     // units) per K = 16 step inside the 128 B swizzle atom
                     uint32_t nk = a + 1 < ka ? nk_full : nk_last;
@@ -1038,7 +1047,9 @@ tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
             // every thread of the row writes the same four values
             sts_f32(st.s_const, na);
             sts_f32(st.s_const + 4u, ab * 4.8828125e-4f * 1.001953125f + 2.384185791015625e-7f * sqrtf((float) p.dim));
-            sts_f32(st.s_const + 8u, ab * ab * 1.52587890625e-5f + 1e-6f);
+            // accumulation slop: measured bound 2^-16 ab^2 up to 40 K steps; KS: 2^-21 ab^2 per K step (DESIGN.md §4)
+            sts_f32(st.s_const + 8u, KS ? ab * ab * ((float) p.ksteps * 4.76837158203125e-7f) + 1e-6f
+                                        : ab * ab * 1.52587890625e-5f + 1e-6f);
             sts_f32(st.s_const + 12u, 1.f + 2.2f * (float) (p.dim + 4) * 5.9604644775390625e-8f);
         }
         asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");   // shared row state initialised
@@ -1421,9 +1432,9 @@ int get_tmap(b200m_ctx *ctx, int side, bool as_query, int cluster, const CUtenso
     return 0;
 }
 
-template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG, bool SEG>
+template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG, bool SEG, bool KS = false>
 int launch_tc(b200m_ctx *ctx, const CUtensorMap *mq, const CUtensorMap *mt, const TcParams &p, dim3 grid, size_t smem) {
-    CK(cudaFuncSetAttribute(tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG, SEG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+    CK(cudaFuncSetAttribute(tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG, SEG, KS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = grid;
     cfg.blockDim = dim3(EPI ? 640 : 64 + 128 * EH + (SPLITN ? 32 : 0), 1, 1);
@@ -1436,7 +1447,7 @@ int launch_tc(b200m_ctx *ctx, const CUtensorMap *mq, const CUtensorMap *mt, cons
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG, SEG>, *mq, *mt, p);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG, SEG, KS>, *mq, *mt, p);
     if (e != cudaSuccess) {
         cudaGetLastError();   // do not leave the launch error behind for the next call
         return b200m_fail_msg(ctx, std::string("tc_candidates launch failed: ") + cudaGetErrorString(e) + " (grid " +
@@ -1449,10 +1460,12 @@ int launch_tc(b200m_ctx *ctx, const CUtensorMap *mq, const CUtensorMap *mt, cons
 
 }  // namespace
 
+// kp <= 640: the A-resident kernels (any mode); 640 < kp <= 2048 (dim <= 2045): the K-streamed kernel, which exists in
+// pair mode only.  Everything else is answered on the exact path.
 bool tc_supported(const b200m_ctx *ctx, int dim, int k) {
-    (void) ctx;
     int kp = (dim + B200M_AUG_COLS + 63) / 64 * 64;
-    return kp / 64 <= kMaxKAtoms && k <= 16;
+    if (k > 16) return false;
+    return kp / 64 <= kMaxKAtoms || (ctx->tc_pair && kp / 64 <= kMaxKAtomsStreamed);
 }
 
 void tc_release(b200m_ctx *ctx) {
@@ -1478,11 +1491,15 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
     TcParams p{};
     p.cluster = cluster;
     p.pair = pair;
-    p.stage_bytes = pair ? kStageBytes / 2 : kStageBytes;
     p.ka = q.kp / 64;
+    // long descriptors (kp > 640): the query tile does not fit next to a useful ring, both operands are streamed
+    const bool ks = p.ka > kMaxKAtoms;
+    if (ks && (!pair || p.ka > kMaxKAtomsStreamed)) return b200m_fail_msg(ctx, "tc_candidates: descriptor too long for this mode");
+    p.stage_bytes = ks ? kATileBytes + kStageBytes / 2 : pair ? kStageBytes / 2 : kStageBytes;
     p.ksteps = (q.dim + B200M_AUG_COLS + 15) / 16;
     const size_t smem_limit = 227 * 1024;
-    const size_t fixed = (size_t) p.ka * kATileBytes + 1024 /*alignment*/ + kTailBytes /*barriers + per-row shared state*/;
+    const size_t a_bytes = ks ? 0 : (size_t) p.ka * kATileBytes;   // the resident query tile
+    const size_t fixed = a_bytes + 1024 /*alignment*/ + kTailBytes /*barriers + per-row shared state*/;
     int stages = (int) ((smem_limit - fixed) / p.stage_bytes);
     if (stages > kMaxStages) stages = kMaxStages;
     if ((ctx->tc_debug & 8) && stages > 4) stages = 4;     // timing experiment: shallow ring
@@ -1498,7 +1515,7 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
     // also records the accumulator values so that the re-rank can prune by the row's final threshold.
     int eh = p.ka <= 2 ? 2 : 1;
     if (ctx->tc_debug & 64) eh = 1;
-    if (ctx->tc_debug & 128) eh = 2;
+    if ((ctx->tc_debug & 128) && !ks) eh = 2;
     // One-atom descriptors (FPFH) in pair mode with the full 12-stage ring: fully unrolled issue loop (B200M_TC_LEAN=0
     // falls back to the general loop).
     p.lean = (pair && p.ka == 1 && stages == kMaxStages && ctx->tc_lean != 0) ? 1 : 0;
@@ -1583,7 +1600,7 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
     p.sweep_hint = ctx->ws_sweep_hint.as<int>();
     p.debug_flags = ctx->tc_debug;
     if (dump) p.tiles_per_split = (int) dump_t_tile;
-    const size_t smem = (size_t) p.ka * kATileBytes + (size_t) stages * p.stage_bytes + 1024 + kTailBytes;
+    const size_t smem = a_bytes + (size_t) stages * p.stage_bytes + 1024 + kTailBytes;
     dim3 grid((unsigned) (dump ? cluster : (n_qtiles + cluster - 1) / cluster * cluster), (unsigned) n_splits, 1);
     int kt = k <= 1 ? 1 : k <= 2 ? 2 : k <= 4 ? 4 : k <= 8 ? 8 : 16;
     int rc;
@@ -1600,8 +1617,13 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
                          : launch_tc<KT_, true, 1, false, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem))                  \
               : (eh == 2 ? launch_tc<KT_, false, 2, false, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)                  \
                          : launch_tc<KT_, false, 1, false, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem))
+#define B200M_TC_CASE_KS(KT_)                                                                                  \
+    if (p.seg_range) rc = launch_tc<KT_, true, 1, false, 0, false, true, true>(ctx, mq, mt, p, grid, smem);        \
+    else if (dbg) rc = launch_tc<KT_, true, 1, false, 0, true, false, true>(ctx, mq, mt, p, grid, smem);           \
+    else rc = launch_tc<KT_, true, 1, false, 0, false, false, true>(ctx, mq, mt, p, grid, smem);
 #define B200M_TC_CASE(KT_)                              \
-    if (p.seg_range) { B200M_TC_CASE2(KT_, false, true); } \
+    if (ks) { B200M_TC_CASE_KS(KT_) }                      \
+    else if (p.seg_range) { B200M_TC_CASE2(KT_, false, true); } \
     else if (dbg) { B200M_TC_CASE2(KT_, true, false); }    \
     else { B200M_TC_CASE2(KT_, false, false); }
     switch (kt) {
@@ -1612,6 +1634,7 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
         default: B200M_TC_CASE(16); break;
     }
 #undef B200M_TC_CASE
+#undef B200M_TC_CASE_KS
 #undef B200M_TC_CASE2
     if (rc) return rc;
     ctx->stats.launches += 1;

@@ -424,7 +424,9 @@ __device__ __forceinline__ void bar_wait_parity(uint32_t bar, uint32_t parity) {
 __host__ __device__ inline int rerank_pitch_bytes(int dp) { return (dp / 4) % 2 ? dp * 4 : dp * 4 + 16; }
 // Slab rows per warp.  Short rows: one per lane.  Long rows (RoPS, SHOT): 8 -- the live candidates of a row (after
 // pruning, typically k plus a few) are compacted into the slab, a full slab of 32 x 1.4 KB would leave room for only four
-// warps per SM, and this kernel lives on the number of gathers in flight, not on lanes.
+// warps per SM, and this kernel lives on the number of gathers in flight, not on lanes.  Rows over 4 KB (USC-1960: a
+// 7856-byte pitch) keep 8 too: 3 warps x 8 slots hold 24 of the 27 rows that fit in 220 KB with one query row per warp,
+// and no other slot count holds more (4: 5 x 4 = 20, 6: 4 x 6 = 24, 12: 2 x 12 = 24).
 __host__ __device__ inline int rerank_slots(int dp) { return rerank_pitch_bytes(dp) <= 256 ? 32 : 8; }
 __host__ __device__ inline size_t rerank_warp_bytes(int dp) { return (size_t) (rerank_slots(dp) + 1) * rerank_pitch_bytes(dp); }   // + the query
 
@@ -1024,7 +1026,7 @@ cudaError_t launch_rerank(const float *q_f32, const uint8_t *q_valid, int dp, in
     const size_t per_warp = rerank_warp_bytes(dp) + 8;
     int warps = (int) ((220 * 1024) / per_warp);
     if (warps > 16) warps = 16;
-    if (warps < 1) return cudaErrorInvalidValue;   // dp <= 1024 needs at most 136 KB per warp
+    if (warps < 1) return cudaErrorInvalidValue;   // dp <= 2048 needs at most 74 KB per warp
     const size_t smem = (size_t) warps * per_warp;
     size_t want = (n_rows + warps - 1) / warps;
     // small descriptors leave room for two CTAs per SM

@@ -9,7 +9,7 @@
 #include "../../include/b200match.h"
 
 #define B200M_MAX_K 32
-#define B200M_MAX_DIM 1024
+#define B200M_MAX_DIM 2048
 #define B200M_TILE_N 256     // train rows per candidate-kernel tile; operand row counts are padded to this
 #define B200M_TILE_M 128     // query rows per CTA
 #define B200M_AUG_COLS 3     // extra K columns carrying |b|^2 as an FP16 triple

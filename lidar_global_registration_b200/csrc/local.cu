@@ -444,6 +444,8 @@ int launch_local_cells(b200m_ctx *ctx, int direction, const float *d_query_xyz, 
     const float r2 = radius * radius;   // radiusSearch is handed radius * radius (FP32 product)
 #define B200M_LOCALC_CASE(K)                                                                                                   \
     do {                                                                                                                       \
+        if (smem > 48 * 1024) /* rows over 1536 floats */                                                                    \
+            CK(cudaFuncSetAttribute(local_cells_kernel<K, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));   \
         local_cells_kernel<K, false><<<blocks, kLocalWarps * 32, smem, st>>>(                                                  \
             g, q.f32.as<float>(), q.valid.as<uint8_t>(), q.dp, t.f32.as<float>(), (long long) t.index_offset, q.n, d_query_xyz, \
             d_train_xyz, stride, r2, k, ls->starts.as<int>(), ls->rows.as<int32_t>(), d_idx, d_dist, d_count);                 \
@@ -515,6 +517,8 @@ int launch_local_cells_batch(b200m_ctx *ctx, const LocalBatch &a, int32_t *d_idx
     ctx->stats.launches += launches + 1;
 #define B200M_LOCALB_CASE(K)                                                                                                    \
     do {                                                                                                                        \
+        if (smem > 48 * 1024) /* rows over 1536 floats */                                                                     \
+            CK(cudaFuncSetAttribute(local_cells_kernel<K, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));     \
         local_cells_kernel<K, true><<<blocks, kLocalWarps * 32, smem, st>>>(                                                    \
             none, q.f32.as<float>(), q.valid.as<uint8_t>(), q.dp, t.f32.as<float>(), 0, nq, &xq->x, &xt->x, 4, r2, a.k,         \
             nullptr, ls->rows.as<int32_t>(), d_idx, d_dist, d_count, grids, a.blk[qs], ls->starts.as<int>());                  \

@@ -112,6 +112,64 @@ pack_f32_kernel(const float *__restrict__ aos, size_t n, size_t stride_floats, i
     if (threadIdx.x == 0) out[3 * dp] = sh_cnt;
 }
 
+// Long rows (dp > 1024: NI = 64 would not fit the register file, NI = 32 already spills) in two passes.  First the copy and
+// the validity, one warp per row walking the row in 32-column slices, with the same SEG handling as pack_f32_kernel.
+template <bool SEG>
+__global__ void __launch_bounds__(kPackWarps * 32)
+pack_f32_long_kernel(const float *__restrict__ aos, size_t n, size_t stride_floats, int dim, int dp,
+                     float *__restrict__ f32, uint8_t *__restrict__ valid,
+                     const int32_t *__restrict__ seg_blk, const SetRef *__restrict__ sets) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (size_t row = (size_t) blockIdx.x * kPackWarps + warp; row < n; row += (size_t) gridDim.x * kPackWarps) {
+        float *dst = f32 + row * (size_t) dp;
+        const float *src = aos + row * stride_floats;
+        bool gap = false;
+        if constexpr (SEG) {
+            const SetRef set = sets[seg_blk[row / B200M_TILE_N]];
+            const size_t local = row - (size_t) set.first;
+            gap = local >= (size_t) set.rows;
+            src = set.base + (gap ? 0 : local) * stride_floats;
+        }
+        bool ok = true;
+        for (int d = lane; d < dp; d += 32) {
+            const float v = d < dim ? (gap ? __int_as_float(-1) : __ldg(src + d)) : 0.f;
+            ok = ok && isfinite(v);
+            dst[d] = v;
+        }
+        ok = __all_sync(0xffffffffu, ok);
+        if (lane == 0) valid[row] = ok ? 1 : 0;
+    }
+}
+
+// ... then the column statistics of the rows just written, in the layout pack_f32_kernel leaves: CTA b of the grid folds
+// the valid rows of its contiguous share of the rows, a thread per column (coalesced across the threads of a row).  The
+// summation order differs from the short form; the centre only has to be some centre (DESIGN.md §4).
+__global__ void __launch_bounds__(kPackWarps * 32)
+pack_stats_long_kernel(const float *__restrict__ f32, const uint8_t *__restrict__ valid, size_t n, int dp,
+                       float *__restrict__ stats) {
+    const size_t per = (n + gridDim.x - 1) / gridDim.x;
+    const size_t r0 = min(n, (size_t) blockIdx.x * per), r1 = min(n, r0 + per);
+    float *out = stats + (size_t) blockIdx.x * stats_floats(dp);
+    for (int d = threadIdx.x; d < dp; d += blockDim.x) {
+        float s = 0.f, mn = INFINITY, mx = -INFINITY;
+        for (size_t r = r0; r < r1; ++r) {
+            if (!valid[r]) continue;
+            const float v = __ldg(f32 + r * (size_t) dp + d);
+            s += v;
+            mn = fminf(mn, v);
+            mx = fmaxf(mx, v);
+        }
+        out[d] = s;
+        out[dp + d] = mn;
+        out[2 * dp + d] = mx;
+    }
+    if (threadIdx.x == 0) {
+        float cnt = 0.f;
+        for (size_t r = r0; r < r1; ++r) cnt += valid[r] ? 1.f : 0.f;
+        out[3 * dp] = cnt;
+    }
+}
+
 // device-resident results of the statistics pass (read by the operand pack; copied to the host once, afterwards)
 struct PrepDev {
     int maxabs_bits;        // max |x - mean| over the valid rows of both sides, as the bits of a non-negative float
@@ -182,15 +240,17 @@ prep_finalize_kernel(const float *__restrict__ sa, int ga, const float *__restri
 // values at a time (128-bit loads, 64-bit stores); the scale word is read once per warp and the side's largest norm
 // leaves through ONE atomic per warp (a per-row atomic on the line that also holds the scale serialises the kernel
 // in a single L2 slice: 0.9 ms instead of 0.25 ms for 500k SHOT rows).
+// NS: 128-column sweeps of the row held in registers (5: kp <= 640; 16: the long form, kp <= 2048).
+template <int NS>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32)
 pack_operands_kernel(const float *__restrict__ f32, const uint8_t *__restrict__ valid, size_t n, size_t n_pad,
                      int dim, int dp, int kp, const float *__restrict__ mean, PrepDev *__restrict__ prep, int side,
                      __half *__restrict__ op_query, __half *__restrict__ op_train, float *__restrict__ norm16) {
     const int lane = threadIdx.x & 31;
     const float scale = scale_for(__int_as_float(prep->maxabs_bits));
-    float4 mu[5];
+    float4 mu[NS];
 #pragma unroll
-    for (int i = 0; i < 5; ++i) {
+    for (int i = 0; i < NS; ++i) {
         const int d0 = 4 * lane + 128 * i;
         mu[i] = d0 < dp ? __ldg(reinterpret_cast<const float4 *>(mean + d0)) : make_float4(0.f, 0.f, 0.f, 0.f);
     }
@@ -203,15 +263,15 @@ pack_operands_kernel(const float *__restrict__ f32, const uint8_t *__restrict__ 
         const float *src = f32 + row * (size_t) dp;
         double nrm = 0.0;
         // the descriptor columns (dp is a multiple of 4, kp of 64; columns dim..dp-1 of f32 are zero): every load of
-        // the row is issued before the first conversion (kp <= 640: at most five 128-column sweeps)
-        float4 v[5];
+        // the row is issued before the first conversion (at most NS 128-column sweeps)
+        float4 v[NS];
 #pragma unroll
-        for (int i = 0; i < 5; ++i) {
+        for (int i = 0; i < NS; ++i) {
             const int d0 = 4 * lane + 128 * i;
             v[i] = (row < n && d0 < dp) ? __ldg(reinterpret_cast<const float4 *>(src + d0)) : mu[i];   // x - mu = 0 beyond the row
         }
 #pragma unroll
-        for (int i = 0; i < 5; ++i) {
+        for (int i = 0; i < NS; ++i) {
             const int d0 = 4 * lane + 128 * i;
             if (d0 >= kp) break;
             const float x[4] = {(v[i].x - mu[i].x) * scale, (v[i].y - mu[i].y) * scale, (v[i].z - mu[i].z) * scale,
@@ -265,6 +325,15 @@ cudaError_t launch_pack_f32(const float *aos, size_t n, size_t stride_bytes, int
     const unsigned blocks = (unsigned) pack_stats_blocks(sm_count);
     const size_t smem = sizeof(float) * 3 * (size_t) dp;
     const int ni = (dp + 31) / 32;
+    if (ni > 32) {   // long rows: copy + validity, then the column statistics over what was written
+        if (sets)
+            pack_f32_long_kernel<true><<<blocks, kPackWarps * 32, 0, st>>>(aos, n, stride_bytes / 4, dim, dp, f32, valid, seg_blk, sets);
+        else
+            pack_f32_long_kernel<false><<<blocks, kPackWarps * 32, 0, st>>>(aos, n, stride_bytes / 4, dim, dp, f32, valid, nullptr,
+                                                                            nullptr);
+        pack_stats_long_kernel<<<blocks, kPackWarps * 32, 0, st>>>(f32, valid, n, dp, stats);
+        return cudaGetLastError();
+    }
 #define B200M_PACK_CASE(NI)                                                                                          \
     do {                                                                                                             \
         if (sets)                                                                                                    \
@@ -306,9 +375,14 @@ cudaError_t launch_tc_prepare(b200m_ctx *ctx) {
         if ((e = sd.norm16.reserve(sizeof(float) * sd.n_pad)) != cudaSuccess) return e;
         size_t want = (sd.n_pad + kWarpsPerBlock - 1) / kWarpsPerBlock, cap_blocks = (size_t) ctx->sm_count * 8;
         unsigned blocks = (unsigned) (want < cap_blocks ? want : cap_blocks);
-        pack_operands_kernel<<<blocks, kWarpsPerBlock * 32, 0, st>>>(
-            sd.f32.as<float>(), sd.valid.as<uint8_t>(), sd.n, sd.n_pad, dim, dp, sd.kp, pr.mean.as<float>(), dev, s,
-            sd.op_query.as<__half>(), sd.op_train.as<__half>(), sd.norm16.as<float>());
+        if (sd.kp <= 640)
+            pack_operands_kernel<5><<<blocks, kWarpsPerBlock * 32, 0, st>>>(
+                sd.f32.as<float>(), sd.valid.as<uint8_t>(), sd.n, sd.n_pad, dim, dp, sd.kp, pr.mean.as<float>(), dev, s,
+                sd.op_query.as<__half>(), sd.op_train.as<__half>(), sd.norm16.as<float>());
+        else
+            pack_operands_kernel<16><<<blocks, kWarpsPerBlock * 32, 0, st>>>(
+                sd.f32.as<float>(), sd.valid.as<uint8_t>(), sd.n, sd.n_pad, dim, dp, sd.kp, pr.mean.as<float>(), dev, s,
+                sd.op_query.as<__half>(), sd.op_train.as<__half>(), sd.norm16.as<float>());
         ctx->stats.launches += 1;
     }
     if ((e = cudaGetLastError()) != cudaSuccess) return e;

@@ -9,8 +9,9 @@ include/b200match.h).  Names and argument meaning follow the reference:
     AlignmentParameters (hot-path subset)         <- include/common.h:135-163
 
 Descriptors are float32 arrays [n, stride_floats] whose leading `dim` columns are the
-descriptor -- the AoS layout PCL hands to the reference (`&cloud.points[0]`, `sizeof(FeatureT)`).
-There is no CPU path here: without the CUDA library and a B200 every call raises.
+descriptor -- the AoS layout PCL hands to the reference (`&cloud.points[0]`, `sizeof(FeatureT)`):
+FPFH-33 (33 floats), RoPS-135 (135), SHOT-352 (361: descriptor + rf[9]), USC-1960 (1969: descriptor + rf[9]); any
+dim up to 2048.  There is no CPU path here: without the CUDA library and a B200 every call raises.
 """
 import ctypes as C
 import dataclasses

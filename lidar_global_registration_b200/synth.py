@@ -5,8 +5,10 @@ Layouts mirror PCL's point structs as the reference hands them to the matcher
     FPFH  = pcl::FPFHSignature33  : float histogram[33]                -> 132 B / row
     RoPS  = pcl::Histogram<135>   : float histogram[135]               -> 540 B / row
     SHOT  = pcl::SHOT352          : float descriptor[352]; float rf[9] -> 1444 B / row
+    USC   = pcl::UniqueShapeContext1960 : float descriptor[1960]; float rf[9] -> 7876 B / row
 The generators return the AoS buffer (float32 [n, stride/4]); the descriptor is
-columns [0, dim).
+columns [0, dim).  The value statistics are stand-ins of the descriptors' shape (sign, sparsity,
+normalisation), not measured from PCL's estimators.
 """
 import numpy as np
 
@@ -17,6 +19,7 @@ DESCRIPTORS = {
     "fpfh": (33, 33),
     "rops": (135, 135),
     "shot": (352, 361),
+    "usc": (1960, 1969),
 }
 
 
@@ -63,7 +66,20 @@ def _rops_like(rng, n, dim=135):
     return (protos[which] + 0.3 * rng.standard_normal((n, dim)).astype(np.float32)).astype(np.float32)
 
 
-_GEN = {"fpfh": _fpfh_like, "shot": _shot_like, "rops": _rops_like}
+def _usc_like(rng, n, dim=1960):
+    """Shape-context-like histogram: non-negative, ~85 % zeros, bin weights growing along
+    the row (outer shells hold more points); rows cluster around n/64 prototypes."""
+    n_proto = max(n // 64, 4)
+    shell = np.linspace(0.5, 2.0, dim).astype(np.float32)
+    protos = rng.gamma(0.5, 1.0, size=(n_proto, dim)).astype(np.float32) * shell
+    protos *= (rng.random((n_proto, dim)) < 0.15)
+    which = rng.integers(0, n_proto, size=n)
+    rows = protos[which] * (1.0 + 0.25 * rng.standard_normal((n, dim)).astype(np.float32))
+    extra = rng.gamma(0.5, 1.0, size=(n, dim)).astype(np.float32) * (rng.random((n, dim)) < 0.01)
+    return (np.abs(rows) + 0.5 * extra).astype(np.float32)
+
+
+_GEN = {"fpfh": _fpfh_like, "shot": _shot_like, "rops": _rops_like, "usc": _usc_like}
 
 
 def to_aos(rows, stride_floats, rng=None):
@@ -92,7 +108,7 @@ def make_pair(descriptor, n_src, n_tgt, seed=SEED, nan_frac=0.001, distractor_fr
     pick = rng_t.integers(0, n_src, size=n_cpy) if n_cpy > n_src else rng_t.permutation(n_src)[:n_cpy]
     scale = float(np.sqrt((src.astype(np.float64) ** 2).sum(1).mean() / dim))
     tgt_c = src[pick] + (noise * scale) * rng_t.standard_normal((n_cpy, dim)).astype(np.float32)
-    if descriptor in ("fpfh", "shot"):
+    if descriptor in ("fpfh", "shot", "usc"):
         tgt_c = np.abs(tgt_c)
     tgt = np.concatenate([tgt_c, gen(rng_t, n_dis, dim)], axis=0) if n_dis else tgt_c
     tgt = tgt[rng_t.permutation(n_tgt)].astype(np.float32)
@@ -137,6 +153,13 @@ def make_pair_torch(descriptor, n_src, n_tgt, device, seed=SEED, nan_frac=0.001,
             extra = gamma_like((n, dim), 2.5) * (torch.rand((n, dim), generator=g, device=device) < 0.02)
             rows = rows + 0.25 * extra
             return rows / rows.norm(dim=1, keepdim=True).clamp_min(1e-12)
+        if descriptor == "usc":
+            shell = torch.linspace(0.5, 2.0, dim, device=device)
+            protos = gamma_like((n_proto, dim), 2.5) * shell
+            protos = protos * (torch.rand((n_proto, dim), generator=g, device=device) < 0.15)
+            rows = protos[which] * (1.0 + 0.25 * torch.randn((n, dim), generator=g, device=device))
+            extra = gamma_like((n, dim), 2.5) * (torch.rand((n, dim), generator=g, device=device) < 0.01)
+            return rows.abs_() + 0.5 * extra
         protos = torch.randn((n_proto, dim), generator=g, device=device)
         return protos[which] + 0.3 * torch.randn((n, dim), generator=g, device=device)
 
@@ -149,7 +172,7 @@ def make_pair_torch(descriptor, n_src, n_tgt, device, seed=SEED, nan_frac=0.001,
         pick = torch.randperm(n_src, generator=g, device=device)[:n_cpy]
     scale = float(src.pow(2).sum(1).mean().div(dim).sqrt())
     tgt = src[pick] + (noise * scale) * torch.randn((n_cpy, dim), generator=g, device=device)
-    if descriptor in ("fpfh", "shot"):
+    if descriptor in ("fpfh", "shot", "usc"):
         tgt = tgt.abs_()
     if n_dis:
         tgt = torch.cat([tgt, gen(n_dis)], dim=0)
