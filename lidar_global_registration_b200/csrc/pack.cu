@@ -14,6 +14,7 @@
 //
 // All HBM-bound: algorithmic bytes per row = stride_in + 4*dp + 1 (pack_f32) and
 // 4*dp + 2*2*kp + 4 (operand pack) -- see DESIGN.md.
+#include <float.h>
 #include <math.h>
 #include <string.h>
 
@@ -394,9 +395,13 @@ cudaError_t launch_tc_prepare(b200m_ctx *ctx) {
     memcpy(&maxabs, &h.maxabs_bits, 4);
     const float scale = scale_for(maxabs);
     pr.scale = scale;
-    // data whose spread cannot be brought into FP16 range (non-finite after centring, or a spread so small/large that
-    // the power-of-two scale leaves float range) stays on the exact path
-    pr.usable = isfinite(maxabs) && isfinite(scale) && scale > 0.f && maxabs < 1e30f && (maxabs == 0.f || maxabs > 1e-30f);
+    // The certificate's window (DESIGN.md §4); data outside it stays on the exact path.  Upper edge: the reference's
+    // FP32 sum of D squared differences, each at most (2 maxabs)^2, stays finite.  Lower edge: the subnormal rounding
+    // of those terms (at most 2^-150 each, D 2^-150 s^2 in scaled units) stays under 2^-25, inside the 1e-6 that slop
+    // carries on top of the accumulator bound.
+    const double m = maxabs, s = scale, gam = (dim + 4) * 0x1p-24;
+    pr.usable = isfinite(maxabs) && isfinite(scale) && scale > 0.f &&
+                (maxabs == 0.f || (dim * 4.0 * m * m * (1.0 + gam) < (double) FLT_MAX && dim * s * s <= 0x1p125));
     memcpy(&pr.max_norm[0], &h.max_norm_bits[0], 4);
     memcpy(&pr.max_norm[1], &h.max_norm_bits[1], 4);
     pr.ver[0] = a.version;
