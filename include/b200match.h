@@ -432,6 +432,33 @@ B200M_API int b200m_match_multiscale_local_batch_device(b200m_ctx *ctx, const b2
                                                         const float *d_thr_tgt, b200m_corr *d_out, size_t cap,
                                                         size_t *offsets, float *avg);
 
+/* ---- batch plans: device batch calls bound once, enqueued without the host --------------------------------------------
+ * A plan binds b200m_knn_batch_device's / b200m_match_batch_device's arguments: *p, the pairs (their device pointers and
+ * sizes), the stride, dim, the threshold and output pointers.  Creation does every check of the device form (same error
+ * texts, in ctx's last error), builds and uploads the batch tables, allocates every workspace in a context of the plan's
+ * own (on ctx's device, with the same environment settings; later calls on ctx cannot move the plan's memory) and runs the
+ * batch once on ctx's stream, synchronised (the outputs are written), so that every kernel module is loaded.
+ * b200m_plan_run then only enqueues kernels and memsets on `cuda_stream` (NULL: the legacy default stream): no host round
+ * trip, allocation, host <-> device copy or pointer query, so it may be captured into a CUDA graph (global capture mode),
+ * and a run (or a replay) after the inputs were rewritten in place gives what the device form gives on the new data.  The
+ * routing between tensor cores and the exact path is decided on the device.  Profiling (b200m_set_profiling) does not
+ * apply to plans.  Destroy a plan only when no work or graph that uses it is left.
+ * Match plans: records of pair p are d_out[d_offsets[p] .. d_offsets[p+1]) as b200m_match_batch_device's; d_n_out gets the
+ * number of records found and only the first min(*d_n_out, cap) are written (*d_n_out > cap: truncated, nothing past cap
+ * is touched); d_offsets are always the full offsets; d_avg (may be NULL) gets the averages (FLT_MAX for a batch without
+ * source rows).  d_offsets [n_pairs + 1], d_n_out [1]. */
+typedef struct b200m_plan b200m_plan;
+B200M_API int b200m_plan_knn_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                                   size_t stride_bytes, int dim, int32_t *d_idx, float *d_dist, int32_t *d_count,
+                                   b200m_plan **plan);
+B200M_API int b200m_plan_match_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                                     size_t stride_bytes, int dim, const float *d_thr_src, const float *d_thr_tgt,
+                                     b200m_corr *d_out, size_t cap, uint64_t *d_offsets, float *d_avg, uint64_t *d_n_out,
+                                     b200m_plan **plan);
+B200M_API int b200m_plan_run(b200m_plan *plan, void *cuda_stream); /* enqueue only */
+B200M_API void b200m_plan_destroy(b200m_plan *plan);
+B200M_API const char *b200m_plan_last_error(const b200m_plan *plan); /* plan may be NULL: errors without a plan */
+
 B200M_API int b200m_version(void);
 
 /* ---- test hooks (used by tests/ only; not part of the reference-facing surface) ----

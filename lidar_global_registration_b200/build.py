@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libb200match.so")
-SOURCES = ["api.cu", "pack.cu", "exact.cu", "filter.cu", "candidates_tc.cu", "multiscale.cu", "cluster.cu", "wide.cu", "multi.cu", "local.cu", "batch.cu", "wide_batch.cu"]
+SOURCES = ["api.cu", "pack.cu", "exact.cu", "filter.cu", "candidates_tc.cu", "multiscale.cu", "cluster.cu", "wide.cu", "multi.cu", "local.cu", "batch.cu", "wide_batch.cu", "plan.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 LINK_VERSION = "cudart-shared-2-dl-pthread"
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

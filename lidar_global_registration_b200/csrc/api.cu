@@ -439,7 +439,8 @@ int b200m_knn_rows(b200m_ctx *ctx, const b200m_params *p, int direction, size_t 
             CK(launch_tc_prepare(ctx));
             tp.stop();
         }
-        use_tc = ctx->prep.usable;
+        // device prepare (batch plans): the candidate kernel routes data outside the window to the exact fallback itself
+        use_tc = ctx->device_prepare || ctx->prep.usable;
     }
     // row selection: compact list of the rows to answer (the one host round trip of this path: the launch geometry
     // of the candidate kernel depends on how many there are)

@@ -111,11 +111,10 @@ int check_device_ptr(b200m_ctx *ctx, const std::string &where, const void *ptr) 
     return 0;
 }
 
-// Validates the batch, packs both sides in the padded layout (replacing what b200m_upload put in the context) and
-// uploads the segment tables.  dev: the descriptor pointers are device pointers, checked here and read in place by the
-// segmented pack (the per-pair SetRef tables and side 1's block table go up with the other tables).
-int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
-                size_t stride_bytes, int dim, BatchLayout *L, bool dev, const float *d_thr_src, const float *d_thr_tgt) {
+// Validates the batch and uploads the segment tables.  dev: the descriptor pointers are device pointers, checked here and
+// read in place by the segmented pack (the per-pair SetRef tables and side 1's block table go up with the other tables).
+int stage_batch_tables(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                       size_t stride_bytes, int dim, BatchLayout *L, bool dev, const float *d_thr_src, const float *d_thr_tgt) {
     const std::string f(fn);
     if (n_pairs < 0) return b200m_fail_msg(ctx, f + ": n_pairs < 0");
     if (n_pairs > 0 && !pairs) return b200m_fail_msg(ctx, f + ": null pairs");
@@ -210,26 +209,39 @@ int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b20
     }
     L->max_rows[0] = max_rows[0];
     L->max_rows[1] = max_rows[1];
+    if (dev) {
+        L->seg_blk[0] = L->block_pair;
+        L->seg_blk[1] = reinterpret_cast<const int32_t *>(d + o_bpair1);
+        L->sets[0] = reinterpret_cast<const SetRef *>(d + o_sets0);
+        L->sets[1] = reinterpret_cast<const SetRef *>(d + o_sets1);
+    }
+    return 0;
+}
+
+int stage_batch_pack(b200m_ctx *ctx, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim, const BatchLayout &L,
+                     bool dev) {
     if (dev) {   // the segmented pack reads every pair's rows where they are and writes the gap rows itself
-        const int32_t *blk[2] = {L->block_pair, reinterpret_cast<const int32_t *>(d + o_bpair1)};
-        const SetRef *d_sets[2] = {reinterpret_cast<const SetRef *>(d + o_sets0), reinterpret_cast<const SetRef *>(d + o_sets1)};
         for (int s = 0; s < 2; ++s)
-            if (upload_common(ctx, s, nullptr, L->n_rows[s], stride_bytes, dim, 0, blk[s], d_sets[s])) return 1;
+            if (upload_common(ctx, s, nullptr, L.n_rows[s], stride_bytes, dim, 0, L.seg_blk[s], L.sets[s])) return 1;
         return 0;
     }
     // descriptors: gap bytes 0xFF (NaN rows), then every pair's rows at its offset -- (n - 1) * stride + dim floats, as
     // b200m_upload copies: the caller owns only `dim` floats of a set's last row
+    cudaStream_t st = ctx->stream;
     for (int s = 0; s < 2; ++s) {
         Side &sd = ctx->side[s];
-        if (L->n_rows[s]) {
-            CK(sd.staging.reserve(L->n_rows[s] * stride_bytes));
-            CK(cudaMemsetAsync(sd.staging.p, 0xFF, L->n_rows[s] * stride_bytes, st));
+        if (L.n_rows[s]) {
+            CK(sd.staging.reserve(L.n_rows[s] * stride_bytes));
+            CK(cudaMemsetAsync(sd.staging.p, 0xFF, L.n_rows[s] * stride_bytes, st));
+            size_t start = 0;   // pair i's first padded row
             for (int i = 0; i < n_pairs; ++i) {
                 const size_t n = s ? pairs[i].n_tgt : pairs[i].n_src;
+                const size_t first = start;
+                start += pad_rows(n);
                 if (!n) continue;
                 const float *src = s ? pairs[i].tgt : pairs[i].src;
                 const size_t bytes = (n - 1) * stride_bytes + (size_t) dim * 4;
-                char *dst = sd.staging.as<char>() + start[s][i] * stride_bytes;
+                char *dst = sd.staging.as<char>() + first * stride_bytes;
                 if (bytes >= ((size_t) 32 << 20) && is_pageable(src)) {
                     if (staged_h2d(ctx, dst, src, bytes)) return 1;
                 } else {
@@ -237,85 +249,36 @@ int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b20
                 }
             }
         }
-        if (upload_common(ctx, s, sd.staging.as<float>(), L->n_rows[s], stride_bytes, dim, 0)) return 1;
+        if (upload_common(ctx, s, sd.staging.as<float>(), L.n_rows[s], stride_bytes, dim, 0)) return 1;
     }
     return 0;
 }
 
-namespace {
+int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                size_t stride_bytes, int dim, BatchLayout *L, bool dev, const float *d_thr_src, const float *d_thr_tgt) {
+    if (stage_batch_tables(ctx, fn, p, pairs, n_pairs, stride_bytes, dim, L, dev, d_thr_src, d_thr_tgt)) return 1;
+    return stage_batch_pack(ctx, pairs, n_pairs, stride_bytes, dim, *L, dev);
+}
 
-// dev: b200m_knn_batch_device (device descriptors, the k-lists are written to the caller's device arrays in place)
-int knn_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
-              size_t stride_bytes, int dim, int32_t *idx, float *dist, int32_t *count) {
-    REQUIRE_CTX();
-    if (check_params(ctx, p)) return 1;
-    const std::string f(fn);
-    if (dev && (check_device_ptr(ctx, f + ": idx", idx) || check_device_ptr(ctx, f + ": dist", dist) ||
-                check_device_ptr(ctx, f + ": count", count)))
-        return 1;
-    BatchLayout L;
-    if (stage_batch(ctx, fn, p, pairs, n_pairs, stride_bytes, dim, &L, dev)) return 1;
-    if (L.real_src == 0) return 0;
-    if (!idx || !dist || !count) return b200m_fail_msg(ctx, f + ": null output pointer");
+int knn_batch_lists(b200m_ctx *ctx, const b200m_params *p, const BatchLayout &L, int32_t *o_idx, float *o_dist, int32_t *o_cnt) {
     const int k = p->k;
     const size_t S = L.n_rows[0];
-    cudaStream_t st = ctx->stream;
     CK(ctx->ws_fidx.reserve(sizeof(int32_t) * S * k));
     CK(ctx->ws_fdist.reserve(sizeof(float) * S * k));
     CK(ctx->ws_fcnt.reserve(sizeof(int32_t) * S));
     if (b200m_knn_rows(ctx, p, 0, 0, S, nullptr, ctx->ws_fidx.as<int32_t>(), ctx->ws_fdist.as<float>(), ctx->ws_fcnt.as<int32_t>(),
                        &L.seg[0]))
         return 1;
-    // the pairs' real rows back to back, with pair-local train indices (the reverse-table buffers are free here; a device
-    // call writes the caller's arrays directly)
-    const size_t R = L.real_src;
-    if (dev) {
-        localize_lists_kernel<<<(unsigned) ((S + 255) / 256), 256, 0, st>>>(
-            ctx->ws_fidx.as<int32_t>(), ctx->ws_fdist.as<float>(), ctx->ws_fcnt.as<int32_t>(), S, k, L.block_pair, L.pair_info,
-            idx, dist, count);
-        CK(cudaGetLastError());
-        ctx->stats.launches += 1;
-        return 0;
-    }
-    CK(ctx->ws_ridx.reserve(sizeof(int32_t) * R * k));
-    CK(ctx->ws_rdist.reserve(sizeof(float) * R * k));
-    CK(ctx->ws_rcnt.reserve(sizeof(int32_t) * R));
-    localize_lists_kernel<<<(unsigned) ((S + 255) / 256), 256, 0, st>>>(
-        ctx->ws_fidx.as<int32_t>(), ctx->ws_fdist.as<float>(), ctx->ws_fcnt.as<int32_t>(), S, k, L.block_pair, L.pair_info,
-        ctx->ws_ridx.as<int32_t>(), ctx->ws_rdist.as<float>(), ctx->ws_rcnt.as<int32_t>());
+    localize_lists_kernel<<<(unsigned) ((S + 255) / 256), 256, 0, ctx->stream>>>(
+        ctx->ws_fidx.as<int32_t>(), ctx->ws_fdist.as<float>(), ctx->ws_fcnt.as<int32_t>(), S, k, L.block_pair, L.pair_info, o_idx,
+        o_dist, o_cnt);
     CK(cudaGetLastError());
     ctx->stats.launches += 1;
-    CK(cudaMemcpyAsync(idx, ctx->ws_ridx.p, sizeof(int32_t) * R * k, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(dist, ctx->ws_rdist.p, sizeof(float) * R * k, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(count, ctx->ws_rcnt.p, sizeof(int32_t) * R, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
     return 0;
 }
 
-// dev: b200m_match_batch_device (device descriptors and thresholds, records to the caller's device buffer)
-int match_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
-                size_t stride_bytes, int dim, const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
-                size_t *offsets, float *avg) {
-    REQUIRE_CTX();
-    if (check_params(ctx, p)) return 1;
-    const std::string f(fn);
-    if (p->mode == B200M_MODE_KNN_ONLY) return b200m_fail_msg(ctx, f + ": use b200m_knn_batch for raw k-lists");
-    if (p->mode == B200M_MODE_CLUSTER)
-        return b200m_fail_msg(ctx, f + ": the cluster filter needs keypoint coordinates, use b200m_match_cluster");
-    if (!offsets) return b200m_fail_msg(ctx, f + ": null offsets");
-    if ((thr_src == nullptr) != (thr_tgt == nullptr))
-        return b200m_fail_msg(ctx, f + ": give both threshold arrays or neither");
-    if (dev && (check_device_ptr(ctx, f + ": thr_src", thr_src) || check_device_ptr(ctx, f + ": thr_tgt", thr_tgt) ||
-                check_device_ptr(ctx, f + ": out", out)))
-        return 1;
-    for (int i = 0; i <= n_pairs; ++i) offsets[i] = 0;
-    BatchLayout L;
-    if (stage_batch(ctx, fn, p, pairs, n_pairs, stride_bytes, dim, &L, dev, thr_src, thr_tgt)) return 1;
-    if (L.real_src == 0) {
-        if (avg)
-            for (int i = 0; i < n_pairs; ++i) avg[i] = 3.402823466e+38F;   // FLT_MAX, reference include/matching.h:41
-        return 0;
-    }
+int match_batch_records(b200m_ctx *ctx, const b200m_params *p, const BatchLayout &L, const b200m_pair *pairs, int n_pairs,
+                        bool dev, const float *thr_src, const float *thr_tgt, bool want_avg) {
     const int k = p->k;
     const bool mutual = p->mode == B200M_MODE_MUTUAL || p->mode == B200M_MODE_RATIO_MUTUAL;
     const size_t S = L.n_rows[0], T = L.n_rows[1];
@@ -371,7 +334,7 @@ int match_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p,
                             d_thr_s, d_thr_t, ctx->ws_corr.as<b200m_corr>(), max_out, L.n_out, nullptr))
         return 1;
     CK(cudaMemsetAsync(L.counts, 0, sizeof(unsigned) * n_pairs, st));
-    if (avg) {
+    if (want_avg) {
         CK(launch_average_segments(ctx->ws_fdist.as<float>(), ctx->ws_fcnt.as<int32_t>(), L.avg_segs, n_pairs, k, L.avgs, st));
         ctx->stats.launches += 1;
     }
@@ -379,6 +342,67 @@ int match_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p,
                                                                           L.block_pair, L.pair_info, L.counts);
     CK(cudaGetLastError());
     ctx->stats.launches += 1;
+    return 0;
+}
+
+namespace {
+
+// dev: b200m_knn_batch_device (device descriptors, the k-lists are written to the caller's device arrays in place)
+int knn_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+              size_t stride_bytes, int dim, int32_t *idx, float *dist, int32_t *count) {
+    REQUIRE_CTX();
+    if (check_params(ctx, p)) return 1;
+    const std::string f(fn);
+    if (dev && (check_device_ptr(ctx, f + ": idx", idx) || check_device_ptr(ctx, f + ": dist", dist) ||
+                check_device_ptr(ctx, f + ": count", count)))
+        return 1;
+    BatchLayout L;
+    if (stage_batch(ctx, fn, p, pairs, n_pairs, stride_bytes, dim, &L, dev)) return 1;
+    if (L.real_src == 0) return 0;
+    if (!idx || !dist || !count) return b200m_fail_msg(ctx, f + ": null output pointer");
+    // the pairs' real rows back to back, with pair-local train indices (a device call writes the caller's arrays directly,
+    // a host call the reverse-table buffers, which are free here)
+    if (dev) return knn_batch_lists(ctx, p, L, idx, dist, count);
+    const int k = p->k;
+    const size_t R = L.real_src;
+    cudaStream_t st = ctx->stream;
+    CK(ctx->ws_ridx.reserve(sizeof(int32_t) * R * k));
+    CK(ctx->ws_rdist.reserve(sizeof(float) * R * k));
+    CK(ctx->ws_rcnt.reserve(sizeof(int32_t) * R));
+    if (knn_batch_lists(ctx, p, L, ctx->ws_ridx.as<int32_t>(), ctx->ws_rdist.as<float>(), ctx->ws_rcnt.as<int32_t>())) return 1;
+    CK(cudaMemcpyAsync(idx, ctx->ws_ridx.p, sizeof(int32_t) * R * k, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(dist, ctx->ws_rdist.p, sizeof(float) * R * k, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(count, ctx->ws_rcnt.p, sizeof(int32_t) * R, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+// dev: b200m_match_batch_device (device descriptors and thresholds, records to the caller's device buffer)
+int match_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                size_t stride_bytes, int dim, const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
+                size_t *offsets, float *avg) {
+    REQUIRE_CTX();
+    if (check_params(ctx, p)) return 1;
+    const std::string f(fn);
+    if (p->mode == B200M_MODE_KNN_ONLY) return b200m_fail_msg(ctx, f + ": use b200m_knn_batch for raw k-lists");
+    if (p->mode == B200M_MODE_CLUSTER)
+        return b200m_fail_msg(ctx, f + ": the cluster filter needs keypoint coordinates, use b200m_match_cluster");
+    if (!offsets) return b200m_fail_msg(ctx, f + ": null offsets");
+    if ((thr_src == nullptr) != (thr_tgt == nullptr))
+        return b200m_fail_msg(ctx, f + ": give both threshold arrays or neither");
+    if (dev && (check_device_ptr(ctx, f + ": thr_src", thr_src) || check_device_ptr(ctx, f + ": thr_tgt", thr_tgt) ||
+                check_device_ptr(ctx, f + ": out", out)))
+        return 1;
+    for (int i = 0; i <= n_pairs; ++i) offsets[i] = 0;
+    BatchLayout L;
+    if (stage_batch(ctx, fn, p, pairs, n_pairs, stride_bytes, dim, &L, dev, thr_src, thr_tgt)) return 1;
+    if (L.real_src == 0) {
+        if (avg)
+            for (int i = 0; i < n_pairs; ++i) avg[i] = 3.402823466e+38F;   // FLT_MAX, reference include/matching.h:41
+        return 0;
+    }
+    if (match_batch_records(ctx, p, L, pairs, n_pairs, dev, thr_src, thr_tgt, avg != nullptr)) return 1;
+    cudaStream_t st = ctx->stream;
     std::vector<char> res(L.result_bytes);
     CK(cudaMemcpyAsync(res.data(), L.n_out, L.result_bytes, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));

@@ -86,6 +86,8 @@ struct TcParams {
                           // 512 = per-warp cycle totals, 1024 = cycle stamps of a few tiles (CTA pair 0),
                           // (n << 12) = n K steps per tile, 32768 = one accumulator, 65536 = no operand ring,
                           // 131072 / 262144 = service-scheduler / all epilogue warps skip a quarter of their columns
+    const PrepDev *prep;  // DP kernels: the prepare step's device decision (usable) and norm bounds (bmax[train_side])
+    int train_side;
 };
 
 // ---- PTX wrappers -------------------------------------------------------------------------
@@ -632,7 +634,11 @@ __device__ __forceinline__ void chunk_hits(float m0, float m1, float m2, float m
 // KS:   (pair mode, EH = 1, kp > 640: 11..32 K atoms) K-streamed operands.  The query tile no longer stays resident: a ring
 //       stage holds this CTA's A atom (128 rows x 64 halves, 16 KB) followed by its half of the B atom (16 KB), and the
 //       producer loads ka stages per train tile.  The certificate's accumulation slop grows with the K steps (DESIGN.md §4).
-template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG, bool SEG, bool KS = false>
+// DP:   (batch plans, next to the SEG instantiations only) device prepare: the train side's norm bound comes from
+//       TcParams::prep instead of TcParams::bmax, and data outside the certificate's window (prep->usable == 0) leaves every
+//       list of the CTA's rows overflowed (count cap + 1, threshold +inf) before anything else, so that the re-rank flags
+//       every valid row and the exact fallback answers it.  A compile-time switch for the reason SEG is one.
+template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG, bool SEG, bool KS = false, bool DP = false>
 __global__ void __launch_bounds__(EPI ? 640 : 64 + 128 * EH + (SPLITN ? 32 : 0), 1)
 tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_t,
                      const TcParams p) {
@@ -692,6 +698,19 @@ tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
     const int t0 = dump ? p.tiles_per_split : seg_t0 + split * tps;   // dump mode: tiles_per_split holds the tile id
     const int t1 = dump ? t0 + 1 : min(seg_t0 + seg_tiles, t0 + tps);
     const int ka = p.ka;
+    if (DP && !p.prep->usable) {
+        // outside the window: both CTAs of a pair read the same word and leave here, before any barrier, TMEM allocation
+        // or pipeline exists, as below
+        const int local = qtile * B200M_TILE_M + (int) threadIdx.x;
+        if (threadIdx.x < B200M_TILE_M && local < p.n_rows) {
+            for (int l = 0; l < kListsPerSplit; ++l) {
+                const size_t list_row = (size_t) (split * kListsPerSplit + l) * p.n_rows + local;
+                p.cand_cnt[list_row] = p.cap + 1;
+                if (p.cand_thr) p.cand_thr[list_row] = INFINITY;
+            }
+        }
+        return;
+    }
     if (SEG && t1 <= t0) {
         // batch: a pair with fewer train tiles than there are splits (or none) leaves this CTA nothing to sweep.  Its rows'
         // lists are empty, with the final threshold an empty list has; the range is the same for both CTAs of a pair, so
@@ -1042,7 +1061,7 @@ tc_candidates_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_co
         }
         {
             const float na = active ? p.q_norm16[p.q_row0 + local] : 0.f;
-            const float ab = sqrtf(na) + p.bmax;
+            const float ab = sqrtf(na) + (DP ? p.prep->bmax[p.train_side] : p.bmax);
             st.s_const = s_rowc + 16u * (uint32_t) row_in_tile;
             // every thread of the row writes the same four values
             sts_f32(st.s_const, na);
@@ -1432,9 +1451,9 @@ int get_tmap(b200m_ctx *ctx, int side, bool as_query, int cluster, const CUtenso
     return 0;
 }
 
-template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG, bool SEG, bool KS = false>
+template <int KT, bool PAIR, int EH, bool SPLITN, int EPI, bool DBG, bool SEG, bool KS = false, bool DP = false>
 int launch_tc(b200m_ctx *ctx, const CUtensorMap *mq, const CUtensorMap *mt, const TcParams &p, dim3 grid, size_t smem) {
-    CK(cudaFuncSetAttribute(tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG, SEG, KS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+    CK(cudaFuncSetAttribute(tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG, SEG, KS, DP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = grid;
     cfg.blockDim = dim3(EPI ? 640 : 64 + 128 * EH + (SPLITN ? 32 : 0), 1, 1);
@@ -1447,7 +1466,7 @@ int launch_tc(b200m_ctx *ctx, const CUtensorMap *mq, const CUtensorMap *mt, cons
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG, SEG, KS>, *mq, *mt, p);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, tc_candidates_kernel<KT, PAIR, EH, SPLITN, EPI, DBG, SEG, KS, DP>, *mq, *mt, p);
     if (e != cudaSuccess) {
         cudaGetLastError();   // do not leave the launch error behind for the next call
         return b200m_fail_msg(ctx, std::string("tc_candidates launch failed: ") + cudaGetErrorString(e) + " (grid " +
@@ -1559,6 +1578,11 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
     p.k = k;
     p.dim = q.dim;
     p.bmax = ctx->prep.max_norm[1 - direction];
+    // device prepare (batch plans): the bound and the routing come from the device; only the SEG kernels have the DP form
+    const bool dp = ctx->device_prepare;
+    if (dp && (!seg || dump)) return b200m_fail_msg(ctx, "tc_candidates: device prepare is a batch form");
+    p.prep = dp ? ctx->prep.red.as<PrepDev>() : nullptr;
+    p.train_side = 1 - direction;
     p.q_norm16 = q_ops ? q_norm : q.norm16.as<float>();
     // A list receives a column whenever it is under the running threshold: for columns in random order that is a
     // record process, E = k (ln(n / k) + 1) appends with variance about E, n = the columns the list's thread sees.
@@ -1607,25 +1631,27 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
     // batch launches (p.seg_range) run the production kernels with the segment lookup: the timing experiments of
     // B200M_TC_DEBUG do not apply to them, and dump mode is single-pair only
     const bool dbg = dump != nullptr || ctx->tc_debug != 0;
-#define B200M_TC_CASE2(KT_, DBG_, SEG_)                                                            \
-    rc = pair ? (eh == 2 ? (epi == 5 ? launch_tc<KT_, true, 2, true, 5, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)        \
-                            : epi == 4 ? launch_tc<KT_, true, 2, true, 4, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)      \
-                            : epi == 2 ? launch_tc<KT_, true, 2, true, 2, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)      \
-                            : epi == 1 ? launch_tc<KT_, true, 2, true, 1, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)      \
-                            : splitn ? launch_tc<KT_, true, 2, true, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)        \
-                                     : launch_tc<KT_, true, 2, false, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem))      \
-                         : launch_tc<KT_, true, 1, false, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem))                  \
-              : (eh == 2 ? launch_tc<KT_, false, 2, false, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem)                  \
-                         : launch_tc<KT_, false, 1, false, 0, DBG_, SEG_>(ctx, mq, mt, p, grid, smem))
+#define B200M_TC_CASE2(KT_, DBG_, SEG_, DP_)                                                                     \
+    rc = pair ? (eh == 2 ? (epi == 5 ? launch_tc<KT_, true, 2, true, 5, DBG_, SEG_, false, DP_>(ctx, mq, mt, p, grid, smem)   \
+                            : epi == 4 ? launch_tc<KT_, true, 2, true, 4, DBG_, SEG_, false, DP_>(ctx, mq, mt, p, grid, smem) \
+                            : epi == 2 ? launch_tc<KT_, true, 2, true, 2, DBG_, SEG_, false, DP_>(ctx, mq, mt, p, grid, smem) \
+                            : epi == 1 ? launch_tc<KT_, true, 2, true, 1, DBG_, SEG_, false, DP_>(ctx, mq, mt, p, grid, smem) \
+                            : splitn ? launch_tc<KT_, true, 2, true, 0, DBG_, SEG_, false, DP_>(ctx, mq, mt, p, grid, smem)   \
+                                     : launch_tc<KT_, true, 2, false, 0, DBG_, SEG_, false, DP_>(ctx, mq, mt, p, grid, smem)) \
+                         : launch_tc<KT_, true, 1, false, 0, DBG_, SEG_, false, DP_>(ctx, mq, mt, p, grid, smem))             \
+              : (eh == 2 ? launch_tc<KT_, false, 2, false, 0, DBG_, SEG_, false, DP_>(ctx, mq, mt, p, grid, smem)             \
+                         : launch_tc<KT_, false, 1, false, 0, DBG_, SEG_, false, DP_>(ctx, mq, mt, p, grid, smem))
 #define B200M_TC_CASE_KS(KT_)                                                                                  \
-    if (p.seg_range) rc = launch_tc<KT_, true, 1, false, 0, false, true, true>(ctx, mq, mt, p, grid, smem);        \
+    if (p.seg_range && dp) rc = launch_tc<KT_, true, 1, false, 0, false, true, true, true>(ctx, mq, mt, p, grid, smem); \
+    else if (p.seg_range) rc = launch_tc<KT_, true, 1, false, 0, false, true, true>(ctx, mq, mt, p, grid, smem);   \
     else if (dbg) rc = launch_tc<KT_, true, 1, false, 0, true, false, true>(ctx, mq, mt, p, grid, smem);           \
     else rc = launch_tc<KT_, true, 1, false, 0, false, false, true>(ctx, mq, mt, p, grid, smem);
-#define B200M_TC_CASE(KT_)                              \
-    if (ks) { B200M_TC_CASE_KS(KT_) }                      \
-    else if (p.seg_range) { B200M_TC_CASE2(KT_, false, true); } \
-    else if (dbg) { B200M_TC_CASE2(KT_, true, false); }    \
-    else { B200M_TC_CASE2(KT_, false, false); }
+#define B200M_TC_CASE(KT_)                                         \
+    if (ks) { B200M_TC_CASE_KS(KT_) }                                 \
+    else if (p.seg_range && dp) { B200M_TC_CASE2(KT_, false, true, true); } \
+    else if (p.seg_range) { B200M_TC_CASE2(KT_, false, true, false); } \
+    else if (dbg) { B200M_TC_CASE2(KT_, true, false, false); }        \
+    else { B200M_TC_CASE2(KT_, false, false, false); }
     switch (kt) {
         case 1: B200M_TC_CASE(1); break;
         case 2: B200M_TC_CASE(2); break;

@@ -40,6 +40,16 @@ struct Side {
     DevBuf norm16;         // [n_pad] float: |x16|^2 in scaled units
 };
 
+// Device-resident results of the prepare step (pack.cu), in TcPrep::red: written by prep_finalize / pack_operands, read by
+// the operand pack, copied to the host once afterwards -- or, in a context with device_prepare, turned into the routing
+// decision by prep_decide_kernel and read by the candidate kernel (DP form) instead.
+struct PrepDev {
+    int maxabs_bits;        // max |x - mean| over the valid rows of both sides, as the bits of a non-negative float
+    int max_norm_bits[2];   // max |x16| per side, likewise (atomicMax)
+    int usable;             // device_prepare: 1 when the data lies inside the certificate's window (tc_window, pack.cu)
+    float bmax[2];          // device_prepare: max |b16| per side, the candidate kernel's norm bound of that side as train side
+};
+
 struct TcPrep {            // state shared by both sides' FP16 operands
     uint64_t ver[2] = {0, 0};
     bool ready = false;
@@ -88,6 +98,10 @@ struct b200m_ctx {
     int tc_lean = 1;       // B200M_TC_LEAN=0: general MMA issue loop also for one-atom descriptors (comparison)
     int tc_debug = 0;      // B200M_TC_DEBUG: timing experiments (results are NOT valid when set)
     int tc_pair = 1;       // 1 = CTA-pair (cta_group::2) candidate kernel; 0 = cta_group::1 + multicast (B200M_TC_MODE=mcast)
+    // Batch plans (plan.cu): the tensor-core / exact routing and the norm bounds stay on the device (prep_decide_kernel and
+    // the candidate kernel's DP form), so the kNN driver enqueues without a host round trip.  Only a plan's private
+    // context sets it.
+    bool device_prepare = false;
     bool profiling = false;
     b200m_stats stats{};
     cudaEvent_t ev[2] = {nullptr, nullptr};
@@ -155,14 +169,31 @@ struct BatchLayout {
     size_t result_bytes = 0;
     size_t max_rows[2] = {0, 0};                   // largest set per side
     const struct GatherSet *thr_sets[2] = {nullptr, nullptr};   // device calls with thresholds: [n_pairs] per side
+    const int32_t *seg_blk[2] = {nullptr, nullptr};   // device calls: per side block -> pair table of the segmented pack
+    const SetRef *sets[2] = {nullptr, nullptr};       // device calls: per side [n_pairs] sets of the segmented pack
 };
 // Validates the pairs, packs both sides in the padded layout (replacing what b200m_upload put in the context) and uploads
 // the segment tables into ctx->ws_batch.  dev: every descriptor pointer is a device pointer of the context's device
 // (checked; the segmented pack reads the sets in place); d_thr_src / d_thr_tgt (dev only): the concatenated device
 // thresholds, for which gather tables into the padded layout go up with the segment tables.
+// = stage_batch_tables, then stage_batch_pack.
 int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
                 size_t stride_bytes, int dim, BatchLayout *L, bool dev = false, const float *d_thr_src = nullptr,
                 const float *d_thr_tgt = nullptr);
+// The validation and the tables (one upload into ctx->ws_batch, reserved here); nothing is packed.
+int stage_batch_tables(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                       size_t stride_bytes, int dim, BatchLayout *L, bool dev, const float *d_thr_src, const float *d_thr_tgt);
+// The pack of both sides into the layout the tables describe.  dev: kernels only (no copy, no allocation once the sides'
+// buffers have grown to the layout), which is what a batch plan's run enqueues.
+int stage_batch_pack(b200m_ctx *ctx, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim, const BatchLayout &L,
+                     bool dev);
+// After stage_batch: the k-lists of every pair, pair-local, rows back to back, into the device arrays o_idx / o_dist / o_cnt.
+int knn_batch_lists(b200m_ctx *ctx, const b200m_params *p, const BatchLayout &L, int32_t *o_idx, float *o_dist, int32_t *o_cnt);
+// After stage_batch (real_src > 0): kNN, thresholds, filter, averages (want_avg: into L.avgs) and the records made pair-local
+// in ctx->ws_corr, their number in *L.n_out and the per-pair counts in L.counts.  dev: thresholds are device pointers (filed
+// by the gather tables), else host arrays.
+int match_batch_records(b200m_ctx *ctx, const b200m_params *p, const BatchLayout &L, const b200m_pair *pairs, int n_pairs,
+                        bool dev, const float *thr_src, const float *thr_tgt, bool want_avg);
 
 // Device batch calls: `rows` rows of `w` 4-byte words, src_stride words apart at `src`, go to rows dst_row.. of a
 // destination (dst_stride words apart).  src = null writes the identity (row r -> r, w = 1): a NULL index map.
@@ -188,7 +219,9 @@ cudaError_t launch_pack_f32(const float *aos, size_t n, size_t stride_bytes, int
                             float *f32, uint8_t *valid, float *stats, int sm_count, cudaStream_t st,
                             const int32_t *seg_blk = nullptr, const SetRef *sets = nullptr);
 size_t pack_stats_bytes(int sm_count, int dp);
-cudaError_t launch_tc_prepare(b200m_ctx *ctx);   // centre/scale + FP16 operand tiles for both sides
+// centre/scale + FP16 operand tiles for both sides; with ctx->device_prepare the routing decision and the norm bounds stay
+// in PrepDev (prep_decide_kernel) and nothing is read back
+cudaError_t launch_tc_prepare(b200m_ctx *ctx);
 
 // exact.cu
 cudaError_t launch_exact_rows(const float *q_f32, const uint8_t *q_valid, int dp, int dim,

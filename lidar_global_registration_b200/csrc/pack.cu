@@ -171,13 +171,6 @@ pack_stats_long_kernel(const float *__restrict__ f32, const uint8_t *__restrict_
     }
 }
 
-// device-resident results of the statistics pass (read by the operand pack; copied to the host once, afterwards)
-struct PrepDev {
-    int maxabs_bits;        // max |x - mean| over the valid rows of both sides, as the bits of a non-negative float
-    int max_norm_bits[2];   // max |x16| per side, likewise (atomicMax)
-    int pad;
-};
-
 // power of two s with maxabs*s in (0.5, 1]; all-equal data (maxabs == 0) keeps s = 1
 __host__ __device__ inline float scale_for(float maxabs) {
     float scale = 1.f;
@@ -188,6 +181,16 @@ __host__ __device__ inline float scale_for(float maxabs) {
         scale = ldexpf(1.f, -ex);
     }
     return scale;
+}
+
+// The certificate's window (DESIGN.md §4); data outside it stays on the exact path.  Upper edge: the reference's FP32 sum
+// of D squared differences, each at most (2 maxabs)^2, stays finite.  Lower edge: the subnormal rounding of those terms (at
+// most 2^-150 each, D 2^-150 s^2 in scaled units) stays under 2^-25, inside the 1e-6 that slop carries on top of the
+// accumulator bound.  The host (launch_tc_prepare) and the device (prep_decide_kernel) decide with this one function.
+__host__ __device__ inline bool tc_window(float maxabs, float scale, int dim) {
+    const double m = maxabs, s = scale, gam = (dim + 4) * 0x1p-24;
+    return isfinite(maxabs) && isfinite(scale) && scale > 0.f &&
+           (maxabs == 0.f || (dim * 4.0 * m * m * (1.0 + gam) < (double) FLT_MAX && dim * s * s <= 0x1p125));
 }
 
 // Combine the per-CTA column statistics of both sides: CTA b owns columns 32b..32b+31, its eight warps each fold
@@ -314,6 +317,14 @@ pack_operands_kernel(const float *__restrict__ f32, const uint8_t *__restrict__ 
     if (lane == 0 && max_nf > 0.f) atomicMax(&prep->max_norm_bits[side], __float_as_int(sqrtf(max_nf)));
 }
 
+// device_prepare: the routing decision and the norm bounds, from the statistics and operand passes before it (one thread)
+__global__ void prep_decide_kernel(PrepDev *__restrict__ prep, int dim) {
+    const float maxabs = __int_as_float(prep->maxabs_bits);
+    prep->usable = tc_window(maxabs, scale_for(maxabs), dim) ? 1 : 0;
+    prep->bmax[0] = __int_as_float(prep->max_norm_bits[0]);
+    prep->bmax[1] = __int_as_float(prep->max_norm_bits[1]);
+}
+
 }  // namespace
 
 int pack_stats_blocks(int sm_count) { return sm_count * 2; }
@@ -386,6 +397,15 @@ cudaError_t launch_tc_prepare(b200m_ctx *ctx) {
                 sd.op_query.as<__half>(), sd.op_train.as<__half>(), sd.norm16.as<float>());
         ctx->stats.launches += 1;
     }
+    if (ctx->device_prepare) {   // no round trip: the candidate kernel's DP form reads the decision from PrepDev
+        prep_decide_kernel<<<1, 1, 0, st>>>(dev, dim);
+        ctx->stats.launches += 1;
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+        pr.ver[0] = a.version;
+        pr.ver[1] = b.version;
+        pr.ready = true;
+        return cudaSuccess;
+    }
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     // the one host round trip of the prepare step: scale, usability and the per-side norm bounds
     PrepDev h;
@@ -395,13 +415,7 @@ cudaError_t launch_tc_prepare(b200m_ctx *ctx) {
     memcpy(&maxabs, &h.maxabs_bits, 4);
     const float scale = scale_for(maxabs);
     pr.scale = scale;
-    // The certificate's window (DESIGN.md §4); data outside it stays on the exact path.  Upper edge: the reference's
-    // FP32 sum of D squared differences, each at most (2 maxabs)^2, stays finite.  Lower edge: the subnormal rounding
-    // of those terms (at most 2^-150 each, D 2^-150 s^2 in scaled units) stays under 2^-25, inside the 1e-6 that slop
-    // carries on top of the accumulator bound.
-    const double m = maxabs, s = scale, gam = (dim + 4) * 0x1p-24;
-    pr.usable = isfinite(maxabs) && isfinite(scale) && scale > 0.f &&
-                (maxabs == 0.f || (dim * 4.0 * m * m * (1.0 + gam) < (double) FLT_MAX && dim * s * s <= 0x1p125));
+    pr.usable = tc_window(maxabs, scale, dim);
     memcpy(&pr.max_norm[0], &h.max_norm_bits[0], 4);
     memcpy(&pr.max_norm[1], &h.max_norm_bits[1], 4);
     pr.ver[0] = a.version;

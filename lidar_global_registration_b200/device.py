@@ -1,6 +1,7 @@
 """Device-resident and multi-GPU drivers of the matcher on torch tensors (HBM buffers, the current torch stream).
 
     GpuBackend      one b200m context working on torch device buffers (no host copies), single pairs and batches
+    BatchPlan       a device batch call bound once (b200m_plan_*): run() only enqueues, so torch.cuda.graph can capture it
     ShardedMatcher  SURVEY 8e, one process per GPU: query-sharded / target-replicated matcher and the target-sharded kNN.
                     With a GpuBackend this is a THIN caller of the library -- partitioning, the NCCL exchange step and
                     the merge live in libb200match.so (csrc/multi.cu: b200m_match_sharded_device,
@@ -9,6 +10,8 @@
                     torch.distributed collectives is kept for backends without native sharding: the CPU tests drive it
                     with gloo and a stand-in backend as an executable statement of the exchange protocol.
 """
+import ctypes as C
+
 import torch
 
 from . import matcher as M
@@ -238,6 +241,71 @@ class GpuBackend:
                                                    ratio_thr, distance_thr, self.precision, self.cand_cap)
         return [(out[int(offsets[i]):int(offsets[i + 1])], float(avg[i])) for i in range(len(pairs))]
 
+    # -- batch plans (b200m_plan_*): bound once, then enqueued without the host ----------------------------------------
+    def plan_knn_batch(self, k, pairs, dim):
+        """A BatchPlan of knn_batch over `pairs` (as knn_batch takes them).  The plan binds the tensors themselves: run()
+        answers on whatever they hold when it runs.  Outputs: plan.idx [sum n_src, k], plan.dist, plan.cnt [sum n_src]."""
+        ptrs, stride = self._set_pairs(pairs, dim)
+        total = sum(p[1] for p in ptrs)
+        out = dict(idx=torch.empty((total, k), dtype=torch.int32, device=self.device),
+                   dist=torch.empty((total, k), dtype=torch.float32, device=self.device),
+                   cnt=torch.empty((total,), dtype=torch.int32, device=self.device))
+        p = M.Context._params(k, M.MODE_KNN_ONLY, precision=self.precision, cand_cap=self.cand_cap)
+        arr = M.Context._device_pairs(ptrs)
+        make = lambda h: self.ctx._L.b200m_plan_knn_batch(self.ctx._h, C.byref(p), arr, len(ptrs), stride, dim,
+                                                          self._ptr(out["idx"]), self._ptr(out["dist"]),
+                                                          self._ptr(out["cnt"]), h)
+        return BatchPlan(self, ptrs, list(pairs), out, make)
+
+    def plan_match_batch(self, k, mode, pairs, dim, cap=None, thr_src=None, thr_tgt=None, ratio_thr=M.MATCHING_RATIO_THRESHOLD,
+                         distance_thr=M.FLT_MAX):
+        """A BatchPlan of match_batch over `pairs`.  thr_src / thr_tgt: None or one 1-D float32 tensor per pair, bound in
+        place, so they must be consecutive slices of one tensor per side in pair order (torch.split of it).  cap: records
+        the plan writes (default sum n_src * (k if MUTUAL else 1), enough for any data).  Outputs: plan.records int32
+        [cap, 4] (CORR_DTYPE layout), plan.offsets int64 [n_pairs + 1], plan.avg float32 [n_pairs], plan.n_out int64 [1]
+        (records found; above cap the records were truncated)."""
+        ptrs, stride = self._set_pairs(pairs, dim)
+        if (thr_src is None) != (thr_tgt is None):
+            raise M.B200MatchError("give both threshold lists or neither")
+        keep = list(pairs)
+        thr = [0, 0]
+        if thr_src is not None:
+            for side, (thrs, col) in enumerate(((thr_src, 1), (thr_tgt, 3))):
+                if len(thrs) != len(ptrs):
+                    raise M.B200MatchError("one threshold array per pair and side")
+                thr[side], t = self._bound_thresholds(thrs, [q[col] for q in ptrs], "thr_src" if side == 0 else "thr_tgt")
+                keep.append(t)
+        kk = k if mode == M.MODE_MUTUAL else 1
+        cap = max(sum(q[1] for q in ptrs) * kk, 1) if cap is None else int(cap)
+        out = dict(records=torch.empty((cap, 4), dtype=torch.int32, device=self.device),
+                   offsets=torch.zeros((len(ptrs) + 1,), dtype=torch.int64, device=self.device),
+                   avg=torch.empty((len(ptrs),), dtype=torch.float32, device=self.device),
+                   n_out=torch.zeros((1,), dtype=torch.int64, device=self.device))
+        p = M.Context._params(k, mode, ratio_thr, distance_thr, self.precision, self.cand_cap)
+        arr = M.Context._device_pairs(ptrs)
+        make = lambda h: self.ctx._L.b200m_plan_match_batch(self.ctx._h, C.byref(p), arr, len(ptrs), stride, dim, thr[0], thr[1],
+                                                            self._ptr(out["records"]), cap, self._ptr(out["offsets"]),
+                                                            self._ptr(out["avg"]), self._ptr(out["n_out"]), h)
+        return BatchPlan(self, ptrs, keep, out, make)
+
+    def _bound_thresholds(self, thrs, counts, what):
+        """per-pair threshold tensors that lie back to back in one tensor -> (device pointer of the first, what to keep)"""
+        base, expect = None, None
+        for i, (t, n) in enumerate(zip(thrs, counts)):
+            self._check_vec(t, "pair %d: %s" % (i, what), n, torch.float32)
+            if n == 0:
+                continue
+            if base is None:
+                base = expect = t.data_ptr()
+            if t.data_ptr() != expect:
+                raise M.B200MatchError("%s: a plan binds the thresholds in place; they must be consecutive slices of one tensor "
+                                       "in pair order (pair %d is not)" % (what, i))
+            expect += 4 * n
+        if base is None:   # no rows on this side: any device word stands for the empty array
+            t = torch.zeros((1,), dtype=torch.float32, device=self.device)
+            return t.data_ptr(), t
+        return base, list(thrs)
+
     def match_wide_batch(self, k, mode, pairs, dim=None, cluster_k=M.MATCHING_CLUSTER_K, distance_thr=M.FLT_MAX, thr_src=None,
                          thr_tgt=None):
         """b200m_match_multiscale_batch_device: the dicts of Context.match_wide_batch (src_scales / tgt_scales = lists of
@@ -306,6 +374,60 @@ class GpuBackend:
                                                                   out.data_ptr(), cap, cluster_k, distance_thr, self._ptr(ts),
                                                                   self._ptr(tt))
         return [(out[int(offsets[i]):int(offsets[i + 1])], float(avg[i])) for i in range(len(pairs))]
+
+
+class BatchPlan:
+    """A device batch call bound once (GpuBackend.plan_knn_batch / plan_match_batch).  run() enqueues it on torch's current
+    stream with no host round trip, allocation or copy, so it may be captured in torch.cuda.graph; a run or a replay
+    answers on what the bound input tensors hold at that time.  The outputs are the plan's static tensors (attributes)."""
+
+    def __init__(self, backend, ptrs, keep, outputs, make):
+        self._L = backend.ctx._L
+        self._h = None
+        self.device = backend.device
+        self.counts = [(q[1], q[3]) for q in ptrs]
+        self._keep = keep            # the bound tensors stay alive as long as the plan
+        self.kind = "match" if "records" in outputs else "knn"
+        for name, t in outputs.items():
+            setattr(self, name, t)
+        backend.use_torch_stream()   # creation runs the batch once on the context's stream: after torch's writes
+        h = C.c_void_p()
+        if make(C.byref(h)) != 0:
+            raise M.B200MatchError(self._L.b200m_last_error(backend.ctx._h).decode())
+        self._h = h
+
+    def run(self):
+        """Enqueue the batch on torch's current stream (nothing is returned; the outputs are the plan's tensors)."""
+        if self._L.b200m_plan_run(self._h, torch.cuda.current_stream(self.device).cuda_stream) != 0:
+            raise M.B200MatchError(self._L.b200m_plan_last_error(self._h).decode())
+
+    def results(self):
+        """Synchronise torch's current stream and split the outputs into per-pair views: knn -> [(idx, dist, cnt)], match
+        -> [(records int32 [n, 4], average)], as GpuBackend.knn_batch / match_batch return them."""
+        torch.cuda.current_stream(self.device).synchronize()
+        out, a = [], 0
+        if self.kind == "knn":
+            for ns, _ in self.counts:
+                out.append((self.idx[a:a + ns], self.dist[a:a + ns], self.cnt[a:a + ns]))
+                a += ns
+            return out
+        n = int(self.n_out.item())
+        if n > self.records.shape[0]:
+            raise M.B200MatchError("plan output capacity too small (%d correspondences)" % n)
+        offsets = self.offsets.cpu().tolist()
+        avg = self.avg.cpu().tolist()
+        return [(self.records[offsets[i]:offsets[i + 1]], avg[i]) for i in range(len(self.counts))]
+
+    def close(self):
+        if self._h:
+            self._L.b200m_plan_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def records_to_numpy(records, n_out):

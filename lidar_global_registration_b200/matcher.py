@@ -92,7 +92,8 @@ EXPORTS = ["b200m_create", "b200m_destroy", "b200m_last_error", "b200m_set_strea
            "b200m_create_multi", "b200m_destroy_multi", "b200m_group_last_error", "b200m_group_size", "b200m_group_ctx",
            "b200m_group_upload", "b200m_group_upload_sharded", "b200m_group_match", "b200m_group_knn", "b200m_knn_batch",
            "b200m_match_batch", "b200m_match_multiscale_batch", "b200m_match_multiscale_local_batch", "b200m_knn_batch_device",
-           "b200m_match_batch_device", "b200m_match_multiscale_batch_device", "b200m_match_multiscale_local_batch_device"]
+           "b200m_match_batch_device", "b200m_match_multiscale_batch_device", "b200m_match_multiscale_local_batch_device",
+           "b200m_plan_knn_batch", "b200m_plan_match_batch", "b200m_plan_run", "b200m_plan_destroy", "b200m_plan_last_error"]
 
 _lib = None
 
@@ -171,6 +172,14 @@ def load_library():
     L.b200m_match_batch_device.argtypes = L.b200m_match_batch.argtypes
     L.b200m_match_multiscale_batch_device.argtypes = L.b200m_match_multiscale_batch.argtypes
     L.b200m_match_multiscale_local_batch_device.argtypes = L.b200m_match_multiscale_local_batch.argtypes
+    L.b200m_plan_knn_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Pair), C.c_int, sz, C.c_int, vp, vp, vp, C.POINTER(vp)]
+    L.b200m_plan_match_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Pair), C.c_int, sz, C.c_int, vp, vp, vp, sz, vp, vp,
+                                         vp, C.POINTER(vp)]
+    L.b200m_plan_run.argtypes = [vp, vp]
+    L.b200m_plan_destroy.argtypes = [vp]
+    L.b200m_plan_destroy.restype = None
+    L.b200m_plan_last_error.argtypes = [vp]
+    L.b200m_plan_last_error.restype = C.c_char_p
     L.b200m_version.restype = C.c_int
     L.b200m_debug_operands.argtypes = [vp, C.c_int, C.c_int, vp, sz, vp, C.POINTER(C.c_float), C.POINTER(i32),
                                        C.POINTER(i64)]
