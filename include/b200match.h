@@ -455,9 +455,36 @@ B200M_API int b200m_plan_match_batch(b200m_ctx *ctx, const b200m_params *p, cons
                                      size_t stride_bytes, int dim, const float *d_thr_src, const float *d_thr_tgt,
                                      b200m_corr *d_out, size_t cap, uint64_t *d_offsets, float *d_avg, uint64_t *d_n_out,
                                      b200m_plan **plan);
+/* Matcher-class plans: b200m_match_multiscale_batch_device's / b200m_match_multiscale_local_batch_device's arguments, with
+ * the offsets and averages on the device and two more device words, d_n_out and d_status.  Creation copies the host arrays
+ * (pairs, their scales, locals) and binds the device pointers inside them; every scale's tables are built once.  A run
+ * re-gathers every map and coordinate table, packs and matches every scale, votes, filters, averages and localises, then
+ * writes d_offsets [n_pairs + 1], d_avg [n_pairs] (may be NULL; FLT_MAX for a pair without voted forward lists and for
+ * every pair of a batch without source keypoints), d_n_out and the first min(*d_n_out, cap) records, as match plans do
+ * (cap = the total source keypoints is always enough: the voted lists hold at most one match per source keypoint).
+ * d_status gets the bad-map key, a public layout: ~0 when every map entry was in range, otherwise the first bad entry by
+ * (scale, pair, side) as (scale << 48) | (pair << 16) | side, side 0 = a source map, 1 = a target map.  Every run starts
+ * from a clean key, so a replay after the map was fixed reports ~0 again.  Creation fails, with the device form's text,
+ * when its own run finds a bad entry. */
+B200M_API int b200m_plan_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs,
+                                                int n_pairs, size_t stride_bytes, int dim, size_t xyz_stride_bytes,
+                                                int cluster_k, const float *d_thr_src, const float *d_thr_tgt,
+                                                b200m_corr *d_out, size_t cap, uint64_t *d_offsets, float *d_avg,
+                                                uint64_t *d_n_out, uint64_t *d_status, b200m_plan **plan);
+B200M_API int b200m_plan_match_multiscale_local_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs,
+                                                      const b200m_local_pair *locals, int n_pairs, size_t stride_bytes,
+                                                      int dim, size_t xyz_stride_bytes, int cluster_k,
+                                                      float match_search_radius, const float *d_thr_src,
+                                                      const float *d_thr_tgt, b200m_corr *d_out, size_t cap,
+                                                      uint64_t *d_offsets, float *d_avg, uint64_t *d_n_out,
+                                                      uint64_t *d_status, b200m_plan **plan);
 B200M_API int b200m_plan_run(b200m_plan *plan, void *cuda_stream); /* enqueue only */
 B200M_API void b200m_plan_destroy(b200m_plan *plan);
 B200M_API const char *b200m_plan_last_error(const b200m_plan *plan); /* plan may be NULL: errors without a plan */
+/* The text of a status word: NULL for ~0, else "pair P, scale S: an index map entry of the source|target cloud is outside
+ * its keypoint range" -- the device forms fail with this text after their name.  Valid until the next call with the same
+ * plan (plan may be NULL). */
+B200M_API const char *b200m_plan_status_error(const b200m_plan *plan, uint64_t status);
 
 B200M_API int b200m_version(void);
 

@@ -114,7 +114,8 @@ int check_device_ptr(b200m_ctx *ctx, const std::string &where, const void *ptr) 
 // Validates the batch and uploads the segment tables.  dev: the descriptor pointers are device pointers, checked here and
 // read in place by the segmented pack (the per-pair SetRef tables and side 1's block table go up with the other tables).
 int stage_batch_tables(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
-                       size_t stride_bytes, int dim, BatchLayout *L, bool dev, const float *d_thr_src, const float *d_thr_tgt) {
+                       size_t stride_bytes, int dim, BatchLayout *L, bool dev, const float *d_thr_src, const float *d_thr_tgt,
+                       DevBuf *dst) {
     const std::string f(fn);
     if (n_pairs < 0) return b200m_fail_msg(ctx, f + ": n_pairs < 0");
     if (n_pairs > 0 && !pairs) return b200m_fail_msg(ctx, f + ": null pairs");
@@ -191,8 +192,9 @@ int stage_batch_tables(b200m_ctx *ctx, const char *fn, const b200m_params *p, co
         avg_segs[i] = make_int2(s0, ns);
         dense += (size_t) ns;
     }
-    CK(ctx->ws_batch.reserve(o_res + L->result_bytes));
-    char *d = ctx->ws_batch.as<char>();
+    if (!dst) dst = &ctx->ws_batch;
+    CK(dst->reserve(o_res + L->result_bytes));
+    char *d = dst->as<char>();
     cudaStream_t st = ctx->stream;
     CK(cudaMemcpyAsync(d, h.data(), o_res, cudaMemcpyHostToDevice, st));
     L->seg[0] = SegTable{reinterpret_cast<const int2 *>(d + o_range0), (int) (pad_rows(max_rows[1]) / B200M_TILE_N)};

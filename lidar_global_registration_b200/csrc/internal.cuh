@@ -5,6 +5,7 @@
 #include <stdint.h>
 
 #include <string>
+#include <vector>
 
 #include "../../include/b200match.h"
 
@@ -180,9 +181,10 @@ struct BatchLayout {
 int stage_batch(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
                 size_t stride_bytes, int dim, BatchLayout *L, bool dev = false, const float *d_thr_src = nullptr,
                 const float *d_thr_tgt = nullptr);
-// The validation and the tables (one upload into ctx->ws_batch, reserved here); nothing is packed.
+// The validation and the tables (one upload into *dst, ctx->ws_batch when null, reserved here); nothing is packed.
 int stage_batch_tables(b200m_ctx *ctx, const char *fn, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
-                       size_t stride_bytes, int dim, BatchLayout *L, bool dev, const float *d_thr_src, const float *d_thr_tgt);
+                       size_t stride_bytes, int dim, BatchLayout *L, bool dev, const float *d_thr_src, const float *d_thr_tgt,
+                       DevBuf *dst = nullptr);
 // The pack of both sides into the layout the tables describe.  dev: kernels only (no copy, no allocation once the sides'
 // buffers have grown to the layout), which is what a batch plan's run enqueues.
 int stage_batch_pack(b200m_ctx *ctx, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim, const BatchLayout &L,
@@ -309,6 +311,49 @@ int ms_vote_batch_device(b200m_ctx *ctx, MultiscaleState *ms, const float *d_tra
 // wide.cu
 void wide_release(b200m_ctx *ctx);
 void wide_batch_release(b200m_ctx *ctx);
+
+// wide_batch.cu: b200m_match_multiscale(_local)_batch(_device) in three parts.  wide_batch_tables validates the call and
+// uploads every table once; wide_batch_enqueue queues the batch with kernels and memsets only (no copy, no read-back, and
+// no allocation once the workspaces have grown to the call's shapes); wide_batch_results reads the result area back (host
+// and device forms).  A batch plan (plan.cu) calls the first at creation and the second on every run.
+struct WideCall {
+    const char *name = "";
+    bool dev = false, gated = false;
+    b200m_params p{};
+    const b200m_wide_pair *pairs = nullptr;
+    const b200m_local_pair *locals = nullptr;   // gated calls
+    int n_pairs = 0;
+    size_t stride_bytes = 0, xyz_stride_bytes = 0;
+    int dim = 0, cluster_k = 0;
+    float radius = 0.f;                          // gated calls: match_search_radius
+    const float *thr_src = nullptr, *thr_tgt = nullptr;
+    const b200m_corr *out = nullptr;             // dev: checked with the other pointers
+    bool want_avg = false;
+};
+struct WideLayout {
+    int n_scales = 0;   // 0: no pair has source keypoints and a scale -- nothing is queued
+    bool two_way = false;
+    size_t NS = 0, NT = 0;   // keypoints per side, all pairs
+    b200m_params pk{};       // the kNN passes' params
+    std::vector<std::vector<b200m_pair>> sets;   // [scale][pair] descriptor sets (empty past a pair's scales)
+    std::vector<BatchLayout> scale_tables;       // keep_scales: every scale's batch tables, staged once
+    char *d = nullptr;                           // the uploaded tables, the result area first
+    size_t result_bytes = 0, o_avgs = 0, o_off[2] = {0, 0}, o_rad[2] = {0, 0}, o_segs = 0, o_gmap = 0, o_gxyz = 0;
+    std::vector<size_t> o_rows, o_blk[2], o_map[2];
+    size_t n_gmap = 0, max_map_rows = 0, max_kps[2] = {0, 0};
+    // the result area: record count, bad-map key (~0 = clean), per-pair counts and averages
+    unsigned long long *n_out = nullptr, *bad = nullptr;
+    unsigned *counts = nullptr;
+    float *avgs = nullptr;
+};
+// keep_scales (plans): also stage every scale's batch tables, each into a buffer of its own
+int wide_batch_tables(b200m_ctx *ctx, const WideCall &c, WideLayout *W, bool keep_scales);
+int wide_batch_enqueue(b200m_ctx *ctx, const WideCall &c, const WideLayout &W);
+int wide_batch_results(b200m_ctx *ctx, const WideCall &c, const WideLayout &W, b200m_corr *out, size_t cap, size_t *offsets,
+                       float *avg);
+// The text of a bad-map key (flag_bad): "pair P, scale S: an index map entry of the source|target cloud is outside its
+// keypoint range"
+std::string map_status_text(unsigned long long key);
 
 // multi.cu
 void comm_release(b200m_ctx *ctx);

@@ -319,7 +319,9 @@ class GpuBackend:
         latter may be None in ONE_SIDED mode), as Context.match_wide_local_batch takes them."""
         return self._wide_batch(k, mode, pairs, float(match_search_radius), dim, cluster_k, distance_thr, thr_src, thr_tgt)
 
-    def _wide_batch(self, k, mode, pairs, radius, dim, cluster_k, distance_thr, thr_src, thr_tgt):
+    def _wide_args(self, pairs, radius, dim):
+        """match_wide_batch's dicts -> (match_wide_batch_device's dicts, [(n_src_kps, n_tgt_kps)], descriptor row stride in
+        bytes, dim, keypoint row stride in bytes)"""
         fs = [dict(pr) if isinstance(pr, dict) else dict(zip(M.Context._WIDE_FIELDS, pr)) for pr in pairs]
         desc_strides, xyz_strides, width, out_pairs, counts = [], [], None, [], []
         for i, f in enumerate(fs):
@@ -361,29 +363,79 @@ class GpuBackend:
             raise M.B200MatchError("dim exceeds the row length")
         stride = self._one_stride(desc_strides, "descriptor sets") or width
         xyz_stride = self._one_stride(xyz_strides, "keypoint coordinates") or 4
+        return out_pairs, counts, stride * 4, dim, xyz_stride * 4
+
+    def _wide_batch(self, k, mode, pairs, radius, dim, cluster_k, distance_thr, thr_src, thr_tgt):
+        out_pairs, counts, stride, dim, xyz_stride = self._wide_args(pairs, radius, dim)
         ts, tt = self._thresholds(thr_src, thr_tgt, counts)
         cap = max(sum(ns for ns, _ in counts), 1)
         out = torch.empty((cap, 4), dtype=torch.int32, device=self.device)
         self.use_torch_stream()
         if radius is None:
-            offsets, avg = self.ctx.match_wide_batch_device(k, mode, out_pairs, stride * 4, dim, xyz_stride * 4, out.data_ptr(), cap,
+            offsets, avg = self.ctx.match_wide_batch_device(k, mode, out_pairs, stride, dim, xyz_stride, out.data_ptr(), cap,
                                                             cluster_k, distance_thr, self._ptr(ts), self._ptr(tt), self.precision,
                                                             self.cand_cap)
         else:
-            offsets, avg = self.ctx.match_wide_local_batch_device(k, mode, out_pairs, radius, stride * 4, dim, xyz_stride * 4,
+            offsets, avg = self.ctx.match_wide_local_batch_device(k, mode, out_pairs, radius, stride, dim, xyz_stride,
                                                                   out.data_ptr(), cap, cluster_k, distance_thr, self._ptr(ts),
                                                                   self._ptr(tt))
         return [(out[int(offsets[i]):int(offsets[i + 1])], float(avg[i])) for i in range(len(pairs))]
 
+    def plan_match_wide_batch(self, k, mode, pairs, dim=None, cluster_k=M.MATCHING_CLUSTER_K, distance_thr=M.FLT_MAX,
+                              thr_src=None, thr_tgt=None, cap=None):
+        """A BatchPlan of match_wide_batch over `pairs` (the same dicts).  Every tensor in them is bound in place; thr_src /
+        thr_tgt: None or one 1-D float32 tensor per pair of its keypoints, consecutive slices of one tensor per side.  cap:
+        records the plan writes (default the total source keypoints, enough for any data).  Outputs as plan_match_batch's,
+        plus plan.status int64 [1]: the bad-map key (-1, i.e. ~0, when clean; results() raises on any other)."""
+        return self._plan_wide(k, mode, pairs, None, dim, cluster_k, distance_thr, thr_src, thr_tgt, cap)
+
+    def plan_match_wide_local_batch(self, k, mode, pairs, match_search_radius, dim=None, cluster_k=M.MATCHING_CLUSTER_K,
+                                    distance_thr=M.FLT_MAX, thr_src=None, thr_tgt=None, cap=None):
+        """A BatchPlan of match_wide_local_batch over `pairs` (its dicts, moved keypoints included)."""
+        return self._plan_wide(k, mode, pairs, float(match_search_radius), dim, cluster_k, distance_thr, thr_src, thr_tgt, cap)
+
+    def _plan_wide(self, k, mode, pairs, radius, dim, cluster_k, distance_thr, thr_src, thr_tgt, cap):
+        out_pairs, counts, stride, dim, xyz_stride = self._wide_args(pairs, radius, dim)
+        if (thr_src is None) != (thr_tgt is None):
+            raise M.B200MatchError("give both threshold lists or neither")
+        keep = list(pairs)
+        thr = [0, 0]
+        if thr_src is not None:
+            for side, thrs in enumerate((thr_src, thr_tgt)):
+                if len(thrs) != len(counts):
+                    raise M.B200MatchError("one threshold array per pair and side")
+                thr[side], t = self._bound_thresholds(thrs, [c[side] for c in counts], "thr_src" if side == 0 else "thr_tgt")
+                keep.append(t)
+        cap = max(sum(ns for ns, _ in counts), 1) if cap is None else int(cap)
+        n = len(counts)
+        out = dict(records=torch.empty((cap, 4), dtype=torch.int32, device=self.device),
+                   offsets=torch.zeros((n + 1,), dtype=torch.int64, device=self.device),
+                   avg=torch.empty((n,), dtype=torch.float32, device=self.device),
+                   n_out=torch.zeros((1,), dtype=torch.int64, device=self.device),
+                   status=torch.full((1,), -1, dtype=torch.int64, device=self.device))
+        p = M.Context._params(k, mode, distance_thr=distance_thr, precision=self.precision, cand_cap=self.cand_cap)
+        arr, locs, _scales = M.Context._wide_device_pairs(out_pairs, radius is not None)
+        L, ptr = self.ctx._L, self._ptr
+        tail = (thr[0], thr[1], ptr(out["records"]), cap, ptr(out["offsets"]), ptr(out["avg"]), ptr(out["n_out"]), ptr(out["status"]))
+        if radius is None:
+            make = lambda h: L.b200m_plan_match_multiscale_batch(self.ctx._h, C.byref(p), arr, n, stride, dim, xyz_stride,
+                                                                 int(cluster_k), *tail, h)
+        else:
+            make = lambda h: L.b200m_plan_match_multiscale_local_batch(self.ctx._h, C.byref(p), arr, locs, n, stride, dim,
+                                                                       xyz_stride, int(cluster_k), radius, *tail, h)
+        return BatchPlan(self, [(0, ns, 0, nt) for ns, nt in counts], keep, out, make)
+
 
 class BatchPlan:
-    """A device batch call bound once (GpuBackend.plan_knn_batch / plan_match_batch).  run() enqueues it on torch's current
-    stream with no host round trip, allocation or copy, so it may be captured in torch.cuda.graph; a run or a replay
-    answers on what the bound input tensors hold at that time.  The outputs are the plan's static tensors (attributes)."""
+    """A device batch call bound once (GpuBackend.plan_knn_batch / plan_match_batch / plan_match_wide_batch /
+    plan_match_wide_local_batch).  run() enqueues it on torch's current stream with no host round trip, allocation or copy,
+    so it may be captured in torch.cuda.graph; a run or a replay answers on what the bound input tensors hold at that time.
+    The outputs are the plan's static tensors (attributes)."""
 
     def __init__(self, backend, ptrs, keep, outputs, make):
         self._L = backend.ctx._L
         self._h = None
+        self.status = None           # matcher-class plans: the bad-map key
         self.device = backend.device
         self.counts = [(q[1], q[3]) for q in ptrs]
         self._keep = keep            # the bound tensors stay alive as long as the plan
@@ -411,6 +463,10 @@ class BatchPlan:
                 out.append((self.idx[a:a + ns], self.dist[a:a + ns], self.cnt[a:a + ns]))
                 a += ns
             return out
+        if self.status is not None:
+            msg = self._L.b200m_plan_status_error(self._h, int(self.status.item()) & 0xFFFFFFFFFFFFFFFF)
+            if msg is not None:
+                raise M.B200MatchError(msg.decode())
         n = int(self.n_out.item())
         if n > self.records.shape[0]:
             raise M.B200MatchError("plan output capacity too small (%d correspondences)" % n)

@@ -93,7 +93,8 @@ EXPORTS = ["b200m_create", "b200m_destroy", "b200m_last_error", "b200m_set_strea
            "b200m_group_upload", "b200m_group_upload_sharded", "b200m_group_match", "b200m_group_knn", "b200m_knn_batch",
            "b200m_match_batch", "b200m_match_multiscale_batch", "b200m_match_multiscale_local_batch", "b200m_knn_batch_device",
            "b200m_match_batch_device", "b200m_match_multiscale_batch_device", "b200m_match_multiscale_local_batch_device",
-           "b200m_plan_knn_batch", "b200m_plan_match_batch", "b200m_plan_run", "b200m_plan_destroy", "b200m_plan_last_error"]
+           "b200m_plan_knn_batch", "b200m_plan_match_batch", "b200m_plan_run", "b200m_plan_destroy", "b200m_plan_last_error",
+           "b200m_plan_match_multiscale_batch", "b200m_plan_match_multiscale_local_batch", "b200m_plan_status_error"]
 
 _lib = None
 
@@ -175,6 +176,13 @@ def load_library():
     L.b200m_plan_knn_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Pair), C.c_int, sz, C.c_int, vp, vp, vp, C.POINTER(vp)]
     L.b200m_plan_match_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Pair), C.c_int, sz, C.c_int, vp, vp, vp, sz, vp, vp,
                                          vp, C.POINTER(vp)]
+    L.b200m_plan_match_multiscale_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_WidePair), C.c_int, sz, C.c_int, sz,
+                                                    C.c_int, vp, vp, vp, sz, vp, vp, vp, vp, C.POINTER(vp)]
+    L.b200m_plan_match_multiscale_local_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_WidePair), C.POINTER(_LocalPair),
+                                                          C.c_int, sz, C.c_int, sz, C.c_int, C.c_float, vp, vp, vp, sz, vp, vp,
+                                                          vp, vp, C.POINTER(vp)]
+    L.b200m_plan_status_error.argtypes = [vp, C.c_uint64]
+    L.b200m_plan_status_error.restype = C.c_char_p
     L.b200m_plan_run.argtypes = [vp, vp]
     L.b200m_plan_destroy.argtypes = [vp]
     L.b200m_plan_destroy.restype = None
@@ -520,8 +528,9 @@ class Context:
         return self._wide_batch_device(k, mode, pairs, float(match_search_radius), stride_bytes, dim, xyz_stride_bytes, out_ptr,
                                        cap, cluster_k, distance_thr, thr_src, thr_tgt, PREC_TC_F16, 0)
 
-    def _wide_batch_device(self, k, mode, pairs, radius, stride_bytes, dim, xyz_stride_bytes, out_ptr, cap, cluster_k,
-                           distance_thr, thr_src, thr_tgt, precision, cand_cap):
+    @staticmethod
+    def _wide_device_pairs(pairs, gated):
+        """match_wide_batch_device's dicts -> (b200m_wide_pair array, b200m_local_pair array, the scale arrays they point to)."""
         keep, arr = [], (_WidePair * max(len(pairs), 1))()
         locs = (_LocalPair * max(len(pairs), 1))()
         for i, f in enumerate(pairs):
@@ -532,8 +541,13 @@ class Context:
             arr[i] = _WidePair(C.cast(sc, C.c_void_p), len(f["scales"]), f.get("src_kps_xyz") or None, int(f["n_src_kps"]),
                                f.get("tgt_kps_xyz") or None, int(f["n_tgt_kps"]), float(f["iss_radius_src"]),
                                float(f["iss_radius_tgt"]))
-            if radius is not None:
+            if gated:
                 locs[i] = _LocalPair(f.get("src_kps_moved") or None, f.get("tgt_kps_moved") or None)
+        return arr, locs, keep
+
+    def _wide_batch_device(self, k, mode, pairs, radius, stride_bytes, dim, xyz_stride_bytes, out_ptr, cap, cluster_k,
+                           distance_thr, thr_src, thr_tgt, precision, cand_cap):
+        arr, locs, keep = self._wide_device_pairs(pairs, radius is not None)
         offsets = np.zeros(len(pairs) + 1, np.uint64)
         avg = np.empty(max(len(pairs), 1), np.float32)
         p = self._params(k, mode, distance_thr=distance_thr, precision=precision, cand_cap=cand_cap)

@@ -1,12 +1,17 @@
 """Compare per-kernel SASS (addresses, immediates and constant-bank offsets masked) and ptxas resource lines of two builds.
 
-    python tools/sass_compare.py BASE_DIR NEW_DIR candidates_tc pack exact local
+    python tools/sass_compare.py [--same-names] BASE_DIR NEW_DIR candidates_tc pack exact local
 
 Each directory holds <name>.sass (cuobjdump -sass <name>.o) and <name>.ptxas.txt (nvcc -Xptxas -v output) per translation
 unit.  Kernels are matched by demangled name; a trailing `, false>` template argument of the new tc_candidates_kernel (the
-K-streamed flag) and pack_operands_kernel<5> are mapped to the parent's names."""
+K-streamed flag) and pack_operands_kernel<5> are mapped to the parent's names, unless --same-names (both builds have the same
+template arguments: kernels are matched by their names as they are)."""
 import re, subprocess, sys, collections
-base, new = sys.argv[1], sys.argv[2]
+args = sys.argv[1:]
+same_names = "--same-names" in args
+if same_names:
+    args.remove("--same-names")
+base, new = args[0], args[1]
 def demangle(names):
     out = subprocess.run(["c++filt"], input="\n".join(names), capture_output=True, text=True).stdout.splitlines()
     return dict(zip(names, out))
@@ -37,11 +42,13 @@ def norm(n, new=False):
     n = n.replace("(anonymous namespace)::", "")
     n = re.sub(r"^void ", "", n)
     n = re.sub(r"\(.*", "", n)
+    if same_names:
+        return n
     if new:
         n = re.sub(r"tc_candidates_kernel<(.*), false>$", r"tc_candidates_kernel<\1>", n)
     n = n.replace("pack_operands_kernel<5>", "pack_operands_kernel")
     return n
-for obj in sys.argv[3:]:
+for obj in args[2:]:
     print("## %s.cu" % obj)
     b, n = sass("%s/%s.sass" % (base, obj)), sass("%s/%s.sass" % (new, obj))
     pb, pn = ptxas("%s/%s.ptxas.txt" % (base, obj)), ptxas("%s/%s.ptxas.txt" % (new, obj))
