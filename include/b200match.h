@@ -455,6 +455,31 @@ B200M_API int b200m_plan_match_batch(b200m_ctx *ctx, const b200m_params *p, cons
                                      size_t stride_bytes, int dim, const float *d_thr_src, const float *d_thr_tgt,
                                      b200m_corr *d_out, size_t cap, uint64_t *d_offsets, float *d_avg, uint64_t *d_n_out,
                                      b200m_plan **plan);
+/* Plans with live counts: the same plans for sets whose sizes change from run to run (a stream of scans with a different
+ * number of keypoints each).  Every n_src / n_tgt of the pairs is a CAPACITY: the most rows the plan will ever answer for
+ * that set (the pointers must hold that many rows).  d_rows [n_pairs][2] (device) holds the live (source rows, target
+ * rows) of every pair; every run reads it at its start, so the caller rewrites counts and rows in place between runs or
+ * graph replays.  Pair p's outputs are, byte for byte, what the device form gives on the live prefixes: the first n rows
+ * of each set and the first n thresholds of the pair's slice.  Rows past a live count are never read (they may hold
+ * anything).  Layouts:
+ *   thresholds   capacity layout: pair p's slice starts at the sum of the earlier pairs' capacities (one tensor per side);
+ *   records      dense, with d_offsets, as the match plan writes them;
+ *   k-lists      capacity layout: pair p's rows start at the sum of the earlier pairs' source capacities (d_idx / d_dist
+ *                [sum n_src][k], d_count [sum n_src]); rows from the live count up to the capacity hold the empty list
+ *                (index -1, distance 0, count 0), so a consumer sees fixed addresses.
+ * A count above its capacity makes its pair answer as empty (no records, empty lists, the average FLT_MAX of a pair without
+ * source rows; nothing past the capacity is read or written; the other pairs are unaffected), and d_status (device, one
+ * word) gets the key of the first such pair, in the layout of the matcher-class plans' status word: (pair << 16) | side
+ * with side 2 = source rows, 3 = target rows and scale 0; ~0 when every count fits.  Every run starts from a clean key.
+ * Creation runs once, synchronised, on the live counts d_rows holds then, and fails with the status text when a count is
+ * above its capacity. */
+B200M_API int b200m_plan_knn_batch_rows(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                                        size_t stride_bytes, int dim, int32_t *d_idx, float *d_dist, int32_t *d_count,
+                                        const uint32_t *d_rows, uint64_t *d_status, b200m_plan **plan);
+B200M_API int b200m_plan_match_batch_rows(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                                          size_t stride_bytes, int dim, const float *d_thr_src, const float *d_thr_tgt,
+                                          b200m_corr *d_out, size_t cap, uint64_t *d_offsets, float *d_avg,
+                                          uint64_t *d_n_out, const uint32_t *d_rows, uint64_t *d_status, b200m_plan **plan);
 /* Matcher-class plans: b200m_match_multiscale_batch_device's / b200m_match_multiscale_local_batch_device's arguments, with
  * the offsets and averages on the device and two more device words, d_n_out and d_status.  Creation copies the host arrays
  * (pairs, their scales, locals) and binds the device pointers inside them; every scale's tables are built once.  A run
@@ -478,12 +503,40 @@ B200M_API int b200m_plan_match_multiscale_local_batch(b200m_ctx *ctx, const b200
                                                       const float *d_thr_tgt, b200m_corr *d_out, size_t cap,
                                                       uint64_t *d_offsets, float *d_avg, uint64_t *d_n_out,
                                                       uint64_t *d_status, b200m_plan **plan);
+/* Matcher-class plans with live counts: the same plans for keypoint clouds whose sizes change from run to run.  Every
+ * n_src_kps / n_tgt_kps and every scale's n_src / n_tgt is a CAPACITY (the bound keypoints, maps, descriptors, moved
+ * keypoints and thresholds hold that many rows).  d_kps [n_pairs][2] (device) holds the live (source, target) keypoints of
+ * every pair and d_rows [sum of the pairs' n_scales][2] (device, pair-then-scale order) the live (source, target) rows of
+ * every scale; every run reads both at its start.  The number of pairs and each pair's number of scales stay as created.
+ * Pair p's records, offsets and average are byte for byte the device form's on the live prefixes: the first n keypoints,
+ * moved keypoints and thresholds, the first n rows of each scale's descriptors and index maps.  Rows past a live count are
+ * never read (out-of-range map entries there are not reported).  Thresholds use the capacity layout: pair p's slice starts
+ * at the sum of the earlier pairs' keypoint capacities.  A count above its capacity makes its pair answer as empty (no
+ * records, average FLT_MAX), and d_status gets the key of the first such count with side 2 = source, 3 = target and
+ * scale = the scale of a row count or 0xFFFF for a keypoint count; a bad map entry in the live rows keys as before, and
+ * the smaller key wins.  Creation fails with the status text when its own run finds either. */
+B200M_API int b200m_plan_match_multiscale_batch_rows(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs,
+                                                     int n_pairs, size_t stride_bytes, int dim, size_t xyz_stride_bytes,
+                                                     int cluster_k, const float *d_thr_src, const float *d_thr_tgt,
+                                                     b200m_corr *d_out, size_t cap, uint64_t *d_offsets, float *d_avg,
+                                                     uint64_t *d_n_out, uint64_t *d_status, const uint32_t *d_kps,
+                                                     const uint32_t *d_rows, b200m_plan **plan);
+B200M_API int b200m_plan_match_multiscale_local_batch_rows(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs,
+                                                           const b200m_local_pair *locals, int n_pairs, size_t stride_bytes,
+                                                           int dim, size_t xyz_stride_bytes, int cluster_k,
+                                                           float match_search_radius, const float *d_thr_src,
+                                                           const float *d_thr_tgt, b200m_corr *d_out, size_t cap,
+                                                           uint64_t *d_offsets, float *d_avg, uint64_t *d_n_out,
+                                                           uint64_t *d_status, const uint32_t *d_kps, const uint32_t *d_rows,
+                                                           b200m_plan **plan);
 B200M_API int b200m_plan_run(b200m_plan *plan, void *cuda_stream); /* enqueue only */
 B200M_API void b200m_plan_destroy(b200m_plan *plan);
 B200M_API const char *b200m_plan_last_error(const b200m_plan *plan); /* plan may be NULL: errors without a plan */
 /* The text of a status word: NULL for ~0, else "pair P, scale S: an index map entry of the source|target cloud is outside
- * its keypoint range" -- the device forms fail with this text after their name.  Valid until the next call with the same
- * plan (plan may be NULL). */
+ * its keypoint range" (side 0 / 1) -- the device forms fail with this text after their name -- or "pair P, scale S: the
+ * live source|target row count is above its capacity" (side 2 / 3, the plans with live counts) or, for scale 0xFFFF, "pair
+ * P: the live source|target keypoint count is above its capacity".  Valid until the next call
+ * with the same plan (plan may be NULL). */
 B200M_API const char *b200m_plan_status_error(const b200m_plan *plan, uint64_t status);
 
 B200M_API int b200m_version(void);

@@ -156,6 +156,8 @@ inline size_t pad_rows(size_t n) { return (n + B200M_TILE_N - 1) / B200M_TILE_N 
 inline size_t align16(size_t b) { return (b + 15) & ~(size_t) 15; }
 
 // batch.cu: what stage_batch leaves on the device.  Pair p's rows start at the sum of pad_rows() of the pairs before it.
+// A batch plan with live counts (plan.cu) rewrites sets, thr_sets, avg_segs and seg[].range in place on every run: they
+// live in a buffer of the plan's own context and are never shared with another layout.
 // pair_info[p] = {first source row, first target row, source rows, first row of the pair in the dense k-list output}
 struct BatchLayout {
     size_t n_rows[2] = {0, 0};   // padded rows per side
@@ -343,6 +345,9 @@ struct WideLayout {
     size_t n_gmap = 0, max_map_rows = 0, max_kps[2] = {0, 0};
     // the result area: record count, bad-map key (~0 = clean), per-pair counts and averages
     unsigned long long *n_out = nullptr, *bad = nullptr;
+    std::vector<int32_t> gmap_keys;   // dev: (side, scale, pair) of every map gather entry, in table order
+    const GatherSet *thr_sets = nullptr;   // plans with live counts: [2][n_pairs] gathers of the thresholds into the dense keypoint
+                                            // layout (else device thresholds are read in place)
     unsigned *counts = nullptr;
     float *avgs = nullptr;
 };
@@ -352,7 +357,8 @@ int wide_batch_enqueue(b200m_ctx *ctx, const WideCall &c, const WideLayout &W);
 int wide_batch_results(b200m_ctx *ctx, const WideCall &c, const WideLayout &W, b200m_corr *out, size_t cap, size_t *offsets,
                        float *avg);
 // The text of a bad-map key (flag_bad): "pair P, scale S: an index map entry of the source|target cloud is outside its
-// keypoint range"
+// keypoint range"; of an over-capacity key of a plan with live counts (side 2 / 3): "... the live source|target row count is
+// above its capacity"
 std::string map_status_text(unsigned long long key);
 
 // multi.cu

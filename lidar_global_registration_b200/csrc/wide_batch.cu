@@ -122,8 +122,13 @@ void wide_batch_release(b200m_ctx *ctx) {
 }
 
 std::string map_status_text(unsigned long long key) {
-    return "pair " + std::to_string((key >> 16) & 0xffffffffull) + ", scale " + std::to_string(key >> 48) +
-           ": an index map entry of the " + ((key & 1) ? "target" : "source") + " cloud is outside its keypoint range";
+    const std::string head = "pair " + std::to_string((key >> 16) & 0xffffffffull) + ", scale " + std::to_string(key >> 48);
+    if ((key & 0xffff) >= 2 && (key >> 48) == 0xffff)   // a batch plan's live keypoint count (plan.cu)
+        return "pair " + std::to_string((key >> 16) & 0xffffffffull) + ": the live " + ((key & 1) ? "target" : "source") +
+               " keypoint count is above its capacity";
+    if ((key & 0xffff) >= 2)   // a batch plan's live row count (plan.cu)
+        return head + ": the live " + ((key & 1) ? "target" : "source") + " row count is above its capacity";
+    return head + ": an index map entry of the " + ((key & 1) ? "target" : "source") + " cloud is outside its keypoint range";
 }
 
 // gated = false: b200m_match_multiscale_batch; true: the guessed form, whose kNN passes are gated by `radius`.
@@ -284,6 +289,7 @@ int wide_batch_tables(b200m_ctx *ctx, const WideCall &c, WideLayout *W, bool kee
                 if (dev) {   // filed on the device, after the table upload (a NULL map: identity)
                     if (n[side]) {
                         gmap[n_gmap++] = GatherSet{given, 1, (int) (W->o_map[side][s] / 4 + start[side]), (int) n[side], 0};
+                        W->gmap_keys.insert(W->gmap_keys.end(), {side, s, i});
                         max_map_rows = std::max(max_map_rows, n[side]);
                     }
                 } else {
@@ -477,7 +483,15 @@ int wide_batch_enqueue(b200m_ctx *ctx, const WideCall &c, const WideLayout &W) {
                                         ws->vri.as<int32_t>(), ws->vrd.as<float>(), ws->vrc.as<int32_t>()))
         return 1;
     const float *d_thr_s = nullptr, *d_thr_t = nullptr;
-    if (c.thr_src && NT && dev) {   // the device thresholds are the dense keypoint-table layout already
+    if (c.thr_src && NT && W.thr_sets) {   // a plan with live counts: capacity-layout thresholds gathered into the dense layout
+        for (int side = 0; side < 2; ++side) {
+            CK(ctx->ws_thr[side].reserve(sizeof(float) * (side ? NT : NS)));
+            CK(launch_gather_sets(W.thr_sets + (size_t) side * n_pairs, n_pairs, W.max_kps[side], 1, 1, ctx->ws_thr[side].p, st));
+            ctx->stats.launches += 1;
+        }
+        d_thr_s = ctx->ws_thr[0].as<float>();
+        d_thr_t = ctx->ws_thr[1].as<float>();
+    } else if (c.thr_src && NT && dev) {   // the device thresholds are the dense keypoint-table layout already
         d_thr_s = c.thr_src;
         d_thr_t = c.thr_tgt;
     } else if (c.thr_src && NT) {   // keypoint tables are dense: the concatenated thresholds are indexed by the global ids as they are

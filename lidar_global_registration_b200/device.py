@@ -242,9 +242,12 @@ class GpuBackend:
         return [(out[int(offsets[i]):int(offsets[i + 1])], float(avg[i])) for i in range(len(pairs))]
 
     # -- batch plans (b200m_plan_*): bound once, then enqueued without the host ----------------------------------------
-    def plan_knn_batch(self, k, pairs, dim):
+    def plan_knn_batch(self, k, pairs, dim, rows=None):
         """A BatchPlan of knn_batch over `pairs` (as knn_batch takes them).  The plan binds the tensors themselves: run()
-        answers on whatever they hold when it runs.  Outputs: plan.idx [sum n_src, k], plan.dist, plan.cnt [sum n_src]."""
+        answers on whatever they hold when it runs.  Outputs: plan.idx [sum n_src, k], plan.dist, plan.cnt [sum n_src].
+        rows: None, or an int32 CUDA tensor [n_pairs, 2] of live (source, target) rows that every run reads (b200m_plan_
+        knn_batch_rows): the pairs' tensors are then capacities, pair p's lists start at the sum of the earlier source
+        capacities, rows past the live count hold the empty list, and plan.status int64 [1] gets the over-capacity key."""
         ptrs, stride = self._set_pairs(pairs, dim)
         total = sum(p[1] for p in ptrs)
         out = dict(idx=torch.empty((total, k), dtype=torch.int32, device=self.device),
@@ -252,18 +255,30 @@ class GpuBackend:
                    cnt=torch.empty((total,), dtype=torch.int32, device=self.device))
         p = M.Context._params(k, M.MODE_KNN_ONLY, precision=self.precision, cand_cap=self.cand_cap)
         arr = M.Context._device_pairs(ptrs)
-        make = lambda h: self.ctx._L.b200m_plan_knn_batch(self.ctx._h, C.byref(p), arr, len(ptrs), stride, dim,
-                                                          self._ptr(out["idx"]), self._ptr(out["dist"]),
-                                                          self._ptr(out["cnt"]), h)
-        return BatchPlan(self, ptrs, list(pairs), out, make)
+        L, ptr = self.ctx._L, self._ptr
+        args = (self.ctx._h, C.byref(p), arr, len(ptrs), stride, dim, ptr(out["idx"]), ptr(out["dist"]), ptr(out["cnt"]))
+        if rows is None:
+            make = lambda h: L.b200m_plan_knn_batch(*args, h)
+        else:
+            self._live_rows(rows, len(ptrs), out)
+            make = lambda h: L.b200m_plan_knn_batch_rows(*args, ptr(rows), ptr(out["status"]), h)
+        return BatchPlan(self, ptrs, list(pairs), out, make, rows)
+
+    def _live_rows(self, rows, n_pairs, out):
+        """checks a live-count tensor and adds the status word to a plan's outputs"""
+        if not isinstance(rows, torch.Tensor) or rows.dtype != torch.int32 or rows.device != self.device or \
+                tuple(rows.shape) != (n_pairs, 2) or not rows.is_contiguous():
+            raise M.B200MatchError("rows: must be a contiguous int32 tensor [%d, 2] on %s" % (n_pairs, self.device))
+        out["status"] = torch.full((1,), -1, dtype=torch.int64, device=self.device)
 
     def plan_match_batch(self, k, mode, pairs, dim, cap=None, thr_src=None, thr_tgt=None, ratio_thr=M.MATCHING_RATIO_THRESHOLD,
-                         distance_thr=M.FLT_MAX):
+                         distance_thr=M.FLT_MAX, rows=None):
         """A BatchPlan of match_batch over `pairs`.  thr_src / thr_tgt: None or one 1-D float32 tensor per pair, bound in
         place, so they must be consecutive slices of one tensor per side in pair order (torch.split of it).  cap: records
         the plan writes (default sum n_src * (k if MUTUAL else 1), enough for any data).  Outputs: plan.records int32
         [cap, 4] (CORR_DTYPE layout), plan.offsets int64 [n_pairs + 1], plan.avg float32 [n_pairs], plan.n_out int64 [1]
-        (records found; above cap the records were truncated)."""
+        (records found; above cap the records were truncated).  rows: as plan_knn_batch's (b200m_plan_match_batch_rows);
+        the pairs' tensors and threshold slices are then capacities, and a run answers on their live prefixes."""
         ptrs, stride = self._set_pairs(pairs, dim)
         if (thr_src is None) != (thr_tgt is None):
             raise M.B200MatchError("give both threshold lists or neither")
@@ -283,10 +298,15 @@ class GpuBackend:
                    n_out=torch.zeros((1,), dtype=torch.int64, device=self.device))
         p = M.Context._params(k, mode, ratio_thr, distance_thr, self.precision, self.cand_cap)
         arr = M.Context._device_pairs(ptrs)
-        make = lambda h: self.ctx._L.b200m_plan_match_batch(self.ctx._h, C.byref(p), arr, len(ptrs), stride, dim, thr[0], thr[1],
-                                                            self._ptr(out["records"]), cap, self._ptr(out["offsets"]),
-                                                            self._ptr(out["avg"]), self._ptr(out["n_out"]), h)
-        return BatchPlan(self, ptrs, keep, out, make)
+        L, ptr = self.ctx._L, self._ptr
+        args = (self.ctx._h, C.byref(p), arr, len(ptrs), stride, dim, thr[0], thr[1], ptr(out["records"]), cap,
+                ptr(out["offsets"]), ptr(out["avg"]), ptr(out["n_out"]))
+        if rows is None:
+            make = lambda h: L.b200m_plan_match_batch(*args, h)
+        else:
+            self._live_rows(rows, len(ptrs), out)
+            make = lambda h: L.b200m_plan_match_batch_rows(*args, ptr(rows), ptr(out["status"]), h)
+        return BatchPlan(self, ptrs, keep, out, make, rows)
 
     def _bound_thresholds(self, thrs, counts, what):
         """per-pair threshold tensors that lie back to back in one tensor -> (device pointer of the first, what to keep)"""
@@ -382,19 +402,26 @@ class GpuBackend:
         return [(out[int(offsets[i]):int(offsets[i + 1])], float(avg[i])) for i in range(len(pairs))]
 
     def plan_match_wide_batch(self, k, mode, pairs, dim=None, cluster_k=M.MATCHING_CLUSTER_K, distance_thr=M.FLT_MAX,
-                              thr_src=None, thr_tgt=None, cap=None):
+                              thr_src=None, thr_tgt=None, cap=None, kps_rows=None, scale_rows=None):
         """A BatchPlan of match_wide_batch over `pairs` (the same dicts).  Every tensor in them is bound in place; thr_src /
         thr_tgt: None or one 1-D float32 tensor per pair of its keypoints, consecutive slices of one tensor per side.  cap:
         records the plan writes (default the total source keypoints, enough for any data).  Outputs as plan_match_batch's,
-        plus plan.status int64 [1]: the bad-map key (-1, i.e. ~0, when clean; results() raises on any other)."""
-        return self._plan_wide(k, mode, pairs, None, dim, cluster_k, distance_thr, thr_src, thr_tgt, cap)
+        plus plan.status int64 [1]: the bad-map key (-1, i.e. ~0, when clean; results() raises on any other).
+        kps_rows / scale_rows: None, or int32 CUDA tensors [n_pairs, 2] of live (source, target) keypoints and [sum of the
+        pairs' scales, 2] of live (source, target) rows per scale, pair-then-scale order, that every run reads
+        (b200m_plan_match_multiscale_batch_rows): every tensor in the dicts is then a capacity, and a count above its
+        capacity empties its pair and sets plan.status."""
+        return self._plan_wide(k, mode, pairs, None, dim, cluster_k, distance_thr, thr_src, thr_tgt, cap, kps_rows, scale_rows)
 
     def plan_match_wide_local_batch(self, k, mode, pairs, match_search_radius, dim=None, cluster_k=M.MATCHING_CLUSTER_K,
-                                    distance_thr=M.FLT_MAX, thr_src=None, thr_tgt=None, cap=None):
-        """A BatchPlan of match_wide_local_batch over `pairs` (its dicts, moved keypoints included)."""
-        return self._plan_wide(k, mode, pairs, float(match_search_radius), dim, cluster_k, distance_thr, thr_src, thr_tgt, cap)
+                                    distance_thr=M.FLT_MAX, thr_src=None, thr_tgt=None, cap=None, kps_rows=None, scale_rows=None):
+        """A BatchPlan of match_wide_local_batch over `pairs` (its dicts, moved keypoints included); kps_rows / scale_rows as
+        plan_match_wide_batch's (b200m_plan_match_multiscale_local_batch_rows)."""
+        return self._plan_wide(k, mode, pairs, float(match_search_radius), dim, cluster_k, distance_thr, thr_src, thr_tgt, cap,
+                               kps_rows, scale_rows)
 
-    def _plan_wide(self, k, mode, pairs, radius, dim, cluster_k, distance_thr, thr_src, thr_tgt, cap):
+    def _plan_wide(self, k, mode, pairs, radius, dim, cluster_k, distance_thr, thr_src, thr_tgt, cap, kps_rows=None,
+                   scale_rows=None):
         out_pairs, counts, stride, dim, xyz_stride = self._wide_args(pairs, radius, dim)
         if (thr_src is None) != (thr_tgt is None):
             raise M.B200MatchError("give both threshold lists or neither")
@@ -417,7 +444,23 @@ class GpuBackend:
         arr, locs, _scales = M.Context._wide_device_pairs(out_pairs, radius is not None)
         L, ptr = self.ctx._L, self._ptr
         tail = (thr[0], thr[1], ptr(out["records"]), cap, ptr(out["offsets"]), ptr(out["avg"]), ptr(out["n_out"]), ptr(out["status"]))
-        if radius is None:
+        if (kps_rows is None) != (scale_rows is None):
+            raise M.B200MatchError("give both kps_rows and scale_rows or neither")
+        if kps_rows is not None:
+            n_rows = sum(len(d["scales"]) for d in out_pairs)
+            for t, shape, what in ((kps_rows, (n, 2), "kps_rows"), (scale_rows, (n_rows, 2), "scale_rows")):
+                if not isinstance(t, torch.Tensor) or t.dtype != torch.int32 or t.device != self.device or \
+                        tuple(t.shape) != shape or not t.is_contiguous():
+                    raise M.B200MatchError("%s: must be a contiguous int32 tensor %s on %s" % (what, list(shape), self.device))
+            keep += [kps_rows, scale_rows]
+            live = (ptr(kps_rows), ptr(scale_rows))
+            if radius is None:
+                make = lambda h: L.b200m_plan_match_multiscale_batch_rows(self.ctx._h, C.byref(p), arr, n, stride, dim, xyz_stride,
+                                                                          int(cluster_k), *tail, *live, h)
+            else:
+                make = lambda h: L.b200m_plan_match_multiscale_local_batch_rows(self.ctx._h, C.byref(p), arr, locs, n, stride, dim,
+                                                                                xyz_stride, int(cluster_k), radius, *tail, *live, h)
+        elif radius is None:
             make = lambda h: L.b200m_plan_match_multiscale_batch(self.ctx._h, C.byref(p), arr, n, stride, dim, xyz_stride,
                                                                  int(cluster_k), *tail, h)
         else:
@@ -432,12 +475,14 @@ class BatchPlan:
     so it may be captured in torch.cuda.graph; a run or a replay answers on what the bound input tensors hold at that time.
     The outputs are the plan's static tensors (attributes)."""
 
-    def __init__(self, backend, ptrs, keep, outputs, make):
+    def __init__(self, backend, ptrs, keep, outputs, make, rows=None):
         self._L = backend.ctx._L
         self._h = None
-        self.status = None           # matcher-class plans: the bad-map key
+        self.status = None           # matcher-class plans: the bad-map key; plans with live counts: the over-capacity key
         self.device = backend.device
-        self.counts = [(q[1], q[3]) for q in ptrs]
+        self.counts = [(q[1], q[3]) for q in ptrs]   # with live counts: the capacities
+        self.rows = rows             # None, or the live counts [n_pairs, 2] every run reads
+        self._live = None if rows is None else torch.empty_like(rows)   # the counts the last run read, in stream order
         self._keep = keep            # the bound tensors stay alive as long as the plan
         self.kind = "match" if "records" in outputs else "knn"
         for name, t in outputs.items():
@@ -447,26 +492,32 @@ class BatchPlan:
         if make(C.byref(h)) != 0:
             raise M.B200MatchError(self._L.b200m_last_error(backend.ctx._h).decode())
         self._h = h
+        if self._live is not None:   # the counts the creation run read
+            self._live.copy_(self.rows)
 
     def run(self):
         """Enqueue the batch on torch's current stream (nothing is returned; the outputs are the plan's tensors)."""
+        if self._live is not None:   # the run reads the counts first, on this stream: results() splits by these
+            self._live.copy_(self.rows)
         if self._L.b200m_plan_run(self._h, torch.cuda.current_stream(self.device).cuda_stream) != 0:
             raise M.B200MatchError(self._L.b200m_plan_last_error(self._h).decode())
 
     def results(self):
         """Synchronise torch's current stream and split the outputs into per-pair views: knn -> [(idx, dist, cnt)], match
-        -> [(records int32 [n, 4], average)], as GpuBackend.knn_batch / match_batch return them."""
+        -> [(records int32 [n, 4], average)], as GpuBackend.knn_batch / match_batch return them (with live counts: for
+        the live rows the run read).  Raises with the status text when the status word is set."""
         torch.cuda.current_stream(self.device).synchronize()
-        out, a = [], 0
-        if self.kind == "knn":
-            for ns, _ in self.counts:
-                out.append((self.idx[a:a + ns], self.dist[a:a + ns], self.cnt[a:a + ns]))
-                a += ns
-            return out
         if self.status is not None:
             msg = self._L.b200m_plan_status_error(self._h, int(self.status.item()) & 0xFFFFFFFFFFFFFFFF)
             if msg is not None:
                 raise M.B200MatchError(msg.decode())
+        out, a = [], 0
+        if self.kind == "knn":
+            live = self.counts if self.rows is None else [tuple(r) for r in self._live.cpu().tolist()]
+            for (cap, _), (ns, _) in zip(self.counts, live):
+                out.append((self.idx[a:a + ns], self.dist[a:a + ns], self.cnt[a:a + ns]))
+                a += cap
+            return out
         n = int(self.n_out.item())
         if n > self.records.shape[0]:
             raise M.B200MatchError("plan output capacity too small (%d correspondences)" % n)

@@ -94,7 +94,9 @@ EXPORTS = ["b200m_create", "b200m_destroy", "b200m_last_error", "b200m_set_strea
            "b200m_match_batch", "b200m_match_multiscale_batch", "b200m_match_multiscale_local_batch", "b200m_knn_batch_device",
            "b200m_match_batch_device", "b200m_match_multiscale_batch_device", "b200m_match_multiscale_local_batch_device",
            "b200m_plan_knn_batch", "b200m_plan_match_batch", "b200m_plan_run", "b200m_plan_destroy", "b200m_plan_last_error",
-           "b200m_plan_match_multiscale_batch", "b200m_plan_match_multiscale_local_batch", "b200m_plan_status_error"]
+           "b200m_plan_match_multiscale_batch", "b200m_plan_match_multiscale_local_batch", "b200m_plan_status_error",
+           "b200m_plan_knn_batch_rows", "b200m_plan_match_batch_rows", "b200m_plan_match_multiscale_batch_rows",
+           "b200m_plan_match_multiscale_local_batch_rows"]
 
 _lib = None
 
@@ -176,11 +178,16 @@ def load_library():
     L.b200m_plan_knn_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Pair), C.c_int, sz, C.c_int, vp, vp, vp, C.POINTER(vp)]
     L.b200m_plan_match_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_Pair), C.c_int, sz, C.c_int, vp, vp, vp, sz, vp, vp,
                                          vp, C.POINTER(vp)]
+    L.b200m_plan_knn_batch_rows.argtypes = L.b200m_plan_knn_batch.argtypes[:-1] + [vp, vp, C.POINTER(vp)]
+    L.b200m_plan_match_batch_rows.argtypes = L.b200m_plan_match_batch.argtypes[:-1] + [vp, vp, C.POINTER(vp)]
     L.b200m_plan_match_multiscale_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_WidePair), C.c_int, sz, C.c_int, sz,
                                                     C.c_int, vp, vp, vp, sz, vp, vp, vp, vp, C.POINTER(vp)]
     L.b200m_plan_match_multiscale_local_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_WidePair), C.POINTER(_LocalPair),
                                                           C.c_int, sz, C.c_int, sz, C.c_int, C.c_float, vp, vp, vp, sz, vp, vp,
                                                           vp, vp, C.POINTER(vp)]
+    L.b200m_plan_match_multiscale_batch_rows.argtypes = L.b200m_plan_match_multiscale_batch.argtypes[:-1] + [vp, vp, C.POINTER(vp)]
+    L.b200m_plan_match_multiscale_local_batch_rows.argtypes = \
+        L.b200m_plan_match_multiscale_local_batch.argtypes[:-1] + [vp, vp, C.POINTER(vp)]
     L.b200m_plan_status_error.argtypes = [vp, C.c_uint64]
     L.b200m_plan_status_error.restype = C.c_char_p
     L.b200m_plan_run.argtypes = [vp, vp]
