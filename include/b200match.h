@@ -546,10 +546,20 @@ B200M_API int b200m_version(void);
  *   as_query=1 -> [n_pad][kp] rows (-2*x16, 1,1,1, 0..), else the train form (x16, |x16|^2 hi/mid/lo, 0..);
  *   norm16 (may be NULL) receives |x16|^2 per row [n_pad]; scale/kp/n_pad are returned through the pointers.
  * b200m_debug_tc_tile: raw tensor-core accumulators (|b16|^2 - 2 a16.b16) of query rows
- *   [q_row0, q_row0+128) x train rows [t_tile*256, +256) of `direction`, row-major [128][256]. */
+ *   [q_row0, q_row0+128) x train rows [t_tile*256, +256) of `direction`, row-major [128][256].  It launches the
+ *   candidate kernel (k = 1, dump mode), which overwrites the candidate lists: read those first.
+ * b200m_debug_candidate_lists: the candidate lists of the last candidate launch on the context, read-only.  n_lists,
+ *   cap, n_rows (the launch's query rows, in launch order) and kind are returned through the pointers; kind 0 = column
+ *   entries, 1 = column entries + accumulator values + per-list thresholds, 2 = chunk entries (first train row of a
+ *   32-row chunk, chunk minimum) + thresholds.  cnt [n_lists][n_rows] (entries appended; above cap = overflowed),
+ *   idx and val [n_lists][n_rows][cap] (entries past cnt are stale), thr [n_lists][n_rows] (each list's final
+ *   threshold); val and thr are not written for kind 0.  Any buffer may be NULL: call once with NULL buffers for the
+ *   sizes. */
 B200M_API int b200m_debug_operands(b200m_ctx *ctx, int side, int as_query, uint16_t *host_out, size_t out_halves,
                                    float *norm16, float *scale, int32_t *kp, int64_t *n_pad);
 B200M_API int b200m_debug_tc_tile(b200m_ctx *ctx, int direction, size_t q_row0, size_t t_tile, float *host_out);
+B200M_API int b200m_debug_candidate_lists(b200m_ctx *ctx, int32_t *n_lists, int32_t *cap, int64_t *n_rows, int32_t *kind,
+                                          int32_t *cnt, int32_t *idx, float *val, float *thr);
 
 #ifdef __cplusplus
 }

@@ -845,4 +845,24 @@ int b200m_debug_tc_tile(b200m_ctx *ctx, int direction, size_t q_row0, size_t t_t
     return 0;
 }
 
+int b200m_debug_candidate_lists(b200m_ctx *ctx, int32_t *n_lists, int32_t *cap, int64_t *n_rows, int32_t *kind, int32_t *cnt,
+                                int32_t *idx, float *val, float *thr) {
+    REQUIRE_CTX();
+    if (ctx->cand_kind < 0) return b200m_fail_msg(ctx, "debug_candidate_lists: no candidate launch on this context yet");
+    if (n_lists) *n_lists = ctx->cand_n_lists;
+    if (cap) *cap = ctx->cand_cap;
+    if (n_rows) *n_rows = (int64_t) ctx->cand_rows;
+    if (kind) *kind = ctx->cand_kind;
+    const size_t lists = (size_t) ctx->cand_n_lists * ctx->cand_rows, entries = lists * (size_t) ctx->cand_cap;
+    cudaStream_t st = ctx->stream;
+    if (cnt) CK(cudaMemcpyAsync(cnt, ctx->ws_cand_cnt.p, sizeof(int32_t) * lists, cudaMemcpyDeviceToHost, st));
+    if (idx) CK(cudaMemcpyAsync(idx, ctx->ws_cand_idx.p, sizeof(int32_t) * entries, cudaMemcpyDeviceToHost, st));
+    if (ctx->cand_kind != 0) {   // kind 0 lists carry no values and no thresholds: val / thr stay untouched
+        if (val) CK(cudaMemcpyAsync(val, ctx->ws_cand_val.p, sizeof(float) * entries, cudaMemcpyDeviceToHost, st));
+        if (thr) CK(cudaMemcpyAsync(thr, ctx->ws_cand_thr.p, sizeof(float) * lists, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaStreamSynchronize(st));
+    return 0;
+}
+
 }  // extern "C"

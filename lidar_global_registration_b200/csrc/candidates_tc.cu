@@ -1665,6 +1665,10 @@ int tc_candidates(b200m_ctx *ctx, int direction, size_t row_begin, size_t n_rows
     if (rc) return rc;
     ctx->stats.launches += 1;
     ctx->stats.candidate_launches += 1;
+    ctx->cand_n_lists = n_lists;
+    ctx->cand_cap = cap;
+    ctx->cand_kind = *has_values_out;
+    ctx->cand_rows = n_rows;
     *n_lists_out = n_lists;
     *cap_out = cap;
     return 0;

@@ -103,6 +103,10 @@ struct b200m_ctx {
     // the candidate kernel's DP form), so the kNN driver enqueues without a host round trip.  Only a plan's private
     // context sets it.
     bool device_prepare = false;
+    // shape of the last candidate launch (tc_candidates), for b200m_debug_candidate_lists: lists, capacity, query rows and
+    // kind (the launch's has_values; -1 = no launch yet)
+    int cand_n_lists = 0, cand_cap = 0, cand_kind = -1;
+    size_t cand_rows = 0;
     bool profiling = false;
     b200m_stats stats{};
     cudaEvent_t ev[2] = {nullptr, nullptr};

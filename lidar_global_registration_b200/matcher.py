@@ -84,7 +84,7 @@ class Stats(C.Structure):
 EXPORTS = ["b200m_create", "b200m_destroy", "b200m_last_error", "b200m_set_stream", "b200m_sync",
            "b200m_set_profiling", "b200m_get_stats", "b200m_reset_stats", "b200m_upload", "b200m_upload_device",
            "b200m_knn", "b200m_knn_device", "b200m_match", "b200m_filter_device", "b200m_merge_device",
-           "b200m_version", "b200m_debug_operands", "b200m_debug_tc_tile", "b200m_multiscale_begin",
+           "b200m_version", "b200m_debug_operands", "b200m_debug_tc_tile", "b200m_debug_candidate_lists", "b200m_multiscale_begin",
            "b200m_multiscale_add", "b200m_multiscale_vote", "b200m_multiscale_add_device", "b200m_multiscale_vote_device", "b200m_match_cluster",
            "b200m_cluster_filter_device", "b200m_knn3d_device", "b200m_knn_local", "b200m_knn_local_device", "b200m_mark_referenced_device", "b200m_knn_masked_device",
            "b200m_match_multiscale", "b200m_comm_unique_id", "b200m_comm_attach", "b200m_comm_rank", "b200m_shard_rows",
@@ -199,6 +199,8 @@ def load_library():
     L.b200m_debug_operands.argtypes = [vp, C.c_int, C.c_int, vp, sz, vp, C.POINTER(C.c_float), C.POINTER(i32),
                                        C.POINTER(i64)]
     L.b200m_debug_tc_tile.argtypes = [vp, C.c_int, sz, sz, vp]
+    L.b200m_debug_candidate_lists.argtypes = [vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i64), C.POINTER(i32), vp, vp, vp,
+                                              vp]
     _lib = L
     return L
 
@@ -819,6 +821,22 @@ class Context:
         out = np.empty((128, 256), np.float32)
         self._ck(self._L.b200m_debug_tc_tile(self._h, direction, q_row0, t_tile, out.ctypes.data))
         return out
+
+    def debug_candidate_lists(self):
+        """The last candidate launch's lists: dict kind, cap, cnt [n_lists][n_rows], idx [n_lists][n_rows][cap] and, for
+        kind 1 / 2, val [n_lists][n_rows][cap] and thr [n_lists][n_rows] (None for kind 0).  debug_tc_tile overwrites them."""
+        n_lists, cap, kind, n_rows = C.c_int32(0), C.c_int32(0), C.c_int32(0), C.c_int64(0)
+        self._ck(self._L.b200m_debug_candidate_lists(self._h, C.byref(n_lists), C.byref(cap), C.byref(n_rows), C.byref(kind),
+                                                     None, None, None, None))
+        shape = (n_lists.value, n_rows.value)
+        cnt = np.empty(shape, np.int32)
+        idx = np.empty(shape + (cap.value,), np.int32)
+        val = np.empty(shape + (cap.value,), np.float32) if kind.value else None
+        thr = np.empty(shape, np.float32) if kind.value else None
+        ptr = lambda a: None if a is None else a.ctypes.data
+        self._ck(self._L.b200m_debug_candidate_lists(self._h, C.byref(n_lists), C.byref(cap), C.byref(n_rows), C.byref(kind),
+                                                     ptr(cnt), ptr(idx), ptr(val), ptr(thr)))
+        return {"kind": kind.value, "cap": cap.value, "cnt": cnt, "idx": idx, "val": val, "thr": thr}
 
 
 def comm_unique_id():
