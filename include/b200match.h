@@ -399,6 +399,46 @@ B200M_API int b200m_match_multiscale_local_batch(b200m_ctx *ctx, const b200m_par
                                                  const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
                                                  size_t *offsets, float *avg);
 
+/* ---- batches on a group: the four host batch calls spread by pairs over the group's devices -------------------------------
+ * Each takes its single-context form's arguments with the group in place of the context (b200m_group_knn_batch ==
+ * b200m_knn_batch, b200m_group_match_batch == b200m_match_batch, b200m_group_match_multiscale_batch ==
+ * b200m_match_multiscale_batch, b200m_group_match_multiscale_local_batch == b200m_match_multiscale_local_batch).  Every
+ * output equals, byte for byte, what the single-context form returns on any one device of the group: the k-lists (rows
+ * back to back in pair order), the records, offsets (also filled when cap is too small) and averages, the return code and
+ * the error text (in b200m_group_last_error; a NULL group fails with the single form's NULL-context text), and after an
+ * error the offsets as the single form leaves them.  One exception: after an error the k-list arrays may already hold the
+ * rows of the ranges that succeeded, where the single form writes none.
+ * The pairs are split into at most b200m_group_size contiguous ranges by b200m_batch_partition over a cost estimate from the
+ * shapes (descriptor rows of every scale and direction times the 64-padded dim + 3; ClusterMatcher adds its 3-D
+ * neighbourhoods, quadratic in the keypoints).  Each device with a non-empty range runs the single-context form on it
+ * concurrently, staging its own pairs from the caller's memory; the pieces are concatenated in pair order.  No collective
+ * runs.  Errors: the checks of the pairs report the failing range with the lowest first pair, a bad index map the smallest
+ * (scale, pair, side) of all devices, pair numbers always those of the whole batch.  The size limits of the single forms
+ * (2^31-1 rows or keypoints per side) apply to each range.  Like the single forms, the calls REPLACE the descriptor sets of
+ * the group's contexts (upload again before b200m_group_match / _knn). */
+B200M_API int b200m_group_knn_batch(b200m_group *group, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                                    size_t stride_bytes, int dim, int32_t *idx, float *dist, int32_t *count);
+B200M_API int b200m_group_match_batch(b200m_group *group, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
+                                      size_t stride_bytes, int dim, const float *thr_src, const float *thr_tgt,
+                                      b200m_corr *out, size_t cap, size_t *offsets, float *avg);
+B200M_API int b200m_group_match_multiscale_batch(b200m_group *group, const b200m_params *p, const b200m_wide_pair *pairs,
+                                                 int n_pairs, size_t stride_bytes, int dim, size_t xyz_stride_bytes,
+                                                 int cluster_k, const float *thr_src, const float *thr_tgt, b200m_corr *out,
+                                                 size_t cap, size_t *offsets, float *avg);
+B200M_API int b200m_group_match_multiscale_local_batch(b200m_group *group, const b200m_params *p, const b200m_wide_pair *pairs,
+                                                       const b200m_local_pair *locals, int n_pairs, size_t stride_bytes,
+                                                       int dim, size_t xyz_stride_bytes, int cluster_k,
+                                                       float match_search_radius, const float *thr_src,
+                                                       const float *thr_tgt, b200m_corr *out, size_t cap, size_t *offsets,
+                                                       float *avg);
+/* The split the group batch calls use (pure host code): pairs [0, n_pairs) with costs cost[i] (finite, >= 0) into n_parts
+ * contiguous ranges, range i = [first[i], first[i + 1]) (first has n_parts + 1 entries, first[0] = 0, first[n_parts] =
+ * n_pairs, non-decreasing), such that the largest range cost is the least possible (an exact linear partition).  Ranges are
+ * cut from the first pair on, each as long as that bound allows while more pairs remain than parts after it (with fewer
+ * pairs than parts: one pair per range); unused parts are empty ranges at the end.  Returns non-zero for bad
+ * arguments (n_pairs < 0, n_parts < 1, a NaN, negative or infinite cost). */
+B200M_API int b200m_batch_partition(const double *cost, int n_pairs, int n_parts, int *first);
+
 /* ---- device-resident batch calls: the four batch calls on descriptors, maps, keypoints and records in HBM -------------
  * For a caller whose sets already live on the GPU (a GPU feature stage, a torch pipeline, sets reused across calls).
  * Each takes its host form's arguments: the arrays of b200m_pair / b200m_wide_pair / b200m_scale / b200m_local_pair and

@@ -661,7 +661,8 @@ protected:
 // registration, one scan against many submaps, an evaluation table.  All matchers must be of one class with the same
 // parameters (the guess aside: each matcher may have its own) and keypoint point stride; each pair's common scales are
 // built as match_impl builds them.  Either every matcher has a guess (b200m_match_multiscale_local_batch) or none has.
-// result[i] equals matchers[i]->match(), finalize included, and matchers[i]->getAverageDistance() is set.  One GPU only.
+// result[i] equals matchers[i]->match(), finalize included, and matchers[i]->getAverageDistance() is set.  With several
+// parameters.devices the pairs are spread over those GPUs (b200m_group_match_multiscale[_local]_batch; same results).
 inline bool sameParameters(const AlignmentParameters &a, const AlignmentParameters &b) {
     return a.use_bfmatcher == b.use_bfmatcher && a.bf_block_size == b.bf_block_size && a.ratio_k == b.ratio_k &&
            a.cluster_k == b.cluster_k && a.randomness == b.randomness && a.distance_thr == b.distance_thr &&
@@ -692,7 +693,6 @@ std::vector<CorrespondencesPtr> matchMany(const std::vector<std::shared_ptr<Feat
         const FeatureBasedMatcherImpl<FeatureT> &m = *matchers[i];
         if (m.mode() != mode || matchers[i]->getClassName() != matchers[0]->getClassName() || !sameParameters(m.parameters_, pa))
             throw std::runtime_error("matchMany: every matcher must be of one class with the same AlignmentParameters");
-        if (m.parameters_.devices.size() > 1) throw std::runtime_error("matchMany: one GPU only (parameters.devices has several)");
         if (m.parameters_.guess.has_value() != guessed)
             throw std::runtime_error("matchMany: give every matcher a guess or none (the guessed and unguessed kNN are different calls)");
         scales[i] = m.commonScales();
@@ -730,16 +730,27 @@ std::vector<CorrespondencesPtr> matchMany(const std::vector<std::shared_ptr<Feat
     Correspondences all(std::max<size_t>(n_src, 1));
     std::vector<size_t> offsets(n + 1);
     std::vector<float> avg(n);
-    Context &ctx = shared_context(pa.device);
-    if (guessed)
-        ctx.check(b200m_match_multiscale_local_batch(ctx.get(), &p, pairs.data(), locals.data(), (int) n, sizeof(FeatureT),
-                                                     feature_dim<FeatureT>(), stride, pa.cluster_k, pa.match_search_radius,
-                                                     thr ? thr_src.data() : nullptr, thr ? thr_tgt.data() : nullptr,
-                                                     reinterpret_cast<b200m_corr *>(all.data()), all.size(), offsets.data(), avg.data()));
-    else
-        ctx.check(b200m_match_multiscale_batch(ctx.get(), &p, pairs.data(), (int) n, sizeof(FeatureT), feature_dim<FeatureT>(), stride,
-                                               pa.cluster_k, thr ? thr_src.data() : nullptr, thr ? thr_tgt.data() : nullptr,
-                                               reinterpret_cast<b200m_corr *>(all.data()), all.size(), offsets.data(), avg.data()));
+    const float *ts = thr ? thr_src.data() : nullptr, *tt = thr ? thr_tgt.data() : nullptr;
+    b200m_corr *rec = reinterpret_cast<b200m_corr *>(all.data());
+    if (pa.devices.size() > 1) {
+        Group &g = shared_group(pa.devices);
+        if (guessed)
+            g.check(b200m_group_match_multiscale_local_batch(g.get(), &p, pairs.data(), locals.data(), (int) n, sizeof(FeatureT),
+                                                             feature_dim<FeatureT>(), stride, pa.cluster_k, pa.match_search_radius, ts, tt,
+                                                             rec, all.size(), offsets.data(), avg.data()));
+        else
+            g.check(b200m_group_match_multiscale_batch(g.get(), &p, pairs.data(), (int) n, sizeof(FeatureT), feature_dim<FeatureT>(),
+                                                       stride, pa.cluster_k, ts, tt, rec, all.size(), offsets.data(), avg.data()));
+    } else {
+        Context &ctx = shared_context(pa.device);
+        if (guessed)
+            ctx.check(b200m_match_multiscale_local_batch(ctx.get(), &p, pairs.data(), locals.data(), (int) n, sizeof(FeatureT),
+                                                         feature_dim<FeatureT>(), stride, pa.cluster_k, pa.match_search_radius, ts, tt,
+                                                         rec, all.size(), offsets.data(), avg.data()));
+        else
+            ctx.check(b200m_match_multiscale_batch(ctx.get(), &p, pairs.data(), (int) n, sizeof(FeatureT), feature_dim<FeatureT>(), stride,
+                                                   pa.cluster_k, ts, tt, rec, all.size(), offsets.data(), avg.data()));
+    }
     for (size_t i = 0; i < n; ++i) {
         matchers[i]->average_distance_ = avg[i];
         result.push_back(matchers[i]->finalize(std::make_shared<Correspondences>(all.begin() + offsets[i], all.begin() + offsets[i + 1])));

@@ -133,7 +133,8 @@ int stage_batch_tables(b200m_ctx *ctx, const char *fn, const b200m_params *p, co
         const size_t n[2] = {pairs[i].n_src, pairs[i].n_tgt};
         const float *base[2] = {pairs[i].src, pairs[i].tgt};
         for (int s = 0; s < 2; ++s) {
-            if (n[s] && !base[s]) return b200m_fail_msg(ctx, f + ": null descriptor pointer in pair " + std::to_string(i));
+            if (n[s] && !base[s])
+                return b200m_fail_msg(ctx, f + ": null descriptor pointer in pair " + std::to_string(i + L->pair_base));
             if (dev && n[s] && check_device_ptr(ctx, f + ": pair " + std::to_string(i) + ": " + (s ? "tgt" : "src"), base[s]))
                 return 1;
             start[s][i] = L->n_rows[s];
@@ -350,8 +351,9 @@ int match_batch_records(b200m_ctx *ctx, const b200m_params *p, const BatchLayout
 namespace {
 
 // dev: b200m_knn_batch_device (device descriptors, the k-lists are written to the caller's device arrays in place)
+// r: a range of a group call (multi.cu), or NULL
 int knn_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
-              size_t stride_bytes, int dim, int32_t *idx, float *dist, int32_t *count) {
+              size_t stride_bytes, int dim, int32_t *idx, float *dist, int32_t *count, BatchRange *r = nullptr) {
     REQUIRE_CTX();
     if (check_params(ctx, p)) return 1;
     const std::string f(fn);
@@ -359,7 +361,9 @@ int knn_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p, c
                 check_device_ptr(ctx, f + ": count", count)))
         return 1;
     BatchLayout L;
+    if (r) L.pair_base = r->pair_base;
     if (stage_batch(ctx, fn, p, pairs, n_pairs, stride_bytes, dim, &L, dev)) return 1;
+    if (r) r->validated = true;
     if (L.real_src == 0) return 0;
     if (!idx || !dist || !count) return b200m_fail_msg(ctx, f + ": null output pointer");
     // the pairs' real rows back to back, with pair-local train indices (a device call writes the caller's arrays directly,
@@ -382,7 +386,7 @@ int knn_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p, c
 // dev: b200m_match_batch_device (device descriptors and thresholds, records to the caller's device buffer)
 int match_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p, const b200m_pair *pairs, int n_pairs,
                 size_t stride_bytes, int dim, const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
-                size_t *offsets, float *avg) {
+                size_t *offsets, float *avg, BatchRange *r = nullptr) {
     REQUIRE_CTX();
     if (check_params(ctx, p)) return 1;
     const std::string f(fn);
@@ -397,7 +401,9 @@ int match_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p,
         return 1;
     for (int i = 0; i <= n_pairs; ++i) offsets[i] = 0;
     BatchLayout L;
+    if (r) L.pair_base = r->pair_base;
     if (stage_batch(ctx, fn, p, pairs, n_pairs, stride_bytes, dim, &L, dev, thr_src, thr_tgt)) return 1;
+    if (r) r->validated = true;
     if (L.real_src == 0) {
         if (avg)
             for (int i = 0; i < n_pairs; ++i) avg[i] = 3.402823466e+38F;   // FLT_MAX, reference include/matching.h:41
@@ -428,11 +434,23 @@ int match_batch(b200m_ctx *ctx, const char *fn, bool dev, const b200m_params *p,
 
 }  // namespace
 
+int knn_batch_host(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
+                   int32_t *idx, float *dist, int32_t *count, BatchRange *r) {
+    return knn_batch(ctx, "b200m_knn_batch", false, p, pairs, n_pairs, stride_bytes, dim, idx, dist, count, r);
+}
+
+int match_batch_host(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
+                     const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap, size_t *offsets, float *avg,
+                     BatchRange *r) {
+    return match_batch(ctx, "b200m_match_batch", false, p, pairs, n_pairs, stride_bytes, dim, thr_src, thr_tgt, out, cap, offsets,
+                       avg, r);
+}
+
 extern "C" {
 
 int b200m_knn_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
                     int32_t *idx, float *dist, int32_t *count) {
-    return knn_batch(ctx, "b200m_knn_batch", false, p, pairs, n_pairs, stride_bytes, dim, idx, dist, count);
+    return knn_batch_host(ctx, p, pairs, n_pairs, stride_bytes, dim, idx, dist, count, nullptr);
 }
 
 int b200m_knn_batch_device(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes,
@@ -442,8 +460,7 @@ int b200m_knn_batch_device(b200m_ctx *ctx, const b200m_params *p, const b200m_pa
 
 int b200m_match_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
                       const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap, size_t *offsets, float *avg) {
-    return match_batch(ctx, "b200m_match_batch", false, p, pairs, n_pairs, stride_bytes, dim, thr_src, thr_tgt, out, cap, offsets,
-                       avg);
+    return match_batch_host(ctx, p, pairs, n_pairs, stride_bytes, dim, thr_src, thr_tgt, out, cap, offsets, avg, nullptr);
 }
 
 int b200m_match_batch_device(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes,

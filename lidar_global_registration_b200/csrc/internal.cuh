@@ -178,6 +178,7 @@ struct BatchLayout {
     const struct GatherSet *thr_sets[2] = {nullptr, nullptr};   // device calls with thresholds: [n_pairs] per side
     const int32_t *seg_blk[2] = {nullptr, nullptr};   // device calls: per side block -> pair table of the segmented pack
     const SetRef *sets[2] = {nullptr, nullptr};       // device calls: per side [n_pairs] sets of the segmented pack
+    int pair_base = 0;   // set by the caller: the number error texts give pair 0 (a group form's range, multi.cu)
 };
 // Validates the pairs, packs both sides in the padded layout (replacing what b200m_upload put in the context) and uploads
 // the segment tables into ctx->ws_batch.  dev: every descriptor pointer is a device pointer of the context's device
@@ -202,6 +203,27 @@ int knn_batch_lists(b200m_ctx *ctx, const b200m_params *p, const BatchLayout &L,
 // by the gather tables), else host arrays.
 int match_batch_records(b200m_ctx *ctx, const b200m_params *p, const BatchLayout &L, const b200m_pair *pairs, int n_pairs,
                         bool dev, const float *thr_src, const float *thr_tgt, bool want_avg);
+
+// One range of pairs of a group batch call (multi.cu) run through a host batch form on one device.  In: pair_base, the
+// batch's number of the range's first pair, which every error text uses.  Out: validated, set once the form's checks of
+// every pair have passed (an error after it is a run-time one); bad_key, the bad-map key (flag_bad) with the batch's pair
+// number, ~0 when clean.
+struct BatchRange {
+    int pair_base = 0;
+    bool validated = false;
+    unsigned long long bad_key = ~0ull;
+};
+// The host batch forms with a range (r may be NULL: the plain b200m_knn_batch / b200m_match_batch /
+// b200m_match_multiscale(_local)_batch).
+int knn_batch_host(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
+                   int32_t *idx, float *dist, int32_t *count, BatchRange *r);
+int match_batch_host(b200m_ctx *ctx, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
+                     const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap, size_t *offsets, float *avg,
+                     BatchRange *r);
+int match_multiscale_batch_host(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs, bool gated,
+                                const b200m_local_pair *locals, int n_pairs, size_t stride_bytes, int dim, size_t xyz_stride_bytes, int cluster_k, float radius,
+                                const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap, size_t *offsets, float *avg,
+                                BatchRange *r);
 
 // Device batch calls: `rows` rows of `w` 4-byte words, src_stride words apart at `src`, go to rows dst_row.. of a
 // destination (dst_stride words apart).  src = null writes the identity (row r -> r, w = 1): a NULL index map.
@@ -335,6 +357,7 @@ struct WideCall {
     const float *thr_src = nullptr, *thr_tgt = nullptr;
     const b200m_corr *out = nullptr;             // dev: checked with the other pointers
     bool want_avg = false;
+    BatchRange *range = nullptr;                 // a group call's range (pair numbers of error texts, bad-map key), or NULL
 };
 struct WideLayout {
     int n_scales = 0;   // 0: no pair has source keypoints and a scale -- nothing is queued

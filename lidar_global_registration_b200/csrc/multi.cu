@@ -18,10 +18,13 @@
 // need no NCCL at all.
 #include <dlfcn.h>
 #include <nccl.h>
+#include <float.h>
 #include <string.h>
 
+#include <algorithm>
 #include <condition_variable>
 #include <functional>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -268,6 +271,7 @@ struct b200m_group {
     std::string err;
     // host-side gather of the per-rank record slices
     std::vector<unsigned long long> counts;
+    int ranges_per_device = 1;   // group batch calls (B200M_GROUP_RANGES)
 
     int run(std::function<int(int)> f) {
         {
@@ -309,6 +313,122 @@ struct b200m_group {
 };
 
 static thread_local std::string g_group_err;
+
+// ---- group batch calls: a batch's pairs split into contiguous ranges, one host batch form per device -------------------
+namespace {
+
+// Estimated cost of one kNN pass of nq x nt descriptor rows: the tensor-core pass's K extent is dim + 3 norm columns,
+// padded to 64.  Shapes only; a guessed (gated) pass sweeps at most this much.
+double desc_cost(size_t nq, size_t nt, int dim) {
+    const int d = std::min(std::max(dim, 1), B200M_MAX_DIM);
+    return (double) nq * (double) nt * (double) ((d + 3 + 63) / 64 * 64);
+}
+
+// ClusterMatcher's 3-D neighbourhoods (knn3d, brute force inside each pair) cost kC3d * (n_src_kps^2 + n_tgt_kps^2) in
+// desc_cost units.  Measured on one B200 with the FPFH-33 20k x 20k one-scale ClusterMatcher batch against the same
+// LeftToRight batch (tools/bench_group_batch.py, DESIGN.md section 3.19).
+constexpr double kC3d = 211.0;
+
+double wide_cost(const b200m_params *p, const b200m_wide_pair &w, int dim) {
+    if (!w.n_src_kps || w.n_scales < 1 || w.n_scales > 32 || !w.scales) return 0.0;   // no scale takes part
+    double c = 0.0;
+    for (int s = 0; s < w.n_scales; ++s) c += desc_cost(w.scales[s].n_src, w.scales[s].n_tgt, dim);
+    if (p->mode != B200M_MODE_ONE_SIDED) c *= 2.0;   // the reverse pass
+    if (p->mode == B200M_MODE_CLUSTER) c += kC3d * ((double) w.n_src_kps * (double) w.n_src_kps + (double) w.n_tgt_kps * (double) w.n_tgt_kps);
+    return c;
+}
+
+// Runs f(device, range index, first pair, end pair, range) on every non-empty range of the cost partition: ranges i, i + W,
+// i + 2W, ... on device i, the devices concurrently.  W * g->ranges_per_device ranges (B200M_GROUP_RANGES, a diagnostic
+// switch: several ranges per device exercise the split on a box with one GPU).  whole: the arguments cannot be split (no
+// pairs, or params the single form rejects before it reads a pair): device 0 runs the whole call as given, f(0, 0, 0,
+// n_pairs).  On failure g->err is the text the single form gives on the whole batch: the error of the lowest range that
+// failed its checks; else the smallest bad-map key; else the lowest range's error.
+int run_ranges(b200m_group *g, int n_pairs, bool whole, const std::vector<double> &cost,
+               const std::function<int(int, int, int, int, BatchRange *)> &f, std::vector<int> *first) {
+    const int W = (int) g->ctx.size(), P = W * g->ranges_per_device;
+    first->assign((size_t) P + 1, whole ? n_pairs : 0);
+    (*first)[0] = 0;
+    if (!whole && b200m_batch_partition(cost.data(), n_pairs, P, first->data())) {
+        g->err = "group batch: bad cost estimate";
+        return 1;
+    }
+    std::vector<BatchRange> r((size_t) P);
+    std::vector<int> rc((size_t) P, 0);
+    std::vector<std::string> err((size_t) P);   // taken at once: a later range on the device overwrites the context's text
+    g->run([&](int i) {
+        for (int j = i; j < P; j += W) {
+            const int p0 = (*first)[(size_t) j], p1 = (*first)[(size_t) j + 1];
+            if (whole ? j != 0 : p0 == p1) continue;
+            r[(size_t) j].pair_base = p0;
+            rc[(size_t) j] = f(i, j, p0, p1, &r[(size_t) j]);
+            if (rc[(size_t) j]) err[(size_t) j] = g->ctx[(size_t) i]->err;
+        }
+        return 0;
+    });
+    int pick = -1;
+    for (int j = 0; j < P && pick < 0; ++j)
+        if (rc[(size_t) j] && !r[(size_t) j].validated) pick = j;
+    unsigned long long key = ~0ull;
+    for (int j = 0; j < P && pick < 0; ++j)
+        if (rc[(size_t) j] && r[(size_t) j].bad_key < key) key = r[(size_t) j].bad_key;
+    for (int j = 0; j < P && pick < 0; ++j)
+        if (rc[(size_t) j] && (key == ~0ull || r[(size_t) j].bad_key == key)) pick = j;
+    if (pick < 0) return 0;
+    g->err = err[(size_t) pick];
+    return 1;
+}
+
+// The host staging of one range's records, offsets and averages, and the merge into the caller's arrays in pair order.
+struct RangeOutputs {
+    std::vector<std::unique_ptr<b200m_corr[]>> rec;   // not zero-filled: the records found are written, nothing else is read
+    std::vector<size_t> cap;
+    std::vector<std::vector<size_t>> off;
+    std::vector<std::vector<float>> avg;
+    explicit RangeOutputs(size_t P) : rec(P), cap(P, 0), off(P), avg(P) {}
+    void size(int j, int n, size_t max_records) {
+        cap[(size_t) j] = std::max<size_t>(max_records, 1);
+        rec[(size_t) j].reset(new b200m_corr[cap[(size_t) j]]);
+        off[(size_t) j].assign((size_t) n + 1, ~(size_t) 0);   // the single form zeroes them once its arguments pass
+        avg[(size_t) j].resize((size_t) std::max(n, 1));
+    }
+    // after an error: the caller's offsets as the single form leaves them -- zeroed when its argument checks had passed
+    // (every range runs the same ones), untouched otherwise
+    void failed(size_t *offsets, int n_pairs) {
+        for (const std::vector<size_t> &o : off)
+            if (!o.empty() && o[0] == 0) {
+                for (int j = 0; j <= n_pairs; ++j) offsets[j] = 0;
+                return;
+            }
+    }
+    // offsets concatenated and rebased, averages copied, then the capacity check on the total (offsets and averages are
+    // written also when it fails, as the single forms write them) and the records
+    int merge(b200m_group *g, const char *name, const std::vector<int> &first, b200m_corr *out, size_t cap, size_t *offsets, float *avg_out) {
+        const int P = (int) first.size() - 1;
+        offsets[0] = 0;
+        for (int r = 0; r < P; ++r)
+            for (int j = first[(size_t) r]; j < first[(size_t) r + 1]; ++j) {
+                offsets[j + 1] = offsets[first[(size_t) r]] + off[(size_t) r][(size_t) (j - first[(size_t) r] + 1)];
+                if (avg_out) avg_out[j] = avg[(size_t) r][(size_t) (j - first[(size_t) r])];
+            }
+        const size_t total = offsets[first[(size_t) P]];
+        if (total > cap) {
+            g->err = std::string(name) + ": output capacity too small (" + std::to_string(total) + " correspondences)";
+            return 1;
+        }
+        if (total && !out) {
+            g->err = std::string(name) + ": null output buffer";
+            return 1;
+        }
+        for (int r = 0; r < P; ++r) {
+            const size_t o = offsets[first[(size_t) r]], n = offsets[first[(size_t) r + 1]] - o;
+            if (n) memcpy(out + o, rec[(size_t) r].get(), sizeof(b200m_corr) * n);
+        }
+        return 0;
+    }
+};
+
+}  // namespace
 
 extern "C" {
 
@@ -470,6 +590,7 @@ int b200m_create_multi(b200m_group **out, const int *device_ids, int n) {
         delete g;
         return 1;
     }
+    if (const char *e = getenv("B200M_GROUP_RANGES")) g->ranges_per_device = std::min(std::max(atoi(e), 1), 64);
     g->rc.assign((size_t) n, 0);
     g->counts.assign((size_t) n, 0);
     for (int i = 0; i < n; ++i) g->workers.emplace_back([g, i] { g->worker(i); });
@@ -577,6 +698,163 @@ int b200m_group_knn(b200m_group *g, const b200m_params *p, int32_t *idx, float *
         if (hi == lo) return 0;
         return b200m_knn(g->ctx[(size_t) i], p, 0, lo, hi, idx + lo * k, dist + lo * k, count + lo);
     });
+}
+
+int b200m_batch_partition(const double *cost, int n_pairs, int n_parts, int *first) {
+    if (n_pairs < 0 || n_parts < 1 || !first || (n_pairs && !cost)) return 1;
+    std::vector<double> pre((size_t) n_pairs + 1, 0.0);
+    for (int i = 0; i < n_pairs; ++i) {
+        if (!(cost[i] >= 0.0) || cost[i] > DBL_MAX) return 1;   // NaN, negative or infinite
+        pre[(size_t) i + 1] = pre[(size_t) i] + cost[i];
+    }
+    // A range [a, b) costs pre[b] - pre[a], which grows as the range grows, so the greedy cut (each range as long as the
+    // bound allows) needs the fewest ranges for a bound, and the least feasible bound is the optimum.  The bound is searched
+    // over the bit patterns of the non-negative doubles, which order as the values do: the result is exactly one of the
+    // range costs.
+    // A range also stops growing once no more pairs are left than parts after it, so that every part gets a pair when there
+    // are enough (the rest of the pairs then go one per part, which any feasible bound allows).
+    auto cut = [&](double bound, int *f) {   // ranges the greedy cut needs (n_parts + 1: infeasible)
+        int parts = 0;
+        for (int a = 0; a < n_pairs;) {
+            int b = a;
+            while (b < n_pairs && pre[(size_t) b + 1] - pre[(size_t) a] <= bound && (b == a || n_pairs - b > n_parts - parts - 1)) ++b;
+            if (b == a || parts == n_parts) return n_parts + 1;
+            if (f) f[parts] = a;
+            ++parts;
+            a = b;
+        }
+        return parts;
+    };
+    const double all = pre[(size_t) n_pairs];
+    if (all > DBL_MAX) return 1;
+    uint64_t lo = 0, hi;
+    memcpy(&hi, &all, sizeof(hi));
+    while (lo < hi) {
+        const uint64_t mid = lo + (hi - lo) / 2;
+        double bound;
+        memcpy(&bound, &mid, sizeof(bound));
+        if (cut(bound, nullptr) <= n_parts) hi = mid; else lo = mid + 1;
+    }
+    double bound;
+    memcpy(&bound, &lo, sizeof(bound));
+    const int used = cut(bound, first);
+    for (int i = used; i <= n_parts; ++i) first[i] = n_pairs;   // unused parts: empty ranges at the end
+    return 0;
+}
+
+int b200m_group_knn_batch(b200m_group *g, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
+                          int32_t *idx, float *dist, int32_t *count) {
+    if (!g) {
+        knn_batch_host(nullptr, p, pairs, n_pairs, stride_bytes, dim, idx, dist, count, nullptr);
+        g_group_err = b200m_last_error(nullptr);
+        return 1;
+    }
+    const bool whole = !p || !pairs || n_pairs <= 0 || p->k < 1 || p->k > B200M_MAX_K;
+    std::vector<double> cost(whole ? 0 : (size_t) n_pairs);
+    std::vector<size_t> rows_before(whole ? 1 : (size_t) n_pairs + 1, 0);
+    for (size_t i = 0; i < cost.size(); ++i) {
+        cost[i] = desc_cost(pairs[i].n_src, pairs[i].n_tgt, dim);
+        rows_before[i + 1] = rows_before[i] + pairs[i].n_src;
+    }
+    std::vector<int> first;
+    return run_ranges(g, n_pairs, whole, cost, [&](int i, int, int p0, int p1, BatchRange *r) {
+        if (whole) return knn_batch_host(g->ctx[0], p, pairs, n_pairs, stride_bytes, dim, idx, dist, count, r);
+        // the k-lists go straight to the caller's arrays at the range's first row
+        const size_t o = rows_before[(size_t) p0], k = (size_t) p->k;
+        return knn_batch_host(g->ctx[(size_t) i], p, pairs + p0, p1 - p0, stride_bytes, dim, idx ? idx + o * k : nullptr,
+                              dist ? dist + o * k : nullptr, count ? count + o : nullptr, r);
+    }, &first);
+}
+
+int b200m_group_match_batch(b200m_group *g, const b200m_params *p, const b200m_pair *pairs, int n_pairs, size_t stride_bytes, int dim,
+                            const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap, size_t *offsets, float *avg) {
+    if (!g) {
+        match_batch_host(nullptr, p, pairs, n_pairs, stride_bytes, dim, thr_src, thr_tgt, out, cap, offsets, avg, nullptr);
+        g_group_err = b200m_last_error(nullptr);
+        return 1;
+    }
+    const bool whole = !p || !pairs || n_pairs <= 0 || p->k < 1 || p->k > B200M_MAX_K;
+    const bool mutual = p && (p->mode == B200M_MODE_MUTUAL || p->mode == B200M_MODE_RATIO_MUTUAL);
+    std::vector<double> cost(whole ? 0 : (size_t) n_pairs);
+    std::vector<size_t> before[2] = {std::vector<size_t>(cost.size() + 1, 0), std::vector<size_t>(cost.size() + 1, 0)};
+    for (size_t i = 0; i < cost.size(); ++i) {
+        cost[i] = desc_cost(pairs[i].n_src, pairs[i].n_tgt, dim) * (mutual ? 2.0 : 1.0);
+        before[0][i + 1] = before[0][i] + pairs[i].n_src;
+        before[1][i + 1] = before[1][i] + pairs[i].n_tgt;
+    }
+    RangeOutputs ro(g->ctx.size() * (size_t) g->ranges_per_device);
+    std::vector<int> first;
+    if (run_ranges(g, n_pairs, whole, cost, [&](int i, int j, int p0, int p1, BatchRange *r) {
+            if (whole)
+                return match_batch_host(g->ctx[0], p, pairs, n_pairs, stride_bytes, dim, thr_src, thr_tgt, out, cap, offsets, avg, r);
+            const size_t kk = p->mode == B200M_MODE_MUTUAL ? (size_t) p->k : 1;
+            ro.size(j, p1 - p0, (before[0][(size_t) p1] - before[0][(size_t) p0]) * kk);
+            return match_batch_host(g->ctx[(size_t) i], p, pairs + p0, p1 - p0, stride_bytes, dim,
+                                    thr_src ? thr_src + before[0][(size_t) p0] : nullptr,
+                                    thr_tgt ? thr_tgt + before[1][(size_t) p0] : nullptr, ro.rec[(size_t) j].get(),
+                                    ro.cap[(size_t) j], offsets ? ro.off[(size_t) j].data() : nullptr,
+                                    avg ? ro.avg[(size_t) j].data() : nullptr, r);
+        }, &first)) {
+        if (!whole && offsets) ro.failed(offsets, n_pairs);
+        return 1;
+    }
+    return whole ? 0 : ro.merge(g, "b200m_match_batch", first, out, cap, offsets, avg);
+}
+
+namespace {
+
+int group_wide_batch(b200m_group *g, const b200m_params *p, const b200m_wide_pair *pairs, bool gated, const b200m_local_pair *locals,
+                     int n_pairs, size_t stride_bytes, int dim, size_t xyz_stride_bytes, int cluster_k, float radius,
+                     const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap, size_t *offsets, float *avg) {
+    if (!g) {
+        match_multiscale_batch_host(nullptr, p, pairs, gated, locals, n_pairs, stride_bytes, dim, xyz_stride_bytes, cluster_k, radius,
+                                    thr_src, thr_tgt, out, cap, offsets, avg, nullptr);
+        g_group_err = b200m_last_error(nullptr);
+        return 1;
+    }
+    const bool whole = !p || !pairs || (gated && !locals) || n_pairs <= 0 || p->k < 1 || p->k > B200M_MAX_K;
+    std::vector<double> cost(whole ? 0 : (size_t) n_pairs);
+    std::vector<size_t> before[2] = {std::vector<size_t>(cost.size() + 1, 0), std::vector<size_t>(cost.size() + 1, 0)};
+    for (size_t i = 0; i < cost.size(); ++i) {
+        cost[i] = wide_cost(p, pairs[i], dim);
+        before[0][i + 1] = before[0][i] + pairs[i].n_src_kps;
+        before[1][i + 1] = before[1][i] + pairs[i].n_tgt_kps;
+    }
+    RangeOutputs ro(g->ctx.size() * (size_t) g->ranges_per_device);
+    std::vector<int> first;
+    if (run_ranges(g, n_pairs, whole, cost, [&](int i, int j, int p0, int p1, BatchRange *r) {
+            if (whole)
+                return match_multiscale_batch_host(g->ctx[0], p, pairs, gated, locals, n_pairs, stride_bytes, dim, xyz_stride_bytes,
+                                                   cluster_k, radius, thr_src, thr_tgt, out, cap, offsets, avg, r);
+            ro.size(j, p1 - p0, before[0][(size_t) p1] - before[0][(size_t) p0]);
+            return match_multiscale_batch_host(g->ctx[(size_t) i], p, pairs + p0, gated, gated ? locals + p0 : nullptr, p1 - p0,
+                                               stride_bytes, dim, xyz_stride_bytes, cluster_k, radius,
+                                               thr_src ? thr_src + before[0][(size_t) p0] : nullptr,
+                                               thr_tgt ? thr_tgt + before[1][(size_t) p0] : nullptr, ro.rec[(size_t) j].get(),
+                                               ro.cap[(size_t) j], offsets ? ro.off[(size_t) j].data() : nullptr,
+                                               avg ? ro.avg[(size_t) j].data() : nullptr, r);
+        }, &first)) {
+        if (!whole && offsets) ro.failed(offsets, n_pairs);
+        return 1;
+    }
+    return whole ? 0 : ro.merge(g, gated ? "b200m_match_multiscale_local_batch" : "b200m_match_multiscale_batch", first, out, cap, offsets, avg);
+}
+
+}  // namespace
+
+int b200m_group_match_multiscale_batch(b200m_group *g, const b200m_params *p, const b200m_wide_pair *pairs, int n_pairs,
+                                       size_t stride_bytes, int dim, size_t xyz_stride_bytes, int cluster_k, const float *thr_src,
+                                       const float *thr_tgt, b200m_corr *out, size_t cap, size_t *offsets, float *avg) {
+    return group_wide_batch(g, p, pairs, false, nullptr, n_pairs, stride_bytes, dim, xyz_stride_bytes, cluster_k, 0.f, thr_src, thr_tgt,
+                            out, cap, offsets, avg);
+}
+
+int b200m_group_match_multiscale_local_batch(b200m_group *g, const b200m_params *p, const b200m_wide_pair *pairs,
+                                             const b200m_local_pair *locals, int n_pairs, size_t stride_bytes, int dim,
+                                             size_t xyz_stride_bytes, int cluster_k, float match_search_radius, const float *thr_src,
+                                             const float *thr_tgt, b200m_corr *out, size_t cap, size_t *offsets, float *avg) {
+    return group_wide_batch(g, p, pairs, true, locals, n_pairs, stride_bytes, dim, xyz_stride_bytes, cluster_k, match_search_radius,
+                            thr_src, thr_tgt, out, cap, offsets, avg);
 }
 
 }  // extern "C"

@@ -143,6 +143,7 @@ int wide_batch_tables(b200m_ctx *ctx, const WideCall &c, WideLayout *W, bool kee
     const b200m_local_pair *locals = c.locals;
     const int n_pairs = c.n_pairs;
     const bool dev = c.dev, gated = c.gated;
+    const int base = c.range ? c.range->pair_base : 0;
     if (n_pairs < 0) return b200m_fail_msg(ctx, fn + "n_pairs < 0");
     if (n_pairs > 0 && !pairs) return b200m_fail_msg(ctx, fn + "null pairs");
     if (gated && n_pairs > 0 && !locals) return b200m_fail_msg(ctx, fn + "null local pairs");
@@ -165,7 +166,7 @@ int wide_batch_tables(b200m_ctx *ctx, const WideCall &c, WideLayout *W, bool kee
     int n_scales = 0;
     for (int i = 0; i < n_pairs; ++i) {
         const b200m_wide_pair &w = pairs[i];
-        const std::string pi = fn + "pair " + std::to_string(i) + ": ";
+        const std::string pi = fn + "pair " + std::to_string(i + base) + ": ";
         if (w.n_scales < 0 || w.n_scales > 32) return b200m_fail_msg(ctx, pi + "n_scales must be in [0, 32]");
         if (w.n_scales && !w.scales) return b200m_fail_msg(ctx, pi + "null scales");
         if (w.n_scales * k > 128) return b200m_fail_msg(ctx, pi + "n_scales * k > 128");
@@ -545,7 +546,13 @@ int wide_batch_results(b200m_ctx *ctx, const WideCall &c, const WideLayout &W, b
     unsigned long long n, bad;
     memcpy(&n, res.data(), sizeof(n));
     memcpy(&bad, res.data() + 8, sizeof(bad));
-    if (bad != ~0ull) return b200m_fail_msg(ctx, fn + map_status_text(bad));
+    if (bad != ~0ull) {
+        if (c.range) {   // the key with the group call's pair number: (scale, pair, side) order is kept
+            bad += (unsigned long long) c.range->pair_base << 16;
+            c.range->bad_key = bad;
+        }
+        return b200m_fail_msg(ctx, fn + map_status_text(bad));
+    }
     const unsigned *cnt = reinterpret_cast<const unsigned *>(res.data() + 16);
     for (int i = 0; i < n_pairs; ++i) offsets[i + 1] = offsets[i] + cnt[i];
     if (avg) memcpy(avg, res.data() + W.o_avgs, sizeof(float) * n_pairs);
@@ -564,10 +571,11 @@ int wide_batch_results(b200m_ctx *ctx, const WideCall &c, const WideLayout &W, b
 
 namespace {
 
+// r: a range of a group call (multi.cu), or NULL
 int match_multiscale_batch(b200m_ctx *ctx, const char *name, bool dev, const b200m_params *p, const b200m_wide_pair *pairs,
                            bool gated, const b200m_local_pair *locals, int n_pairs, size_t stride_bytes, int dim,
                            size_t xyz_stride_bytes, int cluster_k, float radius, const float *thr_src, const float *thr_tgt,
-                           b200m_corr *out, size_t cap, size_t *offsets, float *avg) {
+                           b200m_corr *out, size_t cap, size_t *offsets, float *avg, BatchRange *r = nullptr) {
     if (!ctx) return b200m_fail_msg(nullptr, "null context");
     CK(cudaSetDevice(ctx->device));
     if (!p || !offsets) return b200m_fail_msg(ctx, std::string(name) + ": null params / offsets");
@@ -589,12 +597,24 @@ int match_multiscale_batch(b200m_ctx *ctx, const char *name, bool dev, const b20
     c.thr_tgt = thr_tgt;
     c.out = out;
     c.want_avg = avg != nullptr;
+    c.range = r;
     WideLayout W;
-    if (wide_batch_tables(ctx, c, &W, false) || wide_batch_enqueue(ctx, c, W)) return 1;
+    if (wide_batch_tables(ctx, c, &W, false)) return 1;
+    if (r) r->validated = true;
+    if (wide_batch_enqueue(ctx, c, W)) return 1;
     return wide_batch_results(ctx, c, W, out, cap, offsets, avg);
 }
 
 }  // namespace
+
+int match_multiscale_batch_host(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs, bool gated,
+                                const b200m_local_pair *locals, int n_pairs, size_t stride_bytes, int dim, size_t xyz_stride_bytes,
+                                int cluster_k, float radius, const float *thr_src, const float *thr_tgt, b200m_corr *out, size_t cap,
+                                size_t *offsets, float *avg, BatchRange *r) {
+    return match_multiscale_batch(ctx, gated ? "b200m_match_multiscale_local_batch" : "b200m_match_multiscale_batch", false, p, pairs,
+                                  gated, locals, n_pairs, stride_bytes, dim, xyz_stride_bytes, cluster_k, radius, thr_src, thr_tgt, out,
+                                  cap, offsets, avg, r);
+}
 
 extern "C" int b200m_match_multiscale_batch(b200m_ctx *ctx, const b200m_params *p, const b200m_wide_pair *pairs, int n_pairs,
                                             size_t stride_bytes, int dim, size_t xyz_stride_bytes, int cluster_k,

@@ -13,9 +13,12 @@ descriptor -- the AoS layout PCL hands to the reference (`&cloud.points[0]`, `si
 FPFH-33 (33 floats), RoPS-135 (135), SHOT-352 (361: descriptor + rf[9]), USC-1960 (1969: descriptor + rf[9]); any
 dim up to 2048.  There is no CPU path here: without the CUDA library and a B200 every call raises.
 """
+import atexit
+import contextlib
 import ctypes as C
 import dataclasses
 import os
+import threading
 from dataclasses import dataclass
 
 import numpy as np
@@ -96,7 +99,8 @@ EXPORTS = ["b200m_create", "b200m_destroy", "b200m_last_error", "b200m_set_strea
            "b200m_plan_knn_batch", "b200m_plan_match_batch", "b200m_plan_run", "b200m_plan_destroy", "b200m_plan_last_error",
            "b200m_plan_match_multiscale_batch", "b200m_plan_match_multiscale_local_batch", "b200m_plan_status_error",
            "b200m_plan_knn_batch_rows", "b200m_plan_match_batch_rows", "b200m_plan_match_multiscale_batch_rows",
-           "b200m_plan_match_multiscale_local_batch_rows"]
+           "b200m_plan_match_multiscale_local_batch_rows", "b200m_group_knn_batch", "b200m_group_match_batch",
+           "b200m_group_match_multiscale_batch", "b200m_group_match_multiscale_local_batch", "b200m_batch_partition"]
 
 _lib = None
 
@@ -172,6 +176,11 @@ def load_library():
     L.b200m_match_multiscale_local_batch.argtypes = [vp, C.POINTER(_Params), C.POINTER(_WidePair), C.POINTER(_LocalPair), C.c_int, sz,
                                                      C.c_int, sz, C.c_int, C.c_float, fp, fp, vp, sz, C.POINTER(sz), vp]
     L.b200m_knn_batch_device.argtypes = L.b200m_knn_batch.argtypes
+    L.b200m_group_knn_batch.argtypes = L.b200m_knn_batch.argtypes
+    L.b200m_group_match_batch.argtypes = L.b200m_match_batch.argtypes
+    L.b200m_group_match_multiscale_batch.argtypes = L.b200m_match_multiscale_batch.argtypes
+    L.b200m_group_match_multiscale_local_batch.argtypes = L.b200m_match_multiscale_local_batch.argtypes
+    L.b200m_batch_partition.argtypes = [vp, C.c_int, C.c_int, vp]
     L.b200m_match_batch_device.argtypes = L.b200m_match_batch.argtypes
     L.b200m_match_multiscale_batch_device.argtypes = L.b200m_match_multiscale_batch.argtypes
     L.b200m_match_multiscale_local_batch_device.argtypes = L.b200m_match_multiscale_local_batch.argtypes
@@ -436,6 +445,10 @@ class Context:
             raise B200MatchError("dim exceeds the row length")
         return keep, arr, 4 * (width or dim), [int(s.shape[0]) for s, _ in pairs]
 
+    def _batch_call(self, name):
+        # the host batch calls: b200m_<name> on this context (Group: b200m_group_<name>)
+        return getattr(self._L, "b200m_" + name)
+
     def _batch_sides(self, pairs):
         # what the library's two sides hold after a batch call: every set padded to a multiple of 256 rows
         self._batch_rows([(len(s), len(t)) for s, t in pairs])
@@ -453,8 +466,8 @@ class Context:
         dist = np.empty((total, k), np.float32)
         cnt = np.empty((total,), np.int32)
         p = self._params(k, MODE_KNN_ONLY, precision=precision, cand_cap=cand_cap)
-        self._ck(self._L.b200m_knn_batch(self._h, C.byref(p), arr, len(pairs), stride, dim, idx.ctypes.data, dist.ctypes.data,
-                                         cnt.ctypes.data))
+        self._ck(self._batch_call("knn_batch")(self._h, C.byref(p), arr, len(pairs), stride, dim, idx.ctypes.data, dist.ctypes.data,
+                                               cnt.ctypes.data))
         self._batch_sides(pairs)
         off = np.concatenate([[0], np.cumsum(ns)]).astype(np.int64)
         return [(idx[a:b], dist[a:b], cnt[a:b]) for a, b in zip(off[:-1], off[1:])]
@@ -481,10 +494,10 @@ class Context:
         offsets = np.zeros(len(pairs) + 1, np.uint64)
         avg = np.empty(max(len(pairs), 1), np.float32)
         p = self._params(k, mode, ratio_thr, distance_thr, precision, cand_cap)
-        self._ck(self._L.b200m_match_batch(self._h, C.byref(p), arr, len(pairs), stride, dim,
-                                           None if ts is None else ts.ctypes.data, None if tt is None else tt.ctypes.data,
-                                           out.ctypes.data, out.shape[0], offsets.ctypes.data_as(C.POINTER(C.c_size_t)),
-                                           avg.ctypes.data))
+        self._ck(self._batch_call("match_batch")(self._h, C.byref(p), arr, len(pairs), stride, dim,
+                                                 None if ts is None else ts.ctypes.data, None if tt is None else tt.ctypes.data,
+                                                 out.ctypes.data, out.shape[0], offsets.ctypes.data_as(C.POINTER(C.c_size_t)),
+                                                 avg.ctypes.data))
         self._batch_sides(pairs)
         return [(out[int(offsets[i]):int(offsets[i + 1])], float(avg[i])) for i in range(len(pairs))]
 
@@ -764,11 +777,11 @@ class Context:
         tail = (None if ts is None else ts.ctypes.data, None if tt is None else tt.ctypes.data, out.ctypes.data, out.shape[0],
                 offsets.ctypes.data_as(C.POINTER(C.c_size_t)), avg.ctypes.data)
         if radius is None:
-            self._ck(self._L.b200m_match_multiscale_batch(self._h, C.byref(p), arr, len(pairs), width * 4, d, 4 * (xyz_width or 4),
-                                                          int(cluster_k), *tail))
+            self._ck(self._batch_call("match_multiscale_batch")(self._h, C.byref(p), arr, len(pairs), width * 4, d,
+                                                                4 * (xyz_width or 4), int(cluster_k), *tail))
         else:
-            self._ck(self._L.b200m_match_multiscale_local_batch(self._h, C.byref(p), arr, locs, len(pairs), width * 4, d,
-                                                                4 * (xyz_width or 4), int(cluster_k), radius, *tail))
+            self._ck(self._batch_call("match_multiscale_local_batch")(self._h, C.byref(p), arr, locs, len(pairs), width * 4, d,
+                                                                      4 * (xyz_width or 4), int(cluster_k), radius, *tail))
         # what the library's two sides hold afterwards: the last scale's sets of every pair, each padded to 256 rows
         n_last = max((len(f["src_scales"]) for f, (ns, _) in zip(fs, n_kps) if ns), default=0)
         if n_last:
@@ -893,8 +906,14 @@ class Group:
         self._ck(fn(self._h, side, a.ctypes.data, a.shape[0], stride, dim))
         self.n[side] = a.shape[0]
 
+    def _check_uploaded(self):
+        # the library sizes the whole-problem calls from what device 0 holds; after a batch that is not what self.n says
+        if None in self.n:
+            raise B200MatchError("Group: a batch call replaced the uploaded sets; upload both sides again first")
+
     def match(self, k, mode, ratio_thr=MATCHING_RATIO_THRESHOLD, distance_thr=FLT_MAX, thr_src=None, thr_tgt=None,
               precision=PREC_TC_F16):
+        self._check_uploaded()
         out = np.empty(max(self.n[0] * (k if mode == MODE_MUTUAL else 1), 1), CORR_DTYPE)
         ts = None if thr_src is None else np.ascontiguousarray(thr_src, np.float32)
         tt = None if thr_tgt is None else np.ascontiguousarray(thr_tgt, np.float32)
@@ -906,11 +925,65 @@ class Group:
         return out[:n_out.value], float(avg.value)
 
     def knn(self, k, shard=SHARD_QUERY, precision=PREC_TC_F16):
+        self._check_uploaded()
         nq = self.n[0]
         idx, dist, cnt = np.empty((nq, k), np.int32), np.empty((nq, k), np.float32), np.empty((nq,), np.int32)
         p = Context._params(k, MODE_KNN_ONLY, precision=precision, shard=shard)
         self._ck(self._L.b200m_group_knn(self._h, C.byref(p), idx.ctypes.data, dist.ctypes.data, cnt.ctypes.data))
         return idx, dist, cnt
+
+    # -- the host batch calls spread by pairs over the group's devices (b200m_group_*_batch): Context's methods, with the
+    # same arguments and results (each pair's output is what the Context method gives), over the group forms.  They
+    # replace the sets uploaded before (every device then holds its own range's): match / knn raise until both sides are
+    # uploaded again.
+    knn_batch = Context.knn_batch
+    match_batch = Context.match_batch
+    match_wide_batch = Context.match_wide_batch
+    match_wide_local_batch = Context.match_wide_local_batch
+    _wide_batch = Context._wide_batch
+    _params = staticmethod(Context._params)
+    _pairs = staticmethod(Context._pairs)
+    _scales = staticmethod(Context._scales)
+    _WIDE_FIELDS = Context._WIDE_FIELDS
+    _batch_sides = Context._batch_sides
+
+    def _batch_call(self, name):
+        self.n = [None, None]   # set before the call: a failed batch may have replaced the sets too
+        return getattr(self._L, "b200m_group_" + name)
+
+    def _batch_rows(self, counts):
+        pass
+
+
+_groups = threading.local()
+_all_groups = []
+
+
+def shared_group(devices):
+    """One Group per host thread and device list, created on first use and kept (as the C++ shim's shared_group): creating a
+    group starts a context and a thread per device and an NCCL communicator, which can cost more than a batch."""
+    cache = _groups.__dict__.setdefault("by_devices", {})
+    key = tuple(int(d) for d in devices)
+    if key not in cache:
+        cache[key] = Group(list(key))
+        _all_groups.append(cache[key])
+    return cache[key]
+
+
+@atexit.register
+def _close_groups():
+    for g in _all_groups:
+        g.close()
+
+
+def batch_partition(cost, n_parts):
+    """b200m_batch_partition: the contiguous split of pairs with these costs into n_parts ranges that the group batch calls
+    use (pure host code).  -> int array first [n_parts + 1]; range i is [first[i], first[i + 1])."""
+    c = np.ascontiguousarray(cost, np.float64)
+    first = np.zeros(int(n_parts) + 1, np.int32)
+    if load_library().b200m_batch_partition(c.ctypes.data, c.shape[0], int(n_parts), first.ctypes.data) != 0:
+        raise B200MatchError("batch_partition: n_parts must be >= 1 and every cost finite and >= 0")
+    return first
 
 
 # ---- the reference's free functions ------------------------------------------------------
@@ -1131,14 +1204,16 @@ class RatioMatcher(FeatureBasedMatcher):
         return ctx.match(self._k(), self.mode, p.ratio_thr, p.distance_thr, self.thr_src, self.thr_tgt, p.precision, p.cand_cap)
 
 
-def match_many(matchers):
+def match_many(matchers, devices=None):
     """match() of many matchers at once (multi-view registration, one scan against many submaps, an evaluation table): one
     batch call instead of one call per matcher.  All matchers must be of one class, with equal AlignmentParameters (the guess
     aside: each matcher may have its own), dim and device.  Matchers with a guess go through Context.match_wide_local_batch;
     either every matcher has one or none has.  Without guesses, RatioMatchers and matchers whose vote is the identity and
     that have no keypoint coordinates go through Context.match_batch (as match() sends them to the k-list call), every other
     through Context.match_wide_batch.  Applies each matcher's finalize and sets its average distance; returns one
-    correspondence array per matcher, each equal to what that matcher's match() returns."""
+    correspondence array per matcher, each equal to what that matcher's match() returns.  devices: None (the matchers'
+    device) or a list of device ids; with several, the batch is spread by pairs over them by this thread's shared_group of
+    those devices (same results), with one, it runs on that device."""
     ms = list(matchers)
     if not ms:
         return []
@@ -1151,12 +1226,18 @@ def match_many(matchers):
     if len({m.parameters.guess is None for m in ms}) > 1:
         raise B200MatchError("match_many: give every matcher a guess or none (the guessed and unguessed kNN are different calls)")
     p = m0.parameters
+
+    def backend():
+        if devices and len(devices) > 1:
+            return contextlib.nullcontext(shared_group(devices))
+        return Context(devices[0] if devices else m0.device)
+
     if p.guess is not None:
         guesses = [m._guess() for m in ms]
         ts = None if all(m.thr_src is None and m.thr_tgt is None for m in ms) else [
             np.full(len(m.xyz_src), np.inf, np.float32) if m.thr_src is None else m.thr_src for m in ms]
         tt = None if ts is None else [np.full(len(m.xyz_tgt), np.inf, np.float32) if m.thr_tgt is None else m.thr_tgt for m in ms]
-        with Context(m0.device) as ctx:
+        with backend() as ctx:
             got = ctx.match_wide_local_batch(m0._k(), m0.mode, [m._wide_pair(g) for m, g in zip(ms, guesses)],
                                              p.match_search_radius, m0.dim, p.cluster_k, p.distance_thr, ts, tt)
         return [m._finalize(*r) for m, r in zip(ms, got)]
@@ -1184,7 +1265,7 @@ def match_many(matchers):
         return ts, tt
 
     results = [None] * len(ms)
-    with Context(m0.device) as ctx:
+    with backend() as ctx:
         if narrow:
             ts, tt = thresholds(narrow)
             k = m0._k() if isinstance(m0, RatioMatcher) else 1
